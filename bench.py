@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the erasure-coding + CRC engine (contract: task brief ④).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   (N > 1: launched by torchrun, one rank per GPU; no data-path collective — chunks are independent,
    tiles are dealt round-robin, NCCL is used only for the barrier / max-over-ranks of the timing.)
 
@@ -64,7 +64,24 @@ def parse_args():
     ap.add_argument("--cpu-chunks", type=int, default=0, help="chunks in the CPU baseline sample (0 = auto)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (rank 0): every block "
+                                                          "CRC and a fixed, seeded sample of the parity bytes, to compare two builds output for output")
     return ap.parse_args()
+
+
+DUMP_PARITY_SAMPLES = 1 << 23
+
+
+def dump_outputs(torch, out_dir, d_par, d_crc):
+    """The headline step's results as float arrays: crc.npy holds every block CRC of the tile (float64, exact for uint32) in the
+    layout encode_chunks_dev writes, parity_sample.npy the parity bytes (float32) at DUMP_PARITY_SAMPLES positions drawn with a
+    fixed seed (the whole parity output of a tile is gigabytes).  The inputs come from a fixed seed as well, so two runs with
+    the same arguments dump the same arrays."""
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.default_rng(2024).integers(0, d_par.numel(), size=DUMP_PARITY_SAMPLES, dtype=np.int64))
+    sample = d_par[torch.from_numpy(idx).to(d_par.device)].cpu().numpy()
+    np.save(os.path.join(out_dir, "parity_sample.npy"), sample.astype(np.float32))
+    np.save(os.path.join(out_dir, "crc.npy"), d_crc.cpu().numpy().view(np.uint32).astype(np.float64))
 
 
 def algorithmic_bytes_per_chunk(k, m, chunk_len=CHUNK):
@@ -660,6 +677,8 @@ def main():
     ms_total_max = float(t.item())
     value = world * T * args.steps * CHUNK / GIB / (ms_total_max / 1e3)
     lib_stats = eng.stats()   # the library's own per-batch device timing of the same launches (lzgpu_stats.batch_*)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, d_par, d_crc)
 
     # ---- the timed launches' results against the reference: parity parts and CRCs of chunks spread over the resident tile
     checker, checker_name = _ref_lib()

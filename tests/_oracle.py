@@ -2,6 +2,8 @@
 reference build (oracle/_ref/liblzref.so).  TEST INFRASTRUCTURE ONLY — nothing under
 lizardfs_b200/ imports this module."""
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 
@@ -163,13 +165,34 @@ def load_oracle():
 
 
 def load_ref():
+    """The reference compiled by oracle/Makefile; None where its sources were not there to build it.  The tests compare with
+    what it computed through tests/golden/reference_outputs.json instead (tests/golden/gen_golden.py writes that file)."""
     path = os.path.join(ORACLE_DIR, "_ref", "liblzref.so")
-    if not os.path.exists(path):
-        if os.path.isdir("/root/reference/src/common"):
-            build_oracle()
-        if not os.path.exists(path):
-            return None
-    return Lib(C.CDLL(path), "ref_")
+    return Lib(C.CDLL(path), "ref_") if os.path.exists(path) else None
+
+
+def sha256(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def crc_sha256(crcs):
+    return sha256(np.asarray(crcs, dtype="<u4"))
+
+
+def golden_key(*fields):
+    return "|".join(str(f) for f in fields)
+
+
+_REFERENCE_OUTPUTS = None
+
+
+def reference_outputs(section):
+    """One section of tests/golden/reference_outputs.json: what the unmodified reference computed for the tests' seeded inputs."""
+    global _REFERENCE_OUTPUTS
+    if _REFERENCE_OUTPUTS is None:
+        with open(os.path.join(ROOT, "tests", "golden", "reference_outputs.json")) as f:
+            _REFERENCE_OUTPUTS = json.load(f)
+    return _REFERENCE_OUTPUTS[section]
 
 
 def fill_chunk(oracle, nbytes, seed, chunk_index=0):

@@ -1,22 +1,21 @@
 // GPU test of include/lzgpu_read_plan.hpp — the GPU-backed mirror of ReadPlan::postProcessData — on read plans built by
-// the REFERENCE's own planners.  oracle/_ref/liblzref.so (the unmodified reference compiled from its sources, test
-// infrastructure) runs ChunkReadPlanner for a chunk read with some parts missing, serves the planned read operations from
-// memory the way src/unittests/plan_tester.cc does, and hands back (a) the plan's fields, (b) the buffer as the executor
-// leaves it, (c) the reference's own post-processed result.  The mirror must turn (b) into (c), byte for byte.
+// the REFERENCE's own planners.  tests/golden/read_plans.txt holds, for each chunk read with some parts missing, the plan
+// the reference's ChunkReadPlanner built (recorded by tests/golden/gen_golden.py through oracle/ref_plans.cc
+// ref_plan_chunk_read_staged).  The test serves the planned read operations from memory the way src/unittests/plan_tester.cc
+// does, and the mirror must turn that buffer into the chunk data that was asked for, byte for byte (the reference's own
+// post-processed result, which gen_golden.py checked to be that data).
+#include <algorithm>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <fstream>
+#include <string>
 #include <vector>
 
 #include "lzgpu_read_plan.hpp"
 
-extern "C" {
-long ref_plan_chunk_read_staged(int n_avail, const int *types, const int *parts, const uint8_t *const *data, const size_t *bytes,
-                                int first_block, int block_count, int *desc, int desc_cap, uint8_t *staged, uint8_t *expected,
-                                size_t buffer_cap);
-int ref_encode_chunk(int kind, int k, int m, const uint8_t *chunk, size_t chunk_len, uint8_t *parity, uint32_t *crc);
-}
+extern "C" int lzo_encode_chunk(int kind, int k, int m, const uint8_t *chunk, size_t chunk_len, uint8_t *parity, uint32_t *crc);
 
 static int failures = 0;
 #define EXPECT(cond)                                                        \
@@ -30,16 +29,18 @@ static int failures = 0;
 static const size_t B = LZGPU_BLOCK_SIZE;
 
 struct Case {
-	const char *goal;
+	std::string goal;
 	std::vector<int> lost;  // this library's part indices (data 0..k-1, parity k..)
 	int nb, first_block, block_count;
+	long full;              // the plan's full buffer size
+	std::vector<int> desc;  // the plan, laid out as oracle/ref_plans.cc ref_plan_chunk_read_staged writes it
 };
 
 static void run(const Case &c) {
 	lzgpu_goal g;
-	EXPECT(lzgpu_goal_parse(c.goal, &g) == LZGPU_OK);
+	EXPECT(lzgpu_goal_parse(c.goal.c_str(), &g) == LZGPU_OK);
 	const int k = g.k, m = g.m, pb = (c.nb + k - 1) / k;
-	// chunk data and the parts of the slice (data parts zero-padded, parity from the reference encoder)
+	// chunk data and the parts of the slice (data parts zero-padded, parity from the CPU oracle's encoder)
 	std::vector<uint8_t> chunk(static_cast<size_t>(pb) * k * B, 0);
 	uint64_t s = 0x9E3779B97F4A7C15ull * (c.nb + 7);
 	for (size_t i = 0; i < c.nb * B; ++i) {
@@ -50,30 +51,12 @@ static void run(const Case &c) {
 	for (int b = 0; b < c.nb; ++b) std::memcpy(&part[b % k][(b / k) * B], &chunk[b * B], B);
 	std::vector<uint8_t> parity(static_cast<size_t>(m) * pb * B);
 	std::vector<uint32_t> crc(c.nb + m * pb);
-	EXPECT(ref_encode_chunk(g.kind, k, m, chunk.data(), static_cast<size_t>(c.nb) * B, parity.data(), crc.data()) == 0);
+	EXPECT(lzo_encode_chunk(g.kind, k, m, chunk.data(), static_cast<size_t>(c.nb) * B, parity.data(), crc.data()) == 0);
 	for (int r = 0; r < m; ++r) std::memcpy(part[k + r].data(), &parity[r * pb * B], pb * B);
 
-	// available parts in the reference's terms
 	const int type = lzgpu_goal_slice_type(&g);
-	std::vector<int> types, parts;
-	std::vector<const uint8_t *> data;
-	std::vector<size_t> bytes;
-	for (int i = 0; i < k + m; ++i) {
-		bool lost = false;
-		for (int l : c.lost) lost |= l == i;
-		if (lost) continue;
-		types.push_back(type);
-		parts.push_back(lzgpu_ref_part_index(&g, i));
-		data.push_back(part[i].data());
-		bytes.push_back(static_cast<size_t>(lzgpu_part_blocks(&g, i, c.nb)) * B);  // the real length of the part on a chunkserver
-	}
-	const size_t cap = (static_cast<size_t>(k + m) * pb + c.block_count + 8) * B;
-	std::vector<uint8_t> staged(cap), expected(cap);
-	std::vector<int> desc(1024);
-	const long full = ref_plan_chunk_read_staged(static_cast<int>(types.size()), types.data(), parts.data(), data.data(), bytes.data(), c.first_block,
-	                                             c.block_count, desc.data(), static_cast<int>(desc.size()), staged.data(), expected.data(), cap);
-	EXPECT(full > 0);
-	if (full <= 0) return;
+	const std::vector<int> &desc = c.desc;
+	const long full = c.full;
 
 	// the reference's plan -> the mirror's fields
 	lzgpu::SliceReadPlan plan;
@@ -95,31 +78,70 @@ static void run(const Case &c) {
 	for (int n = desc[p++]; n > 0; --n) available.push_back(desc[p++]);
 	EXPECT(plan.slice_type == type);
 	EXPECT(plan.readOffset() == read_offset && plan.fullBufferSize() == full);
+	EXPECT(p == static_cast<int>(desc.size()));
+
+	// the executor (plan_tester.cc:155-184): every read operation of a part that was read, in wave order, served from the parts
+	// of the chunk cut to their real length on a chunkserver
+	std::vector<uint8_t> staged(full, 0);
+	for (int wave = 0; wave < 10; ++wave)
+		for (const auto &op : plan.read_operations) {
+			if (op.second.wave != wave) continue;
+			bool read = false;
+			for (int a : available) read |= a == op.first;
+			if (!read) continue;
+			int i = 0;
+			while (i < k + m && lzgpu_ref_part_index(&g, i) != op.first) ++i;
+			EXPECT(i < k + m);
+			if (i == k + m) return;
+			const size_t bytes = static_cast<size_t>(lzgpu_part_blocks(&g, i, c.nb)) * B;
+			const size_t off = op.second.request_offset, size = op.second.request_size;
+			if (off < bytes) std::memcpy(&staged[read_offset + op.second.buffer_offset], &part[i][off], std::min(size, bytes - off));
+		}
 
 	const int size = plan.postProcessData(lzgpu_default_ctx(), staged.data(), available);
 	EXPECT(size == c.block_count * static_cast<int>(B));
-	EXPECT(std::memcmp(staged.data(), expected.data(), size) == 0);
-	EXPECT(std::memcmp(staged.data(), &chunk[c.first_block * B], size) == 0);  // and it is the chunk data that was asked for
-	std::printf("%s lost %zu part(s), blocks [%d, %d): %s\n", c.goal, c.lost.size(), c.first_block, c.first_block + c.block_count,
+	EXPECT(std::memcmp(staged.data(), &chunk[c.first_block * B], size) == 0);  // the chunk data that was asked for
+	std::printf("%s lost %zu part(s), blocks [%d, %d): %s\n", c.goal.c_str(), c.lost.size(), c.first_block, c.first_block + c.block_count,
 	            failures ? "FAIL" : "ok");
 }
 
-int main() {
+// argv[1]: tests/golden/read_plans.txt, one case per line:
+//   goal nb first_block block_count full_buffer_size n_lost lost... n_desc desc...
+static std::vector<Case> load_cases(const char *path) {
+	std::vector<Case> cases;
+	std::ifstream in(path);
+	Case c;
+	int n;
+	while (in >> c.goal >> c.nb >> c.first_block >> c.block_count >> c.full >> n) {
+		c.lost.assign(n, 0);
+		for (int &l : c.lost) in >> l;
+		in >> n;
+		c.desc.assign(n, 0);
+		for (int &d : c.desc) in >> d;
+		if (in) cases.push_back(c);
+	}
+	return cases;
+}
+
+int main(int argc, char **argv) {
+	if (argc != 2) {
+		std::fprintf(stderr, "usage: %s tests/golden/read_plans.txt\n", argv[0]);
+		return 2;
+	}
 	if (!lzgpu_default_ctx()) {
 		std::fprintf(stderr, "no GPU context: %s\n", lzgpu_last_error());
 		return 2;
 	}
-	const Case cases[] = {
-	    {"ec(8,2)", {1, 4}, 64, 0, 64},   {"ec(8,2)", {1, 4}, 61, 3, 50}, {"ec(8,2)", {7}, 19, 0, 19},     {"ec(8,2)", {}, 32, 5, 20},
-	    {"ec(3,2)", {0, 2}, 10, 0, 10},   {"ec(3,2)", {1}, 31, 7, 11},    {"ec(3,2)", {0, 4}, 7, 2, 2},     {"ec(5,3)", {0, 1, 4}, 23, 0, 23},
-	    {"ec(5,3)", {2, 6}, 40, 9, 17},   {"xor3", {1}, 22, 0, 22},       {"xor3", {0}, 22, 4, 10},         {"xor3", {3}, 7, 1, 5},
-	    {"xor2", {2}, 9, 0, 9},           {"xor9", {4}, 100, 13, 60},     {"ec(22,4)", {0, 5, 21, 23}, 70, 0, 70}, {"ec(8,2)", {0}, 1024, 0, 1024},
-	};
+	const std::vector<Case> cases = load_cases(argv[1]);
+	if (cases.empty()) {
+		std::fprintf(stderr, "no read plans in %s\n", argv[1]);
+		return 2;
+	}
 	for (const Case &c : cases) run(c);
 	if (failures) {
 		std::fprintf(stderr, "%d failure(s)\n", failures);
 		return 1;
 	}
-	std::printf("read plan mirror: all tests passed\n");
+	std::printf("read plan mirror: %zu plans, all tests passed\n", cases.size());
 	return 0;
 }

@@ -1,5 +1,5 @@
 """GPU parity tests of the BIT-SLICED three- and four-parity-row encoders (fused_stream_kernel, W = 8 items, csrc/bitslice.cuh)
-against the oracle / the compiled reference: every Vandermonde ec(k,4) (k <= 20; larger k use Cauchy rows,
+against the oracle / what the compiled reference computed: every Vandermonde ec(k,4) (k <= 20; larger k use Cauchy rows,
 reed_solomon.h:168-172) and ec(k,3) in all three unit modes (per-chunk, flat, striped), tail stripes, padded strides, full 64 MiB chunks — and, both ways round, that the
 packed-byte Horner route (LZGPU_BITSLICE=0) and the bit-plane route (LZGPU_BITSLICE=7: also the three-row goals with k < 7, which
 the default routes to the packed-byte kernels) give the same bytes."""
@@ -10,6 +10,7 @@ import pytest
 
 import lizardfs_b200 as L
 from tests import _oracle as O
+from tests.test_gpu_chunks import check_encode_against_reference
 
 pytestmark = pytest.mark.gpu
 BLOCK = 65536
@@ -102,32 +103,33 @@ def test_ragged_chunks_striped_and_per_chunk_units(oracle, striped, text, nblock
     e.close()
 
 
-@pytest.mark.parametrize("text", ["ec(8,4)", "ec(6,4)", "ec(4,4)", "ec(10,4)", "ec(12,4)", "ec(7,4)", "ec(20,4)", "ec(5,3)", "ec(6,3)", "ec(8,3)", "ec(4,3)", "ec(9,3)", "ec(31,3)"])
-def test_full_size_chunks_vs_reference(eng_bs, oracle, ref, text):
+FULL_SIZE_GOALS = ["ec(8,4)", "ec(6,4)", "ec(4,4)", "ec(10,4)", "ec(12,4)", "ec(7,4)", "ec(20,4)", "ec(5,3)", "ec(6,3)", "ec(8,3)", "ec(4,3)", "ec(9,3)",
+                   "ec(31,3)"]
+SWEEP_GOALS = ["ec(8,4)", "ec(5,3)"]
+SWEEP_BLOCKS = [16, 64, 256, 597]
+
+
+@pytest.mark.parametrize("text", FULL_SIZE_GOALS)
+def test_full_size_chunks_vs_reference(eng_bs, oracle, text):
     """the size the numbers are quoted on: two full 64 MiB chunks per goal (the second one starts in the unit that straddles the
-    chunk boundary), parity parts and all block CRCs bit-exact against the compiled reference (the restatement where it is absent)"""
+    chunk boundary), parity parts and all block CRCs bit-exact against the compiled reference"""
     goal = L.SliceType(text)
     data = np.stack([O.fill_chunk(oracle, 64 << 20, 4242, c) for c in (1, 2)])
     parity, crc = eng_bs.encode_chunks(goal, data)
-    checker = ref if ref is not None else oracle
-    for c in range(2):
-        p_ref, c_ref = checker.encode_chunk(goal.kind, goal.k, goal.m, data[c])
-        assert (parity[c] == p_ref).all(), (text, c)
-        assert (crc[c] == c_ref).all(), (text, c)
+    for c, chunk_index in enumerate((1, 2)):
+        check_encode_against_reference(text, 4242, chunk_index, 1024, parity[c], crc[c])
 
 
-@pytest.mark.parametrize("clen_blocks", [16, 64, 256, 597])
-@pytest.mark.parametrize("text", ["ec(8,4)", "ec(5,3)"])
-def test_sweep_chunk_sizes(eng_bs, oracle, ref, text, clen_blocks):
+@pytest.mark.parametrize("clen_blocks", SWEEP_BLOCKS)
+@pytest.mark.parametrize("text", SWEEP_GOALS)
+def test_sweep_chunk_sizes(eng_bs, oracle, text, clen_blocks):
     """the other chunk sizes of the mixed sweep (1, 4, 16 and 37.31 MiB) for the three- and four-parity goals of BASELINE configs[4]"""
     goal = L.SliceType(text)
     n = 5
     data = np.stack([O.fill_chunk(oracle, clen_blocks * BLOCK, 778, c) for c in range(n)])
     parity, crc = eng_bs.encode_chunks(goal, data)
-    checker = ref if ref is not None else oracle
     for c in (0, n // 2, n - 1):
-        p_ref, c_ref = checker.encode_chunk(goal.kind, goal.k, goal.m, data[c])
-        assert (parity[c] == p_ref).all() and (crc[c] == c_ref).all(), (text, clen_blocks, c)
+        check_encode_against_reference(text, 778, c, clen_blocks, parity[c], crc[c])
 
 
 @pytest.mark.parametrize("text", ["ec(8,4)", "ec(5,3)"])

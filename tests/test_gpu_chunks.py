@@ -197,14 +197,20 @@ def test_encode_partial_last_block(eng, oracle):
         assert (parity[c] == p_ref).all() and (crc[c] == c_ref).all()
 
 
-def test_encode_full_size_chunk_ec82(eng, oracle, ref):
+def check_encode_against_reference(text, seed, chunk_index, nblocks, parity, crc):
+    """one chunk's parity parts and block CRCs against what the compiled reference computed for the same chunk
+    (O.fill_chunk(seed, chunk_index) of nblocks blocks; recorded by tests/golden/gen_golden.py)"""
+    p_sha, c_sha = O.reference_outputs("encode")[O.golden_key(text, seed, chunk_index, nblocks)]
+    assert O.sha256(parity) == p_sha, (text, seed, chunk_index, nblocks)
+    assert O.crc_sha256(crc) == c_sha, (text, seed, chunk_index, nblocks)
+
+
+def test_encode_full_size_chunk_ec82(eng, oracle):
     """BASELINE config 3 shape: ec(8,2) on a full 64 MiB chunk, bit-exact vs the (compiled) reference."""
     goal = L.SliceType("ec(8,2)")
     data = O.fill_chunk(oracle, 64 << 20, 1, 0).reshape(1, -1)
     parity, crc = eng.encode_chunks(goal, data)
-    checker = ref if ref is not None else oracle
-    p_ref, c_ref = checker.encode_chunk(1, 8, 2, data[0])
-    assert (parity[0] == p_ref).all() and (crc[0] == c_ref).all()
+    check_encode_against_reference("ec(8,2)", 1, 0, 1024, parity[0], crc[0])
     assert crc[0, 0] == 0x7173879a and crc[0, 1023] == 0xfa2e261f          # SURVEY §8c known answers
     assert parity[0, 0, :8].tobytes().hex() == "183a4cd28cd5bfa7" and parity[0, 1, :8].tobytes().hex() == "a1a590174c2d64f0"
     assert crc[0, 1024] == 0x8c7def0b and crc[0, 1024 + 128] == 0x577d57e4
@@ -241,57 +247,64 @@ def test_encode_many_parity_goals_in_passes(eng, oracle, text, nblocks, n_chunks
         assert (crc[c] == c_ref).all(), (text, c)
 
 
-@pytest.mark.parametrize("text", ["xor2", "xor3", "ec(5,3)", "ec(8,4)", "ec(3,2)", "ec(8,2)", "ec(8,3)", "ec(6,4)", "ec(4,4)", "ec(6,3)", "ec(4,2)", "ec(6,2)",
-                                  "xor4", "ec(5,2)", "ec(10,2)", "ec(4,3)", "ec(10,4)", "ec(12,4)"])
-def test_encode_full_size_chunk_every_bench_goal_vs_reference(eng, oracle, ref, text):
+FULL_SIZE_GOALS = ["xor2", "xor3", "ec(5,3)", "ec(8,4)", "ec(3,2)", "ec(8,2)", "ec(8,3)", "ec(6,4)", "ec(4,4)", "ec(6,3)", "ec(4,2)", "ec(6,2)",
+                   "xor4", "ec(5,2)", "ec(10,2)", "ec(4,3)", "ec(10,4)", "ec(12,4)"]
+SWEEP_GOALS = ["xor2", "xor3", "ec(5,3)", "ec(8,4)"]
+SWEEP_BLOCKS = [16, 64, 256, 597]
+
+
+@pytest.mark.parametrize("text", FULL_SIZE_GOALS)
+def test_encode_full_size_chunk_every_bench_goal_vs_reference(eng, oracle, text):
     """BASELINE configs[1], [2], [4] at the size the numbers are quoted on: one full 64 MiB chunk per goal of the mixed sweep,
-    parity parts and all block CRCs bit-exact against the compiled reference (oracle/_ref; the restatement where it is absent).
+    parity parts and all block CRCs bit-exact against the compiled reference.
     Two chunks are encoded so that the second one exercises the unit that straddles the chunk boundary."""
     goal = L.SliceType(text)
     data = np.stack([O.fill_chunk(oracle, 64 << 20, 12345, c) for c in (3, 4)])
     parity, crc = eng.encode_chunks(goal, data)
-    checker = ref if ref is not None else oracle
-    for c in range(2):
-        p_ref, c_ref = checker.encode_chunk(goal.kind, goal.k, goal.m, data[c])
-        assert (parity[c] == p_ref).all(), (text, c)
-        assert (crc[c] == c_ref).all(), (text, c)
+    for c, chunk_index in enumerate((3, 4)):
+        check_encode_against_reference(text, 12345, chunk_index, 1024, parity[c], crc[c])
 
 
-@pytest.mark.parametrize("clen_blocks", [16, 64, 256, 597])
-@pytest.mark.parametrize("text", ["xor2", "xor3", "ec(5,3)", "ec(8,4)"])
-def test_encode_sweep_chunk_sizes_vs_reference(eng, oracle, ref, text, clen_blocks):
+@pytest.mark.parametrize("clen_blocks", SWEEP_BLOCKS)
+@pytest.mark.parametrize("text", SWEEP_GOALS)
+def test_encode_sweep_chunk_sizes_vs_reference(eng, oracle, text, clen_blocks):
     """the other chunk sizes of the mixed sweep (1, 4, 16 and 37.31 MiB), a batch of several chunks each, vs the reference"""
     goal = L.SliceType(text)
     n = 5
     data = np.stack([O.fill_chunk(oracle, clen_blocks * BLOCK, 777, c) for c in range(n)])
     parity, crc = eng.encode_chunks(goal, data)
-    checker = ref if ref is not None else oracle
     for c in (0, n // 2, n - 1):
-        p_ref, c_ref = checker.encode_chunk(goal.kind, goal.k, goal.m, data[c])
-        assert (parity[c] == p_ref).all() and (crc[c] == c_ref).all(), (text, clen_blocks, c)
+        check_encode_against_reference(text, 777, c, clen_blocks, parity[c], crc[c])
 
 
-def test_recover_full_size_every_pair_vs_reference(eng, oracle, ref):
+def full_size_pairs():
+    """the lost pairs of ec(8,2) also checked against the reference's recover: a third of them"""
+    return [lost for lost in itertools.combinations(range(10), 2) if lost[1] - lost[0] in (1, 5)]
+
+
+def test_recover_full_size_every_pair_vs_reference(eng, oracle):
     """BASELINE configs[3] at full size: ec(8,2), one 64 MiB chunk, EVERY pair of lost parts (28 data pairs, 16 data+parity
     pairs, the parity pair), rebuilt parts compared with the reference's own recover (ECReadPlan::recoverParts semantics,
     oracle ref_recover_chunk) and with the withheld originals."""
     goal = L.SliceType("ec(8,2)")
-    k, m, nb, pb = 8, 2, 1024, 128
+    k, m, nb = 8, 2, 1024
     data = O.fill_chunk(oracle, 64 << 20, 4242, 0).reshape(1, -1)
     parity, crc = eng.encode_chunks(goal, data)
+    check_encode_against_reference("ec(8,2)", 4242, 0, nb, parity[0], crc[0])
     parts = all_parts(data, parity, k)
-    checker = ref if ref is not None else oracle
+    gold = O.reference_outputs("recover_pairs")
+    checked = 0
     for lost in itertools.combinations(range(k + m), 2):
         avail = [None if i in lost else parts[i] for i in range(k + m)]
         want = [1 if i in lost else 0 for i in range(k + m)]
         out, _ = eng.recover_chunks(goal, nb, avail, want=want)
         for i in lost:
             assert (out[i][0] == parts[i][0]).all(), (lost, i)
-        if lost[1] - lost[0] in (1, 5):   # a third of the patterns also against the reference's recover (it is slow at this size)
-            rc, ro, _ = checker.recover_chunk(goal.kind, k, m, [None if a is None else a[0] for a in avail], None, want, pb)
-            assert rc == 0
+        if lost in full_size_pairs():
             for i in lost:
-                assert (ro[i] == out[i][0]).all(), (lost, i)
+                assert O.sha256(out[i][0]) == gold[O.golden_key(*lost, i)], (lost, i)
+                checked += 1
+    assert checked == len(gold)
 
 
 def test_full_size_batch_roundtrip_with_verification(eng):

@@ -46,30 +46,28 @@ def test_stripe_batcher_cpp():
 
 
 READ_PLAN = os.path.join(ROOT, "tests", "cpp", "build", "test_read_plan")
+READ_PLANS = os.path.join(ROOT, "tests", "golden", "read_plans.txt")
 
 
 @pytest.mark.gpu
 def test_read_plan_mirror_cpp():
     """lzgpu::SliceReadPlan (include/lzgpu_read_plan.hpp), the GPU-backed mirror of ReadPlan::postProcessData, on plans
-    built and pre-executed by the reference's own ChunkReadPlanner (oracle/_ref) — must reproduce the reference's
+    built by the reference's own ChunkReadPlanner (tests/golden/read_plans.txt) — must reproduce the reference's
     post-processed buffer byte for byte (tests/cpp/test_read_plan.cc)."""
     if not os.path.exists(READ_PLAN):
-        pytest.skip("oracle/_ref/liblzref.so was not built (no /root/reference), so the reference planners are unavailable")
-    r = subprocess.run([READ_PLAN], capture_output=True, text=True, timeout=600)
+        subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "tests", "cpp")], check=True)
+    r = subprocess.run([READ_PLAN, READ_PLANS], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stdout + r.stderr
-    assert "all tests passed" in r.stdout
+    assert "16 plans, all tests passed" in r.stdout
 
 
-def _run_cpu_build(name, needs_ref=False):
+def _run_cpu_build(name, *args):
     """The same C++ test source linked against tests/cpp/oracle_backend.cc (a test-only stand-in for the GPU entry points backed
     by the CPU oracle) instead of liblzgpu.so: covers the HOST logic of the header on a machine without a GPU."""
     exe = os.path.join(ROOT, "tests", "cpp", "build", name)
     if not os.path.exists(exe):
         subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "tests", "cpp")], check=True)
-    if not os.path.exists(exe):
-        assert needs_ref, f"{name} was not built"
-        pytest.skip("oracle/_ref/liblzref.so was not built (no /root/reference), so the reference planners are unavailable")
-    r = subprocess.run([exe], capture_output=True, text=True, timeout=600)
+    r = subprocess.run([exe, *args], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stdout + r.stderr
     assert "all tests passed" in r.stdout
 
@@ -80,8 +78,9 @@ def test_stripe_batcher_host_logic_on_cpu():
 
 
 def test_read_plan_mirror_host_logic_on_cpu():
-    """part numbering, buffer layout, BlockConverter of lzgpu::SliceReadPlan on plans built by the reference's ChunkReadPlanner"""
-    _run_cpu_build("test_read_plan_cpu", needs_ref=True)
+    """part numbering, buffer layout, BlockConverter of lzgpu::SliceReadPlan on plans built by the reference's ChunkReadPlanner
+    (tests/golden/read_plans.txt)"""
+    _run_cpu_build("test_read_plan_cpu", READ_PLANS)
 
 
 LINK_SUB = os.path.join(ROOT, "tests", "cpp", "build", "test_link_substitution")

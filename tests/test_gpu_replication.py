@@ -7,7 +7,7 @@ import pytest
 
 import lizardfs_b200 as L
 from tests import _oracle as O
-from tests.test_oracle_plans import CASES, GOALS, make_slice, ref_sources, true_blocks
+from tests.test_oracle_plans import CASES, GOALS, check_against_reference_parts, make_slice
 
 pytestmark = pytest.mark.gpu
 BLOCK = 65536
@@ -43,26 +43,22 @@ def test_convert_chunks_vs_oracle(eng, oracle, src_name, lost, nb, dst_name):
             assert (ocrc[i][c] == want_crc[i]).all(), (src_name, dst_name, c, i)
 
 
-def test_convert_chunks_vs_reference_planner(eng, oracle, ref):
-    """straight against the reference's SliceRecoveryPlanner + post-processing executed in memory (oracle/ref_plans.cc)"""
-    if ref is None:
-        pytest.skip("compiled reference not present")
-    for (src_name, lost, nb), dst_name in [(("ec(3,2)", (0, 2), 10), "ec(8,2)"), (("xor3", (1,), 10), "ec(3,2)"), (("std", (), 9), "xor2"),
-                                           (("ec(8,2)", (), 16), "std"), (("ec(5,3)", (0, 1, 4), 11), "ec(5,3)")]:
+PLANNER_CONVERSIONS = [(("ec(3,2)", (0, 2), 10), "ec(8,2)"), (("xor3", (1,), 10), "ec(3,2)"), (("std", (), 9), "xor2"), (("ec(8,2)", (), 16), "std"),
+                       (("ec(5,3)", (0, 1, 4), 11), "ec(5,3)")]
+
+
+def test_convert_chunks_vs_reference_planner(eng, oracle):
+    """straight against what the reference's SliceRecoveryPlanner + post-processing executed in memory (oracle/ref_plans.cc)
+    rebuilt from the same chunk"""
+    gold = O.reference_outputs("recover_part")
+    for (src_name, lost, nb), dst_name in PLANNER_CONVERSIONS:
         src, dst = GOALS[src_name], GOALS[dst_name]
         chunk = O.fill_chunk(oracle, nb * BLOCK, 8, 2)
         sparts, _ = make_slice(oracle, src, chunk)
         parts = [None if i in lost else sparts[i][None, :] for i in range(len(sparts))]
         nd = dst[1] + dst[2]
         out, ocrc = eng.convert_chunks(slice_of(src_name), slice_of(dst_name), nb, parts, [1] * nd)
-        sources = ref_sources(src, sparts, nb, lost)
-        for i in range(nd):
-            nblk = true_blocks(dst, i, nb)
-            if nblk == 0:
-                continue
-            data, crc = O.plan_recover_part(ref, sources, O.slice_type(*dst), O.ref_part_number(dst[0], dst[1], i), 0, nblk)
-            assert (out[i][0][: nblk * BLOCK] == data).all(), (src_name, dst_name, i)
-            assert (ocrc[i][0][:nblk] == crc).all()
+        check_against_reference_parts(gold[O.golden_key(src_name, lost, nb, dst_name, 8, 2)], dst, nb, [o[0] for o in out], [c[0] for c in ocrc])
 
 
 def test_convert_only_wanted_parts_and_crc_errors(eng, oracle):
@@ -273,8 +269,34 @@ def test_scrub_moosefs_format(eng, oracle, data_parts):
     assert ei.value.where == (0,)
 
 
-def test_write_blocks_matches_hdd_write(eng, oracle, ref):
-    """batched chunkserver block writes against the restated hdd_write (hddspacemgr.cc:1898-2008), request by request"""
+def test_write_blocks_matches_hdd_write(eng):
+    """batched chunkserver block writes against the transcription of hdd_write (hddspacemgr.cc:1898-2008) onto the compiled
+    reference's crc.cc, request by request"""
+    blocks, stored, writes, shapes = write_block_requests()
+    expect = O.reference_outputs("write_blocks")
+    assert len(expect) == len(writes)
+    before_blocks, before_crc = blocks.copy(), stored.copy()
+    status = eng.write_blocks(blocks, stored, writes)
+    code = {0: 0, -3: L._lib.ERR_CRC, -4: L._lib.ERR_DAMAGED, -1: L._lib.ERR_ARG}
+    seen = set()
+    for i, (rc, blk_sha, new_crc) in enumerate(expect):
+        assert status[i] == code[rc], (i, shapes[i % len(shapes)], status[i], rc)
+        seen.add(rc)
+        if rc == 0:
+            assert O.sha256(blocks[i]) == blk_sha and stored[i] == new_crc, i
+            assert stored[i] == zlib.crc32(blocks[i].tobytes())
+        else:
+            assert (blocks[i] == before_blocks[i]).all() and stored[i] == before_crc[i]
+    assert seen == {0, -3, -4}
+    # argument errors: range outside the block, two writes to one block
+    st = eng.write_blocks(blocks, stored, [dict(block=0, offset=65000, data=np.zeros(1000, np.uint8), crc=0)])
+    assert st == [L._lib.ERR_ARG]
+    with pytest.raises(L.LzGpuError):
+        eng.write_blocks(blocks, stored, [dict(block=1, offset=0, data=np.zeros(4, np.uint8), crc=0), dict(block=1, offset=8, data=np.zeros(4, np.uint8), crc=0)])
+
+
+def write_block_requests():
+    """the stored blocks, their CRCs and the write requests of the test above (three variants of 15 write shapes)"""
     rng = np.random.default_rng(11)
     shapes = [(0, 65536), (0, 1), (0, 4096), (1, 65535), (65535, 1), (100, 1000), (4096, 61440), (12345, 1), (1, 1), (32768, 32768),
               (3, 0), (65533, 3), (7, 4097), (16, 16), (60000, 5536)]
@@ -283,7 +305,7 @@ def test_write_blocks_matches_hdd_write(eng, oracle, ref):
     blocks[5] = 0                                                     # a hole with stored CRC 0 (sparse rule)
     stored = np.array([zlib.crc32(b.tobytes()) for b in blocks], dtype=np.uint32)
     stored[5] = 0
-    writes, expect = [], []
+    writes = []
     for i, (off, size) in enumerate(shapes * 3):
         data = rng.integers(0, 256, size, dtype=np.uint8)
         crc = zlib.crc32(data.tobytes())
@@ -294,27 +316,7 @@ def test_write_blocks_matches_hdd_write(eng, oracle, ref):
         if variant == 2 and i % 4 == 1 and exists:
             stored[i] ^= 1                                            # damaged stored block
         writes.append(dict(block=i, offset=off, data=data, crc=crc, exists=exists))
-        # checker: the transcription of hdd_write onto the compiled reference's crc.cc where oracle/_ref exists, else the restatement
-        expect.append(O.hdd_write_block(ref if ref is not None else oracle, blocks[i] if exists else None, int(stored[i]), off, size, crc,
-                                        data if size else np.zeros(1, np.uint8)))
-    before_blocks, before_crc = blocks.copy(), stored.copy()
-    status = eng.write_blocks(blocks, stored, writes)
-    code = {0: 0, -3: L._lib.ERR_CRC, -4: L._lib.ERR_DAMAGED, -1: L._lib.ERR_ARG}
-    seen = set()
-    for i, (rc, blk, new_crc) in enumerate(expect):
-        assert status[i] == code[rc], (i, shapes[i % len(shapes)], status[i], rc)
-        seen.add(rc)
-        if rc == 0:
-            assert (blocks[i] == blk).all() and stored[i] == new_crc, i
-            assert stored[i] == zlib.crc32(blocks[i].tobytes())
-        else:
-            assert (blocks[i] == before_blocks[i]).all() and stored[i] == before_crc[i]
-    assert seen == {0, -3, -4}
-    # argument errors: range outside the block, two writes to one block
-    st = eng.write_blocks(blocks, stored, [dict(block=0, offset=65000, data=np.zeros(1000, np.uint8), crc=0)])
-    assert st == [L._lib.ERR_ARG]
-    with pytest.raises(L.LzGpuError):
-        eng.write_blocks(blocks, stored, [dict(block=1, offset=0, data=np.zeros(4, np.uint8), crc=0), dict(block=1, offset=8, data=np.zeros(4, np.uint8), crc=0)])
+    return blocks, stored, writes, shapes
 
 
 @pytest.mark.parametrize("idx", range(6))

@@ -1,94 +1,92 @@
-"""CPU fuzz (hypothesis): the oracle's restatements against the UNMODIFIED reference on random shapes — slice conversion and
-degraded reads against the reference planners executed in memory (oracle/ref_plans.cc), the hdd_write CRC algebra against zlib.
-Small sizes, bounded example counts, derandomized (the suite must not be flaky): the whole file runs in a few seconds.  A larger
-offline campaign with fresh randomness (3000 conversions, 2000 degraded reads) agreed everywhere when this file was written."""
+"""CPU fuzz: the oracle's restatements against the UNMODIFIED reference on random shapes — slice conversion and degraded reads
+against what the reference planners executed in memory (oracle/ref_plans.cc) returned for a seeded sample of cases
+(tests/golden/reference_outputs.json), the hdd_write CRC algebra against zlib (hypothesis).  Small sizes, bounded example
+counts, derandomized (the suite must not be flaky): the whole file runs in a few seconds.  A larger offline campaign with fresh
+randomness (3000 conversions, 2000 degraded reads) agreed everywhere when this file was written."""
 import zlib
 
 import numpy as np
-import pytest
 from hypothesis import HealthCheck, given, settings
 from hypothesis import strategies as st
 
 from tests import _oracle as O
-from tests.test_oracle_plans import make_slice, ref_sources, true_blocks
+from tests.test_oracle_plans import make_slice, true_blocks
 
 BLOCK = 65536
 
-goals = st.sampled_from([(2, 1, 0), (0, 2, 1), (0, 3, 1), (0, 5, 1), (0, 9, 1), (1, 2, 1), (1, 3, 2), (1, 4, 2), (1, 5, 3), (1, 8, 2), (1, 8, 4),
-                         (1, 6, 5), (1, 21, 4)])
+GOALS = [(2, 1, 0), (0, 2, 1), (0, 3, 1), (0, 5, 1), (0, 9, 1), (1, 2, 1), (1, 3, 2), (1, 4, 2), (1, 5, 3), (1, 8, 2), (1, 8, 4), (1, 6, 5), (1, 21, 4)]
 
 
-@st.composite
-def conversion_case(draw):
-    src = draw(goals)
-    dst = draw(goals)
-    nb = draw(st.integers(1, 14))
-    n_parts = src[1] + src[2]
-    n_lost = draw(st.integers(0, src[2])) if src[0] != 2 else 0
-    lost = tuple(sorted(draw(st.lists(st.integers(0, n_parts - 1), min_size=n_lost, max_size=n_lost, unique=True))))
-    part = draw(st.integers(0, dst[1] + dst[2] - 1))
-    seed = draw(st.integers(0, 1 << 30))
-    return src, dst, nb, lost, part, seed
+def conversion_cases():
+    """250 seeded random conversions: (source goal, destination goal, blocks, lost source parts, destination part, data seed)"""
+    rng = np.random.default_rng(2501)
+    cases = []
+    for _ in range(250):
+        src, dst = GOALS[rng.integers(len(GOALS))], GOALS[rng.integers(len(GOALS))]
+        nb = int(rng.integers(1, 15))
+        n_lost = int(rng.integers(0, src[2] + 1)) if src[0] != 2 else 0
+        lost = tuple(sorted(int(x) for x in rng.choice(src[1] + src[2], size=n_lost, replace=False)))
+        cases.append((src, dst, nb, lost, int(rng.integers(0, dst[1] + dst[2])), int(rng.integers(0, 1 << 30))))
+    return cases
 
 
-@settings(max_examples=250, deadline=None, derandomize=True, suppress_health_check=[HealthCheck.too_slow, HealthCheck.function_scoped_fixture])
-@given(case=conversion_case())
-def test_convert_restatement_vs_reference_planner_random(oracle, ref, case):
-    if ref is None:
-        pytest.skip("compiled reference not available")
-    src, dst, nb, lost, part, seed = case
-    chunk = O.fill_chunk(oracle, nb * BLOCK, seed, 1)
-    parts, crcs = make_slice(oracle, src, chunk)
-    # parts a short chunk does not reach exist on their chunkservers with zero blocks: the reference plans reads of zero bytes
-    # from them, this repository's layout contract passes them as all-zero buffers
-    sources = ref_sources(src, parts, nb, lost)
-    avail = [None if i in lost else p for i, p in enumerate(parts)]
-    nblk = true_blocks(dst, part, nb)
-    if nblk == 0:
-        return
-    want = [0] * (dst[1] + dst[2])
-    want[part] = 1
-    got = O.plan_recover_part(ref, sources, O.slice_type(*dst), O.ref_part_number(dst[0], dst[1], part), 0, nblk)
-    n_avail = sum(a is not None for a in avail)
-    rc, out, ocrc, _ = O.convert_chunk(oracle, src, avail, [None if a is None else c for a, c in zip(avail, crcs)], dst, want, nb)
-    if got is None:
-        # the reference cannot plan this read: too few parts (a short chunk may leave data parts empty)
-        assert n_avail < src[1] or rc != 0
-        return
-    assert rc == 0, (src, dst, nb, lost, part)
-    data, crc = got
-    assert (out[part][: nblk * BLOCK] == data).all(), (src, dst, nb, lost, part)
-    assert not out[part][nblk * BLOCK:].any()
-    assert (ocrc[part][:nblk] == crc).all()
+def degraded_read_cases():
+    """150 seeded random degraded reads: (goal, blocks, lost parts, first block, block count)"""
+    rng = np.random.default_rng(1501)
+    goals = [g for g in GOALS if g[0] != 2]
+    cases = []
+    for _ in range(150):
+        goal = goals[rng.integers(len(goals))]
+        nb = int(rng.integers(1, 21))
+        lost = tuple(int(x) for x in rng.choice(goal[1] + goal[2], size=int(rng.integers(0, goal[2] + 1)), replace=False))
+        first = int(rng.integers(0, nb))
+        cases.append((goal, nb, lost, first, int(rng.integers(1, nb - first + 1))))
+    return cases
 
 
-@settings(max_examples=150, deadline=None, derandomize=True, suppress_health_check=[HealthCheck.too_slow, HealthCheck.function_scoped_fixture])
-@given(goal=goals.filter(lambda g: g[0] != 2), nb=st.integers(1, 20), data=st.data())
-def test_degraded_read_ranges_vs_reference_planner_random(oracle, ref, goal, nb, data):
+def test_convert_restatement_vs_reference_planner_random(oracle):
+    for case, want in zip(conversion_cases(), O.reference_outputs("fuzz_convert"), strict=True):
+        src, dst, nb, lost, part, seed = case
+        chunk = O.fill_chunk(oracle, nb * BLOCK, seed, 1)
+        parts, crcs = make_slice(oracle, src, chunk)
+        avail = [None if i in lost else p for i, p in enumerate(parts)]
+        nblk = true_blocks(dst, part, nb)
+        if nblk == 0:
+            assert want is None
+            continue
+        req = [0] * (dst[1] + dst[2])
+        req[part] = 1
+        n_avail = sum(a is not None for a in avail)
+        rc, out, ocrc, _ = O.convert_chunk(oracle, src, avail, [None if a is None else c for a, c in zip(avail, crcs)], dst, req, nb)
+        if want is None:
+            # the reference cannot plan this read: too few parts (a short chunk may leave data parts empty)
+            assert n_avail < src[1] or rc != 0, case
+            continue
+        assert rc == 0, case
+        assert O.sha256(out[part][: nblk * BLOCK]) == want[0], case
+        assert not out[part][nblk * BLOCK:].any()
+        assert O.crc_sha256(ocrc[part][:nblk]) == want[1], case
+
+
+def test_degraded_read_ranges_vs_reference_planner_random(oracle):
     """any block range of the chunk, any tolerable set of lost parts: the reference's ChunkReadPlanner result is the chunk data"""
-    if ref is None:
-        pytest.skip("compiled reference not available")
-    kind, k, m = goal
-    n_lost = data.draw(st.integers(0, m))
-    lost = tuple(data.draw(st.lists(st.integers(0, k + m - 1), min_size=n_lost, max_size=n_lost, unique=True)))
-    first = data.draw(st.integers(0, nb - 1))
-    count = data.draw(st.integers(1, nb - first))
-    chunk = O.fill_chunk(oracle, nb * BLOCK, 3, nb)
-    parts, _ = make_slice(oracle, goal, chunk)
-    sources = ref_sources(goal, parts, nb, lost)
-    got = O.plan_read_chunk(ref, sources, first, count)
-    if got is None:
-        return
-    assert (got == chunk[first * BLOCK:(first + count) * BLOCK]).all()
-    # and the restatement rebuilds the same parts the plan needed
-    pb = -(-nb // k)
-    avail = [None if i in lost else p for i, p in enumerate(parts)]
-    if sum(a is not None for a in avail) >= k:
-        rc, out, _ = oracle.recover_chunk(kind, k, m, avail, None, [1] * k + [0] * m, pb)
-        assert rc == 0
-        for j in range(k):
-            if avail[j] is None:
-                assert (out[j] == parts[j]).all()
+    for case, want in zip(degraded_read_cases(), O.reference_outputs("fuzz_read"), strict=True):
+        goal, nb, lost, first, count = case
+        if want is None:                    # the reference could not plan this read
+            continue
+        kind, k, m = goal
+        chunk = O.fill_chunk(oracle, nb * BLOCK, 3, nb)
+        assert O.sha256(chunk[first * BLOCK:(first + count) * BLOCK]) == want, case
+        # and the restatement rebuilds the same parts the plan needed
+        parts, _ = make_slice(oracle, goal, chunk)
+        pb = -(-nb // k)
+        avail = [None if i in lost else p for i, p in enumerate(parts)]
+        if sum(a is not None for a in avail) >= k:
+            rc, out, _ = oracle.recover_chunk(kind, k, m, avail, None, [1] * k + [0] * m, pb)
+            assert rc == 0
+            for j in range(k):
+                if avail[j] is None:
+                    assert (out[j] == parts[j]).all(), case
 
 
 @settings(max_examples=300, deadline=None, derandomize=True, suppress_health_check=[HealthCheck.function_scoped_fixture])
