@@ -110,6 +110,32 @@ typedef struct lzgpu_convert_plan {
 } lzgpu_convert_plan;
 int lzgpu_plan_convert(const lzgpu_goal *src, const lzgpu_goal *dst, const uint8_t *available, const uint8_t *want, lzgpu_convert_plan *out);
 
+/* Which kernel lzgpu_recover_chunks* would run for a degraded read (pure host logic, no GPU needed).  available[i]: part i can be
+ * read; want[i]: part i is requested and given an output buffer; verify: a part among the first k available ones carries stored
+ * CRCs; image: the chunk-order image is wanted.  overrides: the LZGPU_RECOVER_TWO, LZGPU_RECOVER_GEO, LZGPU_RECOVER_K3,
+ * LZGPU_BS_RECOVER, LZGPU_BS_RECOVER_GFW and LZGPU_DIRECT_WIDE switches of a context, -1 = automatic (NULL: all automatic).
+ * fused = 1: ONE kernel verifies the inputs, rebuilds the erased data parts and scatters the image; its template arguments are
+ * form (0 = fused_recover_kernel<e, kt, r0, r1, 64, geo, item_words>, 1 = bs_recover3_kernel<kt>, 2 = the DIRECT form
+ * fused_recover_kernel<e, 0, -2, -1, 64, 2, item_words> for Cauchy generators), e, kt (compile-time k, 0 = runtime), r0 / r1
+ * (parity rows known at compile time, -1 = runtime), geo (0: one 9-warp CTA per SM, 1: two, 2: one 16-warp CTA) and item_words.
+ * fused = 0: the generic kernels (gf_dot + CRC + image passes) take the request. */
+typedef struct lzgpu_recover_overrides {
+	int recover_two, recover_geo, recover_k3, bs_recover, bs_recover_gf_warps, direct_wide;
+} lzgpu_recover_overrides;
+typedef struct lzgpu_recover_plan {
+	int fused, form, e, kt, r0, r1, geo, item_words;
+	uint32_t stripes_per_unit, stages, units_per_chunk, units, ctas_per_sm, threads_per_cta, smem_bytes;
+	uint32_t raid6_dbl;    /* e = 2, parity rows 0 and 1 on a runtime-k kernel: doublings for 2^x0 S0 (0xff: a multiply) */
+	uint32_t elim3_dbl;    /* e = 3, parity rows 0, 1, 2: doublings for 2^x0 S0 and 4^x0 S0 (0xff: two multiplies) */
+	uint8_t used[32];      /* slot -> part index: the first k available parts */
+	uint8_t erased[4];     /* erased data parts, ascending */
+	uint8_t par_row[4];    /* generator rows of the parity parts in use, in slot order */
+	uint8_t par_slot[4];
+} lzgpu_recover_plan;
+int lzgpu_plan_recover(const lzgpu_goal *g, const uint8_t *available, const uint8_t *want, int verify, int image, uint32_t n_chunks,
+                       uint32_t nb, size_t part_stride, size_t chunk_out_stride, const lzgpu_recover_overrides *overrides,
+                       lzgpu_recover_plan *out);
+
 /* Diagnostics (pure host logic, no GPU needed): the host build of the bit-plane arithmetic the four-parity-row encoder runs per
  * item (csrc/bitslice.cuh).  data = k columns of 32 bytes (column j = 32 bytes of data part j, k <= 32); parity receives the
  * 4 x 32 bytes of the Vandermonde parity rows 0..3 (coefficient of column j in row r: (2^r)^j, galois_field_isal.cc:53-69). */

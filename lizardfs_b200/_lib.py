@@ -39,6 +39,19 @@ class LzConvertPlan(C.Structure):
                 ("stages", C.c_uint32), ("worker_warps", C.c_uint32), ("rebuild_warps", C.c_uint32), ("smem_bytes", C.c_uint32)]
 
 
+class LzRecoverOverrides(C.Structure):
+    _fields_ = [("recover_two", C.c_int), ("recover_geo", C.c_int), ("recover_k3", C.c_int), ("bs_recover", C.c_int),
+                ("bs_recover_gf_warps", C.c_int), ("direct_wide", C.c_int)]
+
+
+class LzRecoverPlan(C.Structure):
+    _fields_ = [("fused", C.c_int), ("form", C.c_int), ("e", C.c_int), ("kt", C.c_int), ("r0", C.c_int), ("r1", C.c_int), ("geo", C.c_int),
+                ("item_words", C.c_int), ("stripes_per_unit", C.c_uint32), ("stages", C.c_uint32), ("units_per_chunk", C.c_uint32),
+                ("units", C.c_uint32), ("ctas_per_sm", C.c_uint32), ("threads_per_cta", C.c_uint32), ("smem_bytes", C.c_uint32),
+                ("raid6_dbl", C.c_uint32), ("elim3_dbl", C.c_uint32), ("used", C.c_uint8 * 32), ("erased", C.c_uint8 * 4),
+                ("par_row", C.c_uint8 * 4), ("par_slot", C.c_uint8 * 4)]
+
+
 class LzBlockWrite(C.Structure):
     _fields_ = [("block", C.c_uint32), ("offset", C.c_uint32), ("size", C.c_uint32), ("crc", C.c_uint32),
                 ("payload_off", C.c_uint64), ("exists", C.c_uint32), ("status", C.c_int32)]
@@ -54,6 +67,7 @@ SIGNATURES = {
     "lzgpu_goal_valid": (_int, [_goalp]),
     "lzgpu_plan_encode": (_int, [_goalp, _u32, _u32, _sz, _int, _vp]),
     "lzgpu_plan_convert": (_int, [_goalp, _goalp, _vp, _vp, _vp]),
+    "lzgpu_plan_recover": (_int, [_goalp, _vp, _vp, _int, _int, _u32, _u32, _sz, _sz, _vp, _vp]),
     "lzgpu_debug_bitslice_rows": (_int, [_int, _vp, _vp]),
     "lzgpu_debug_bitslice_recover3": (_int, [_int, _vp, _vp, _int, _vp]),
     "lzgpu_goal_slice_type": (_int, [_goalp]),

@@ -21,8 +21,6 @@ struct BsRecoverMasks {
 	uint32_t m[6][64];   // alpha, beta, gamma, delta of the three-unknown elimination (fused_recover_kernel, E = 3); A = 2^a, A^2
 };
 
-constexpr int kBsRecoverThreads = 512;
-
 template <int KT>
 __global__ void __launch_bounds__(kBsRecoverThreads, 1)
 bs_recover3_kernel(const __grid_constant__ TmapArray tmaps, const __grid_constant__ RecoverParams p, const __grid_constant__ BsRecoverMasks mk) {

@@ -24,13 +24,7 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t
 
 // two CTAs per SM: 228 KiB per SM minus 1 KiB reserved per CTA
 constexpr int kSmemCap128 = 226 * 1024;       // FW = 128 variant: one CTA per SM
-constexpr int kRecoverSmemCap = 200 * 1024;  // recover kernel: one CTA per SM, 6 stages
-constexpr int kRecoverSmemCap2 = 100 * 1024; // two CTAs per SM, 3 stages (E <= 2)
-constexpr int kRecoverSmemCapBig = 208 * 1024; // one 16-warp CTA per SM (GEO 2)
-
-#ifndef LZ_BS_RECOVER_DEFAULT
-#define LZ_BS_RECOVER_DEFAULT 1
-#endif
+// (the degraded read's shared-memory caps kRecoverSmemCap*: fused_plan.h)
 
 struct FusedState {
 	EncodeTiledFn encode_tiled = nullptr;
@@ -89,8 +83,8 @@ static int set_recover_attr() {
 	return LZGPU_OK;
 }
 
-// wide items of the DIRECT degraded read: 16 bytes for one rebuilt part, 8 for more (e x 4 accumulators next to the CRC window spill at 128 registers)
-template <int E> constexpr int kDirectWide = E >= 2 ? 2 : 4;
+// wide items of the DIRECT degraded read (recover_direct_wide_words, fused_plan.h)
+template <int E> constexpr int kDirectWide = recover_direct_wide_words(E);
 template <int E>
 static int set_direct_attr() {
 	CUDA_TRY(cudaFuncSetAttribute(fused_recover_kernel<E, 0, kRecoverDirect, -1, 64, 2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kRecoverSmemCapBig));
@@ -644,109 +638,41 @@ int lz_fused_recover(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chunks, 
 	*verifying = false;
 	if (!fs || fs->disabled) return LZGPU_NOT_HANDLED;
 	const int K = goal->k, M = goal->m, N = K + M;
-	const bool direct = lz::uses_cauchy(K, M);   // no Horner syndromes for a Cauchy generator: general rows over the k inputs
-	if (direct && fs->direct_wide == -2) return LZGPU_NOT_HANDLED;   // LZGPU_DIRECT_WIDE=-2: A/B against the generic route
-	const bool direct_forced = direct && fs->direct_wide >= 0;
-	if ((part_stride % 16) || (chunk_out_stride % 16)) return LZGPU_NOT_HANDLED;
-	// inputs: the first k available parts (ec_read_plan.h:126-133)
-	int used[LZGPU_MAX_DATA], n_used = 0;
-	for (int i = 0; i < N && n_used < K; ++i)
-		if (d_parts[i]) used[n_used++] = i;
-	if (n_used < K) return LZGPU_NOT_HANDLED;
+	// the route: instantiation, geometry, parity rows and erased parts (fused_plan.h recover_plan, unit-tested on the CPU)
+	uint8_t avail[LZGPU_MAX_PARTS] = {0}, wanted[LZGPU_MAX_PARTS] = {0};
+	for (int i = 0; i < N; ++i) {
+		avail[i] = d_parts[i] ? 1 : 0;
+		wanted[i] = want[i] && d_out && d_out[i];
+	}
+	bool any_crc = false;
+	for (int i = 0, n_used = 0; i < N && n_used < K; ++i)
+		if (d_parts[i]) { any_crc |= d_part_crc && d_part_crc[i]; ++n_used; }
+	RecoverOverrides ov;
+	ov.recover_two = fs->recover_two;
+	ov.recover_geo = fs->recover_geo;
+	ov.recover_k3 = fs->recover_k3;
+	ov.bs_recover = fs->bs_recover;
+	ov.bs_recover_gf_warps = fs->bs_recover_gf_warps;
+	ov.direct_wide = fs->direct_wide;
+	const RecoverPlan pl = recover_plan(K, M, lz::uses_cauchy(K, M), avail, wanted, any_crc, d_chunk_out != nullptr, nb, n_chunks, part_stride,
+	                                    chunk_out_stride, ov);
+	if (!pl.ok) return LZGPU_NOT_HANDLED;
+	const bool direct = pl.form == kRecoverDirectForm;
+	const uint32_t e = pl.e;
 	RecoverParams p{};
-	std::memset(p.slot_of_data, 0xff, sizeof(p.slot_of_data));
-	uint32_t e = 0, n_par = 0;
+	std::memcpy(p.slot_of_data, pl.slot_of_data, sizeof(p.slot_of_data));
+	std::memcpy(p.erased_idx, pl.erased_idx, sizeof(p.erased_idx));
+	std::memcpy(p.par_slot, pl.par_slot, sizeof(p.par_slot));
+	std::memcpy(p.par_row, pl.par_row, sizeof(p.par_row));
 	for (int a = 0; a < K; ++a) {
-		const int idx = used[a];
+		const int idx = pl.used[a];
 		p.part_id[a] = static_cast<uint8_t>(idx);
 		p.data_of_slot[a] = idx < K ? static_cast<uint8_t>(idx) : 0xff;
-		if (idx < K) p.slot_of_data[idx] = static_cast<uint8_t>(a);
-		else if (n_par < 4) { p.par_slot[n_par] = static_cast<uint8_t>(a); p.par_row[n_par] = static_cast<uint8_t>(idx - K); ++n_par; }
-		else return LZGPU_NOT_HANDLED;
 	}
-	for (int j = 0; j < K; ++j)
-		if (p.slot_of_data[j] == 0xff) {
-			if (e >= 4) return LZGPU_NOT_HANDLED;
-			p.erased_idx[e++] = static_cast<uint8_t>(j);
-		}
-	if (e == 0 || e != n_par) return LZGPU_NOT_HANDLED;
-	// Measured (profiles/sweep_r2.md, run 8): with general coefficients the rebuild is bound by the bit-plane multiplies, not by HBM, and
-	// the grid-stride gf_dot_kernel (full occupancy, no stage barriers) does e >= 2 rows faster than this kernel's 16 warps per SM
-	// even though it needs separate CRC and image passes: ec(8,6) three lost 2.7 ms against 6.2 ms per 64 chunks.  One lost part
-	// (ec(8,6): 2.45 ms against 3.98 with verification and image), and two lost parts when the call verifies and wants the image
-	// (ec(4,5) 4.39 against 4.87, ec(21,4) 5.05 against 5.38), stay here.
-	if (direct && !direct_forced && !(e == 1 || (e == 2 && d_part_crc && d_chunk_out))) return LZGPU_NOT_HANDLED;
-	// every requested missing part must be a data part
-	for (int i = K; i < N; ++i)
-		if (want[i] && !d_parts[i] && d_out && d_out[i]) return LZGPU_NOT_HANDLED;
-	// geometry: even G (1024-byte aligned slot regions), K*G*4 rows <= 256
-	// Two CTAs per SM with a 3-stage ring, or one CTA with 6 stages?  Measured on the same box (64 MiB chunks, fraction of
-	// the HBM copy peak, two / one):  ec(3,2) 2 lost 0.48 / 0.42 (+image 0.64 / 0.58),  xor3 1 lost 0.93 / 0.70 (+image
-	// 0.73 / 0.77),  ec(8,2) 2 lost 0.66 / 0.70 (+image 0.72 / 0.78),  ec(8,2) 1 lost 0.94 / 0.99.  So: the runtime-k
-	// shapes, except the single-erasure case that also writes the image.  LZGPU_RECOVER_TWO=0|1 forces either.
-	const bool two_auto = K != 8 && (e == 2 || (e == 1 && !d_chunk_out));
-	const bool two = e <= 2 && (fs->recover_two < 0 ? two_auto : fs->recover_two != 0);
-	// Measured (profiles/sweep_r2.md, fraction of the HBM peak, recover only / verify + image): the 16-warp CTA wins for the
-	// runtime-k shapes with two or more erased parts — ec(3,2) two lost 0.69 / 0.69 against 0.52 / 0.67 on two 9-warp CTAs, ec(5,3)
-	// three lost 0.29 / 0.42 against 0.23 / 0.32 and two lost 0.59 / 0.74 against 0.46 / 0.65 on one — while the k = 8 instantiation
-	// keeps one 9-warp CTA with six stages (two lost: 0.81 with verification and image against 0.70).  LZGPU_RECOVER_GEO=0|1|2 forces one.
-	int geo = fs->recover_geo >= 0 ? fs->recover_geo : (K != 8 && e >= 2) ? 2 : (two ? 1 : 0);
-	if (direct) geo = 2;
-	if (geo == 1 && e > 2) geo = 0;
-	// three lost data parts with parity rows 0, 1, 2 in use: bit planes + dedicated GF warps (bs_recover_kernel.cuh) — geometry: G even,
-	// the 16 G items of a step on the last ceil(16 G / 32) warps, the k G 4 input rows on the warps before them when the call verifies
-	// stored CRCs (no stream warps otherwise), one TMA box per part (G 4 <= 256 rows), at least three stages
-	bool bs3 = !direct && e == 3 && fs->bs_recover && p.par_row[0] == 0 && p.par_row[1] == 1 && p.par_row[2] == 2;
-	uint32_t G = 0, n_stages = 0;
-	if (bs3) {
-		// Run 33 (fraction of the HBM peak, at most four / at most eight GF warps): rebuild only — no stream warps, G = 16, eight GF warps —
-		// ec(5,3) 0.440 / 0.682, ec(6,3) 0.388 / 0.628, ec(8,3) 0.452 / 0.648; with verification and image ec(5,3) 0.589 / 0.722 (seven GF
-		// warps), ec(6,3) 0.570 / 0.640 (six), but ec(8,3) 0.689 / 0.658 (five: one scheduler gets two of them).  So: the largest G, unless
-		// it only buys a fifth GF warp.
-		bool any_crc = false;
-		for (int a = 0; a < K; ++a) any_crc |= d_part_crc && d_part_crc[used[a]];
-		uint32_t g4 = 0;
-		for (uint32_t g = 2; g <= 64; g += 2) {
-			const size_t stage = static_cast<size_t>(K) * g * 4 * kStepBytes;
-			const uint32_t gf_warps = (16 * g + 31) / 32, stream_warps = any_crc ? (K * g * 4 + 31) / 32 : 0;
-			if (gf_warps > static_cast<uint32_t>(fs->bs_recover_gf_warps) || gf_warps + stream_warps > kBsRecoverThreads / 32 || 3 * stage + 256 > static_cast<size_t>(kRecoverSmemCapBig)) break;
-			G = g;
-			if (gf_warps <= 4) g4 = g;
-		}
-		if (G && g4 && (16 * G + 31) / 32 == 5) G = g4;
-		if (G) n_stages = static_cast<uint32_t>(std::min<size_t>(6, (kRecoverSmemCapBig - 256) / (static_cast<size_t>(K) * G * 4 * kStepBytes)));
-		else bs3 = false;
-	}
-	if (bs3) {
-		// (geometry chosen above)
-	} else if (geo == 2) {
-		// one 16-warp CTA: the largest G whose K*G*4 input rows fit 512 threads (one TMA box per part: G*4 <= 256 rows) and whose
-		// 32*G items fill whole rounds of the CTA (G a multiple of 16) where K allows, with at least three stages in 200 KiB
-		uint32_t best = 0, best16 = 0;
-		for (uint32_t g = 2; g <= 64; g += 2) {
-			const uint32_t rows = K * g * 4;
-			if (rows > 512 || 3 * static_cast<size_t>(rows) * kStepBytes + 256 > kRecoverSmemCapBig) break;
-			best = g;
-			if (g % 16 == 0) best16 = g;
-		}
-		G = best16 ? best16 : best;
-		if (G) n_stages = static_cast<uint32_t>(std::min<size_t>(6, (kRecoverSmemCapBig - 256) / (static_cast<size_t>(K) * G * 4 * kStepBytes)));
-	} else {
-		n_stages = static_cast<uint32_t>(recover_stages(geo));
-		const size_t smem_cap = geo == 1 ? kRecoverSmemCap2 : kRecoverSmemCap;
-		for (uint32_t g = 2; g <= 64; g += 2) {
-			const uint32_t rows = K * g * 4;
-			if (rows > kMaxRows || static_cast<size_t>(n_stages) * rows * kStepBytes + 256 > smem_cap) break;
-			G = g;
-		}
-	}
-	if (G == 0) return LZGPU_NOT_HANDLED;
-	const uint32_t pb = (nb + K - 1) / K;
 	for (uint32_t x = 0; x < e; ++x) {
 		const int j = p.erased_idx[x];
 		void *o = d_out ? d_out[j] : nullptr;
-		p.out[x] = (want[j] || d_chunk_out) ? static_cast<uint8_t *>(o) : nullptr;
-		if (!p.out[x] && !d_chunk_out) {}  // nothing requested for this part: still solved (cheap), not stored
+		p.out[x] = (want[j] || d_chunk_out) ? static_cast<uint8_t *>(o) : nullptr;   // nothing requested for a part: still solved (cheap), not stored
 	}
 	p.image = static_cast<uint8_t *>(d_chunk_out);
 	p.out_stride = part_stride;
@@ -755,15 +681,15 @@ int lz_fused_recover(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chunks, 
 	p.first_bad = d_first_bad;
 	p.n_chunks = n_chunks;
 	p.nb = nb;
-	p.pb = pb;
+	p.pb = pl.pb;
 	p.K = K;
-	p.G = G;
-	p.units_per_chunk = (pb + G - 1) / G;
-	const uint64_t total = static_cast<uint64_t>(p.units_per_chunk) * n_chunks;
-	if (total > 0x7fffffffull) return LZGPU_NOT_HANDLED;
-	p.total_units = static_cast<uint32_t>(total);
+	p.G = pl.G;
+	p.units_per_chunk = pl.units_per_chunk;
+	p.total_units = pl.total_units;
 	p.e = e;
-	p.n_stages = n_stages;
+	p.n_stages = pl.n_stages;
+	p.raid6_dbl = pl.raid6_dbl;
+	p.elim3_dbl = pl.elim3_dbl;
 #ifdef LZ_ENABLE_FOLD128
 	std::memcpy(p.qmult, fs->fold == 128 ? fs->qmult128 : fs->qmult64, sizeof(p.qmult));
 #else
@@ -771,39 +697,30 @@ int lz_fused_recover(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chunks, 
 #endif
 	p.zconst = lz::crc_of_zeros(LZGPU_BLOCK_SIZE);
 	for (int a = 0; a < K; ++a) {
-		p.stored[a] = d_part_crc ? static_cast<const uint32_t *>(d_part_crc[used[a]]) : nullptr;
+		p.stored[a] = d_part_crc ? static_cast<const uint32_t *>(d_part_crc[pl.used[a]]) : nullptr;
 		if (p.stored[a]) *verifying = true;
 	}
-	// V[r][x] = (2^row_r)^(erased_x); W = V^-1
-	uint8_t V[16], W[16];
-	for (uint32_t r = 0; r < e; ++r) {
-		uint8_t gen = 1;
-		for (int t = 0; t < p.par_row[r]; ++t) gen = lz::gf_mul_host(gen, 2);
-		for (uint32_t x = 0; x < e; ++x) {
-			uint8_t v = 1;
-			for (int t = 0; t < p.erased_idx[x]; ++t) v = lz::gf_mul_host(v, gen);
-			V[r * e + x] = v;
-		}
-	}
-	if (!direct && gf_invert_matrix(V, W, static_cast<int>(e)) != 0) return LZGPU_NOT_HANDLED;  // generic path reports the singular case
-	if (direct) {
+	// W = V^-1 (the plan has checked that V is invertible)
+	uint8_t V[16], W[16] = {0};
+	if (!direct) {
+		recover_syndrome_matrix(p.par_row, p.erased_idx, e, V);
+		if (gf_invert_matrix(V, W, static_cast<int>(e)) != 0) return LZGPU_NOT_HANDLED;
+	} else {
 		// rows of the reference's inverted k x k system for the erased data parts, over the k used parts in slot order
-		uint8_t erased_flags[LZGPU_MAX_PARTS] = {0}, wanted[LZGPU_MAX_PARTS] = {0}, rows[LZGPU_MAX_PARITY * LZGPU_MAX_DATA];
+		uint8_t erased_flags[LZGPU_MAX_PARTS] = {0}, wanted_rows[LZGPU_MAX_PARTS] = {0}, rows[LZGPU_MAX_PARITY * LZGPU_MAX_DATA];
 		for (int i = 0; i < N; ++i) erased_flags[i] = 1;
-		for (int a = 0; a < K; ++a) erased_flags[used[a]] = 0;
-		for (uint32_t x = 0; x < e; ++x) wanted[p.erased_idx[x]] = 1;
+		for (int a = 0; a < K; ++a) erased_flags[pl.used[a]] = 0;
+		for (uint32_t x = 0; x < e; ++x) wanted_rows[p.erased_idx[x]] = 1;
 		bool singular = false;
-		if (lz::rs_recovery_matrix(K, M, erased_flags, wanted, rows, &singular) != static_cast<int>(e)) return LZGPU_NOT_HANDLED;
+		if (lz::rs_recovery_matrix(K, M, erased_flags, wanted_rows, rows, &singular) != static_cast<int>(e)) return LZGPU_NOT_HANDLED;
 		for (uint32_t x = 0; x < e; ++x)   // rs_recovery_matrix emits its rows in ascending part order = erased_idx order
 			for (int a = 0; a < K; ++a) coef_planes_set(p.rw[x * 32 + a], rows[x * K + a]);
-		std::memset(W, 0, sizeof(W));
 	}
 	for (uint32_t x = 0; x < e; ++x)
 		for (uint32_t r = 0; r < e; ++r) {
 			coef_planes_set(p.w[x * 4 + r], W[x * e + r]);
 		}
-	p.raid6_dbl = 0xffu;
-	const bool k8 = K == 8 && (G == 8 || geo == 2);
+	const bool k8 = K == 8 && (pl.G == 8 || pl.geo == 2);
 	if (e == 2 && p.par_row[0] == 0 && p.par_row[1] == 1 && !k8) {
 		// RAID-6 shape on a runtime-k instantiation: w[0] = planes of 2^x0, w[1] = planes of (2^x0 ^ 2^x1)^-1 (see the kernel)
 		uint8_t gx0 = 1, gx1 = 1;
@@ -811,107 +728,79 @@ int lz_fused_recover(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chunks, 
 		for (int t = 0; t < p.erased_idx[1]; ++t) gx1 = lz::gf_mul_host(gx1, 2);
 		coef_planes_set(p.w[0], gx0);
 		coef_planes_set(p.w[1], lz::gf_inv_host(gx0 ^ gx1));
-		if (p.erased_idx[0] <= 4) p.raid6_dbl = p.erased_idx[0];
 	}
-	// "rows 0, 1, .., e-1 in use" (the first e parity parts are the available ones — the common case): instantiations that
-	// multiply row r by 2^r in one step
-	bool consecutive = true;
-	for (uint32_t r = 0; r < e; ++r) consecutive &= p.par_row[r] == r;
-	p.elim3_dbl = 0xffu;
-	if (e == 3 && consecutive) {
-		// three unknowns, parity rows 0, 1, 2: the elimination of the kernel comment (w[0..3] = alpha, beta, gamma, delta; w[4], w[5]
-		// = 2^a, 4^a when a > 3).  p, q, p^q are non-zero because 2 has order 255 and the positions differ by less than 32.
+	// the constants of the three-unknown elimination, parity rows 0, 1, 2 (see the kernel comment): alpha, beta, gamma, delta, A = 2^a,
+	// A^2.  p, q, p^q are non-zero because 2 has order 255 and the positions differ by less than 32.
+	uint8_t elim[6] = {0};
+	if (e == 3 && p.par_row[0] == 0 && p.par_row[1] == 1 && p.par_row[2] == 2) {
 		auto pw2 = [](int t) { uint8_t v = 1; for (int i = 0; i < t; ++i) v = lz::gf_mul_host(v, 2); return v; };
 		const uint8_t A = pw2(p.erased_idx[0]), B = pw2(p.erased_idx[1]), C = pw2(p.erased_idx[2]);
 		const uint8_t pp = A ^ B, qq = A ^ C;
 		const uint8_t alpha = lz::gf_inv_host(lz::gf_mul_host(qq, pp ^ qq)), beta = lz::gf_mul_host(pp, alpha);
 		const uint8_t gamma = lz::gf_inv_host(pp), delta = lz::gf_mul_host(qq, gamma);
-		coef_planes_set(p.w[0], alpha);
-		coef_planes_set(p.w[1], beta);
-		coef_planes_set(p.w[2], gamma);
-		coef_planes_set(p.w[3], delta);
-		coef_planes_set(p.w[4], A);
-		coef_planes_set(p.w[5], lz::gf_mul_host(A, A));
-		if (p.erased_idx[0] <= 3) p.elim3_dbl = p.erased_idx[0];
+		const uint8_t c6[6] = {alpha, beta, gamma, delta, A, lz::gf_mul_host(A, A)};
+		std::memcpy(elim, c6, sizeof(elim));
+		for (int i = 0; i < 6; ++i) coef_planes_set(p.w[i], elim[i]);
 	}
 	TmapArray maps;
 	for (int a = 0; a < K; ++a) {
-		const cuuint64_t dims[3] = {static_cast<cuuint64_t>(kRowBytes), static_cast<cuuint64_t>(pb) * 4, n_chunks};
+		const cuuint64_t dims[3] = {static_cast<cuuint64_t>(kRowBytes), static_cast<cuuint64_t>(pl.pb) * 4, n_chunks};
 		const cuuint64_t strides[2] = {static_cast<cuuint64_t>(kRowBytes), part_stride};
-		const cuuint32_t box[3] = {kStepBytes, G * 4, 1};
+		const cuuint32_t box[3] = {kStepBytes, pl.G * 4, 1};
 		const cuuint32_t estr[3] = {1, 1, 1};
-		CUresult r = fs->encode_tiled(&maps.m[a], CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void *>(d_parts[used[a]]), dims, strides, box, estr,
+		CUresult r = fs->encode_tiled(&maps.m[a], CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void *>(d_parts[pl.used[a]]), dims, strides, box, estr,
 		                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, static_cast<CUtensorMapL2promotion>(fs->promo),
 		                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
 		if (r != CUDA_SUCCESS) return LZGPU_NOT_HANDLED;
 	}
 	if (*verifying && !d_first_bad) return LZGPU_NOT_HANDLED;  // (callers that pass stored CRCs always pass the result word, initialised to ~0)
-	const size_t smem = static_cast<size_t>(n_stages) * K * G * 4 * kStepBytes + 16 * n_stages + 64;
-	const bool row0 = p.par_row[0] == 0, row01 = e >= 2 && consecutive;
-	if (bs3) {
-		// the six constants of the elimination (computed above for the packed-word kernel) as 8 x 8 bit matrices of all-ones / zero words
+	const size_t smem = pl.smem;
+	if (pl.form == kRecoverBs3) {
+		// the six constants of the elimination as 8 x 8 bit matrices of all-ones / zero words
 		BsRecoverMasks mk;
-		auto pw2 = [](int t) { uint8_t v = 1; for (int i = 0; i < t; ++i) v = lz::gf_mul_host(v, 2); return v; };
-		const uint8_t A = pw2(p.erased_idx[0]), B = pw2(p.erased_idx[1]), C = pw2(p.erased_idx[2]);
-		const uint8_t pp = A ^ B, qq = A ^ C;
-		const uint8_t alpha = lz::gf_inv_host(lz::gf_mul_host(qq, pp ^ qq)), beta = lz::gf_mul_host(pp, alpha);
-		const uint8_t gamma = lz::gf_inv_host(pp), delta = lz::gf_mul_host(qq, gamma);
-		bs_mask_set(mk.m[0], alpha);
-		bs_mask_set(mk.m[1], beta);
-		bs_mask_set(mk.m[2], gamma);
-		bs_mask_set(mk.m[3], delta);
-		bs_mask_set(mk.m[4], A);
-		bs_mask_set(mk.m[5], lz::gf_mul_host(A, A));
+		for (int i = 0; i < 6; ++i) bs_mask_set(mk.m[i], elim[i]);
 		const int grid = static_cast<int>(std::min<uint64_t>(p.total_units, static_cast<uint64_t>(ctx->sm_count)));
-		if (K == 5) bs_recover3_kernel<5><<<grid, kBsRecoverThreads, smem, st>>>(maps, p, mk);
-		else if (K == 8) bs_recover3_kernel<8><<<grid, kBsRecoverThreads, smem, st>>>(maps, p, mk);
+		if (pl.KT == 5) bs_recover3_kernel<5><<<grid, kBsRecoverThreads, smem, st>>>(maps, p, mk);
+		else if (pl.KT == 8) bs_recover3_kernel<8><<<grid, kBsRecoverThreads, smem, st>>>(maps, p, mk);
 		else bs_recover3_kernel<0><<<grid, kBsRecoverThreads, smem, st>>>(maps, p, mk);
 		CUDA_TRY(cudaGetLastError());
 		ctx->stats.kernel_launches++;
 		return LZGPU_OK;
 	}
 	if (direct) {
-		// item width: 16-byte items leave most of the 16 warps without work when k is large (G small)
-		// run 8: the 8 / 16-byte items win on every shape (ec(32,4) four lost: 12.0 ms against 38.0 per 64 chunks); 4-byte items stay for A/B
-		const bool wide = fs->direct_wide >= 0 ? fs->direct_wide != 0 : true;
-		switch (e) {
+		const bool wide = pl.item_words != 1;
+		switch (pl.E) {
 			case 1: return launch_direct<1>(ctx, maps, p, smem, st, wide);
 			case 2: return launch_direct<2>(ctx, maps, p, smem, st, wide);
 			case 3: return launch_direct<3>(ctx, maps, p, smem, st, wide);
 			default: return launch_direct<4>(ctx, maps, p, smem, st, wide);
 		}
 	}
-	// ec(3,2) / ec(5,3) on the 16-warp geometry: compile-time k (the walk over the columns unrolls, parameter loads become immediates).
-	// Measured (run 18): ec(3,2) two lost, rebuild only 0.689 -> 0.827 of the HBM peak; with verification and image 0.692 -> 0.703.
-	if (K == 3 && geo == 2 && fs->recover_k3) {
-		if (e == 1 && row0) return launch_recover_geo2<1, 3, 0, -1>(ctx, maps, p, smem, st);
-		if (e == 2 && row01) return launch_recover_geo2<2, 3, 0, 1>(ctx, maps, p, smem, st);
-	}
-	// ec(5,3) (run 19): two lost, rebuild only 0.585 -> 0.682 but with verification and image 0.749 -> 0.717 (the unrolled walk costs the CRC
-	// role registers), so that combination keeps the runtime-k kernel; three lost 0.329 -> 0.373 and 0.471 -> 0.519
-	if (K == 5 && geo == 2 && fs->recover_k3) {
-		if (e == 2 && row01 && !(*verifying && d_chunk_out)) return launch_recover_geo2<2, 5, 0, 1>(ctx, maps, p, smem, st);
-		if (e == 3 && row01) return launch_recover_geo2<3, 5, 0, 1>(ctx, maps, p, smem, st);
-	}
-	// ec(4,2), ec(6,2), ec(6,3): the same rule as for k = 5
-	if (K == 4 && geo == 2 && fs->recover_k3 && e == 2 && row01 && !(*verifying && d_chunk_out)) return launch_recover_geo2<2, 4, 0, 1>(ctx, maps, p, smem, st);
-	if (K == 6 && geo == 2 && fs->recover_k3) {
-		if (e == 2 && row01 && !(*verifying && d_chunk_out)) return launch_recover_geo2<2, 6, 0, 1>(ctx, maps, p, smem, st);
-		if (e == 3 && row01) return launch_recover_geo2<3, 6, 0, 1>(ctx, maps, p, smem, st);
-	}
-	switch (e) {
+	// compile-time k other than 8 (the 16-warp geometry only)
+#define LZ_GEO2(EE, KK, R1_) \
+	if (pl.E == EE && pl.KT == KK) return launch_recover_geo2<EE, KK, 0, R1_>(ctx, maps, p, smem, st);
+	LZ_GEO2(1, 3, -1)
+	LZ_GEO2(2, 3, 1)
+	LZ_GEO2(2, 4, 1)
+	LZ_GEO2(2, 5, 1)
+	LZ_GEO2(3, 5, 1)
+	LZ_GEO2(2, 6, 1)
+	LZ_GEO2(3, 6, 1)
+#undef LZ_GEO2
+	const bool r01 = pl.R0 == 0 && pl.R1 == 1, r0 = pl.R0 == 0;
+	switch (pl.E) {
 		case 1:
-			if (row0) return k8 ? launch_recover<1, 8, 0>(ctx, maps, p, smem, st, geo) : launch_recover<1, 0, 0>(ctx, maps, p, smem, st, geo);
-			return launch_recover<1, 0>(ctx, maps, p, smem, st, geo);
+			if (r0) return pl.KT == 8 ? launch_recover<1, 8, 0>(ctx, maps, p, smem, st, pl.geo) : launch_recover<1, 0, 0>(ctx, maps, p, smem, st, pl.geo);
+			return launch_recover<1, 0>(ctx, maps, p, smem, st, pl.geo);
 		case 2:
-			if (row01) return k8 ? launch_recover<2, 8, 0, 1>(ctx, maps, p, smem, st, geo) : launch_recover<2, 0, 0, 1>(ctx, maps, p, smem, st, geo);
-			return launch_recover<2, 0>(ctx, maps, p, smem, st, geo);
+			if (r01) return pl.KT == 8 ? launch_recover<2, 8, 0, 1>(ctx, maps, p, smem, st, pl.geo) : launch_recover<2, 0, 0, 1>(ctx, maps, p, smem, st, pl.geo);
+			return launch_recover<2, 0>(ctx, maps, p, smem, st, pl.geo);
 		case 3:
-			if (row01) return launch_recover<3, 0, 0, 1>(ctx, maps, p, smem, st, geo);
-			return launch_recover<3, 0>(ctx, maps, p, smem, st, geo);
+			if (r01) return launch_recover<3, 0, 0, 1>(ctx, maps, p, smem, st, pl.geo);
+			return launch_recover<3, 0>(ctx, maps, p, smem, st, pl.geo);
 		default:
-			if (row01) return launch_recover<4, 0, 0, 1>(ctx, maps, p, smem, st, geo);
-			return launch_recover<4, 0>(ctx, maps, p, smem, st, geo);
+			if (r01) return launch_recover<4, 0, 0, 1>(ctx, maps, p, smem, st, pl.geo);
+			return launch_recover<4, 0>(ctx, maps, p, smem, st, pl.geo);
 	}
 }
 

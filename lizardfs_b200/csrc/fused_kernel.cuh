@@ -716,14 +716,7 @@ struct RecoverParams {
 // GEO 2 ("big"): ONE 16-warp CTA per SM (512 threads x 128 registers fill the register file), G chosen so that the K*G*4 input rows
 // and the 32*G items both fill whole warps (ec(8,2): G = 16 -> every thread owns one row and one item), ring depth at run time.
 // Twice the resident warps of GEO 0 and, unlike GEO 1, room for the solve's registers.
-__host__ __device__ constexpr int recover_stages(int geo) { return geo == 1 ? 3 : 6; }
-__host__ __device__ constexpr int recover_threads(int geo) { return geo == 2 ? 512 : kFusedThreads; }
-
-#ifndef LZ_RW3
-#define LZ_RW3 2   // words per GF item for three or four erased parts on the 16-warp geometry (narrower items = fewer live accumulators)
-#endif
-__host__ __device__ constexpr int recover_item_words(int e, int geo) { return (geo == 2 && e >= 3) ? LZ_RW3 : 4; }
-constexpr int kRecoverDirect = -2;   // value of R0 that selects the DIRECT form (4-byte items on the 16-warp geometry: k > 20 leaves G = 4)
+// (recover_stages, recover_threads, recover_item_words, kRecoverDirect: fused_plan.h, next to the host's route decision)
 
 // the elimination forms end their item with `continue` under a template-constant condition: the general solve below them is
 // dead code in those instantiations (warning 128)

@@ -5,6 +5,8 @@
 #include <cstddef>
 #include <cstdint>
 
+#include "host_math.h"
+
 #ifndef __CUDACC__
 #define LZ_HD
 #else
@@ -256,6 +258,242 @@ inline ConvertPlan convert_plan(int Ks, int Ms, bool src_cauchy, int Kd, int Md,
 			pl.smem = ns * stage + 24 * ns + fixed;
 		}
 	}
+	return pl;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Fused degraded read (fused_recover_kernel in fused_kernel.cuh, bs_recover3_kernel in bs_recover_kernel.cuh): which instantiation a
+// request reaches and its geometry, as a pure function shared by lz_fused_recover and lzgpu_plan_recover.
+// ---------------------------------------------------------------------------------------------------
+constexpr int kRecoverSmemCap = 200 * 1024;    // geometry 0: one 9-warp CTA per SM, 6 stages
+constexpr int kRecoverSmemCap2 = 100 * 1024;   // geometry 1: two 9-warp CTAs per SM, 3 stages (E <= 2)
+constexpr int kRecoverSmemCapBig = 208 * 1024; // geometry 2: one 16-warp CTA per SM (also the DIRECT form and bs_recover3_kernel)
+constexpr int kBsRecoverThreads = 512;
+LZ_HD constexpr int recover_stages(int geo) { return geo == 1 ? 3 : 6; }
+LZ_HD constexpr int recover_threads(int geo) { return geo == 2 ? 512 : kFusedThreads; }
+#ifndef LZ_RW3
+#define LZ_RW3 2   // words per GF item for three or four erased parts on the 16-warp geometry (narrower items = fewer live accumulators)
+#endif
+LZ_HD constexpr int recover_item_words(int e, int geo) { return (geo == 2 && e >= 3) ? LZ_RW3 : 4; }
+constexpr int kRecoverDirect = -2;   // value of R0 that selects the DIRECT form (4-byte items on the 16-warp geometry: k > 20 leaves G = 4)
+// wide items of the DIRECT degraded read: 16 bytes for one rebuilt part, 8 for more (e x 4 accumulators next to the CRC window spill at 128 registers)
+LZ_HD constexpr int recover_direct_wide_words(int e) { return e >= 2 ? 2 : 4; }
+#ifndef LZ_BS_RECOVER_DEFAULT
+#define LZ_BS_RECOVER_DEFAULT 1
+#endif
+
+// The environment switches of a context (fused.cu lz_fused_init); -1 = automatic.  recover_two: LZGPU_RECOVER_TWO (0 one CTA per SM,
+// 1 two for e <= 2); recover_geo: LZGPU_RECOVER_GEO (0, 1, 2); recover_k3: LZGPU_RECOVER_K3 (0 = runtime-k kernels for k = 3..6);
+// bs_recover: LZGPU_BS_RECOVER (0 = packed-word kernel for three lost parts); bs_recover_gf_warps: LZGPU_BS_RECOVER_GFW (most GF warps
+// of bs_recover3_kernel, 1..16, default 8); direct_wide: LZGPU_DIRECT_WIDE (0 = 4-byte items, 1 = wide items, -2 = DIRECT route off).
+struct RecoverOverrides {
+	int recover_two = -1, recover_geo = -1, recover_k3 = -1, bs_recover = -1, bs_recover_gf_warps = -1, direct_wide = -1;
+};
+
+enum RecoverForm { kRecoverPacked = 0, kRecoverBs3 = 1, kRecoverDirectForm = 2 };
+
+// ok = false: the generic kernels take the request.  Otherwise the instantiation, as its template arguments:
+//   form kRecoverPacked      fused_recover_kernel<E, KT, R0, R1, 64, geo, item_words>
+//   form kRecoverBs3         bs_recover3_kernel<KT> (E = 3, parity rows 0, 1, 2; item_words = 8: 32-byte items on bit planes)
+//   form kRecoverDirectForm  fused_recover_kernel<E, 0, kRecoverDirect, -1, 64, 2, item_words>
+struct RecoverPlan {
+	bool ok = false;
+	int form = kRecoverPacked, E = 0, KT = 0, R0 = -1, R1 = -1, geo = 0, item_words = 0;
+	uint32_t G = 0, n_stages = 0, pb = 0, units_per_chunk = 0, total_units = 0, ctas_per_sm = 0, threads = 0;
+	size_t smem = 0;
+	uint32_t raid6_dbl = 0xffu, elim3_dbl = 0xffu;
+	uint32_t e = 0;
+	uint8_t used[32] = {0};          // slot a -> part index (the first k available parts)
+	uint8_t slot_of_data[32] = {0};  // data index j -> slot, 0xff = erased
+	uint8_t erased_idx[4] = {0};     // data index of erased part x, ascending
+	uint8_t par_slot[4] = {0}, par_row[4] = {0};  // parity parts in use: slot and generator row
+};
+
+// V[r][x] = (2^row_r)^(erased_x): the syndrome system of the Vandermonde generator for the erased data parts
+inline void recover_syndrome_matrix(const uint8_t *par_row, const uint8_t *erased_idx, uint32_t e, uint8_t *V) {
+	for (uint32_t r = 0; r < e; ++r) {
+		uint8_t gen = 1;
+		for (int t = 0; t < par_row[r]; ++t) gen = lz::gf_mul_host(gen, 2);
+		for (uint32_t x = 0; x < e; ++x) {
+			uint8_t v = 1;
+			for (int t = 0; t < erased_idx[x]; ++t) v = lz::gf_mul_host(v, gen);
+			V[r * e + x] = v;
+		}
+	}
+}
+
+// as many stages as fit the 16-warp geometry's shared memory, at most six
+inline uint32_t recover_big_stages(uint32_t K, uint32_t G) {
+	const size_t fit = (kRecoverSmemCapBig - 256) / (static_cast<size_t>(K) * G * 4 * kStepBytes);
+	return static_cast<uint32_t>(fit < 6 ? fit : 6);
+}
+
+// available[i] != 0: part i can be read; want[i] != 0: part i is requested and has an output buffer; any_crc: a part among the first k
+// available ones carries stored CRCs (the call verifies); image: the chunk-order image is wanted.
+inline RecoverPlan recover_plan(int K, int M, bool cauchy, const uint8_t *available, const uint8_t *want, bool any_crc, bool image, uint32_t nb,
+                                uint32_t n_chunks, size_t part_stride, size_t chunk_out_stride, const RecoverOverrides &ov) {
+	RecoverPlan pl;
+	const int N = K + M;
+	if (K < 1 || K > 32 || M < 1 || N > 64 || nb == 0) return pl;
+	const bool direct = cauchy;   // no Horner syndromes for a Cauchy generator: general rows over the k inputs
+	if (direct && ov.direct_wide == -2) return pl;   // LZGPU_DIRECT_WIDE=-2: A/B against the generic route
+	const bool direct_forced = direct && ov.direct_wide >= 0;
+	if ((part_stride % 16) || (chunk_out_stride % 16)) return pl;
+	// inputs: the first k available parts (ec_read_plan.h:126-133)
+	int n_used = 0;
+	for (int i = 0; i < N && n_used < K; ++i)
+		if (available[i]) pl.used[n_used++] = static_cast<uint8_t>(i);
+	if (n_used < K) return pl;
+	for (int j = 0; j < 32; ++j) pl.slot_of_data[j] = 0xff;
+	uint32_t e = 0, n_par = 0;
+	for (int a = 0; a < K; ++a) {
+		const int idx = pl.used[a];
+		if (idx < K) pl.slot_of_data[idx] = static_cast<uint8_t>(a);
+		else if (n_par < 4) { pl.par_slot[n_par] = static_cast<uint8_t>(a); pl.par_row[n_par] = static_cast<uint8_t>(idx - K); ++n_par; }
+		else return pl;
+	}
+	for (int j = 0; j < K; ++j)
+		if (pl.slot_of_data[j] == 0xff) {
+			if (e >= 4) return pl;
+			pl.erased_idx[e++] = static_cast<uint8_t>(j);
+		}
+	if (e == 0 || e != n_par) return pl;
+	pl.e = e;
+	// Measured (profiles/sweep_r2.md, run 8): with general coefficients the rebuild is bound by the bit-plane multiplies, not by HBM, and
+	// the grid-stride gf_dot_kernel (full occupancy, no stage barriers) does e >= 2 rows faster than this kernel's 16 warps per SM
+	// even though it needs separate CRC and image passes: ec(8,6) three lost 2.7 ms against 6.2 ms per 64 chunks.  One lost part
+	// (ec(8,6): 2.45 ms against 3.98 with verification and image), and two lost parts when the call verifies and wants the image
+	// (ec(4,5) 4.39 against 4.87, ec(21,4) 5.05 against 5.38), stay here.
+	if (direct && !direct_forced && !(e == 1 || (e == 2 && any_crc && image))) return pl;
+	// every requested missing part must be a data part
+	for (int i = K; i < N; ++i)
+		if (want[i] && !available[i]) return pl;
+	// geometry: even G (1024-byte aligned slot regions), K*G*4 rows <= 256
+	// Two CTAs per SM with a 3-stage ring, or one CTA with 6 stages?  Measured on the same box (64 MiB chunks, fraction of
+	// the HBM copy peak, two / one):  ec(3,2) 2 lost 0.48 / 0.42 (+image 0.64 / 0.58),  xor3 1 lost 0.93 / 0.70 (+image
+	// 0.73 / 0.77),  ec(8,2) 2 lost 0.66 / 0.70 (+image 0.72 / 0.78),  ec(8,2) 1 lost 0.94 / 0.99.  So: the runtime-k
+	// shapes, except the single-erasure case that also writes the image.  LZGPU_RECOVER_TWO=0|1 forces either.
+	const bool two_auto = K != 8 && (e == 2 || (e == 1 && !image));
+	const bool two = e <= 2 && (ov.recover_two < 0 ? two_auto : ov.recover_two != 0);
+	// Measured (profiles/sweep_r2.md, fraction of the HBM peak, recover only / verify + image): the 16-warp CTA wins for the
+	// runtime-k shapes with two or more erased parts — ec(3,2) two lost 0.69 / 0.69 against 0.52 / 0.67 on two 9-warp CTAs, ec(5,3)
+	// three lost 0.29 / 0.42 against 0.23 / 0.32 and two lost 0.59 / 0.74 against 0.46 / 0.65 on one — while the k = 8 instantiation
+	// keeps one 9-warp CTA with six stages (two lost: 0.81 with verification and image against 0.70).  LZGPU_RECOVER_GEO=0|1|2 forces one.
+	int geo = ov.recover_geo >= 0 ? ov.recover_geo : (K != 8 && e >= 2) ? 2 : (two ? 1 : 0);
+	if (geo > 2) geo = 0;   // (any other forced value runs as geometry 0)
+	if (direct) geo = 2;
+	if (geo == 1 && e > 2) geo = 0;
+	// three lost data parts with parity rows 0, 1, 2 in use: bit planes + dedicated GF warps (bs_recover_kernel.cuh) — geometry: G even,
+	// the 16 G items of a step on the last ceil(16 G / 32) warps, the k G 4 input rows on the warps before them when the call verifies
+	// stored CRCs (no stream warps otherwise), one TMA box per part (G 4 <= 256 rows), at least three stages
+	const int bs_recover = ov.bs_recover < 0 ? LZ_BS_RECOVER_DEFAULT : ov.bs_recover;
+	const uint32_t bs_gf_warps = ov.bs_recover_gf_warps < 0 ? 8u : static_cast<uint32_t>(ov.bs_recover_gf_warps < 1 ? 1 : ov.bs_recover_gf_warps > 16 ? 16 : ov.bs_recover_gf_warps);
+	bool bs3 = !direct && e == 3 && bs_recover && pl.par_row[0] == 0 && pl.par_row[1] == 1 && pl.par_row[2] == 2;
+	uint32_t G = 0, n_stages = 0;
+	if (bs3) {
+		// Run 33 (fraction of the HBM peak, at most four / at most eight GF warps): rebuild only — no stream warps, G = 16, eight GF warps —
+		// ec(5,3) 0.440 / 0.682, ec(6,3) 0.388 / 0.628, ec(8,3) 0.452 / 0.648; with verification and image ec(5,3) 0.589 / 0.722 (seven GF
+		// warps), ec(6,3) 0.570 / 0.640 (six), but ec(8,3) 0.689 / 0.658 (five: one scheduler gets two of them).  So: the largest G, unless
+		// it only buys a fifth GF warp.
+		uint32_t g4 = 0;
+		for (uint32_t g = 2; g <= 64; g += 2) {
+			const size_t stage = static_cast<size_t>(K) * g * 4 * kStepBytes;
+			const uint32_t gf_warps = (16 * g + 31) / 32, stream_warps = any_crc ? (K * g * 4 + 31) / 32 : 0;
+			if (gf_warps > bs_gf_warps || gf_warps + stream_warps > kBsRecoverThreads / 32 || 3 * stage + 256 > static_cast<size_t>(kRecoverSmemCapBig)) break;
+			G = g;
+			if (gf_warps <= 4) g4 = g;
+		}
+		if (G && g4 && (16 * G + 31) / 32 == 5) G = g4;
+		if (G) n_stages = recover_big_stages(K, G);
+		else bs3 = false;
+	}
+	if (bs3) {
+		// (geometry chosen above)
+	} else if (geo == 2) {
+		// one 16-warp CTA: the largest G whose K*G*4 input rows fit 512 threads (one TMA box per part: G*4 <= 256 rows) and whose
+		// 32*G items fill whole rounds of the CTA (G a multiple of 16) where K allows, with at least three stages in 200 KiB
+		uint32_t best = 0, best16 = 0;
+		for (uint32_t g = 2; g <= 64; g += 2) {
+			const uint32_t rows = K * g * 4;
+			if (rows > 512 || 3 * static_cast<size_t>(rows) * kStepBytes + 256 > kRecoverSmemCapBig) break;
+			best = g;
+			if (g % 16 == 0) best16 = g;
+		}
+		G = best16 ? best16 : best;
+		if (G) n_stages = recover_big_stages(K, G);
+	} else {
+		n_stages = static_cast<uint32_t>(recover_stages(geo));
+		const size_t smem_cap = geo == 1 ? kRecoverSmemCap2 : kRecoverSmemCap;
+		for (uint32_t g = 2; g <= 64; g += 2) {
+			const uint32_t rows = K * g * 4;
+			if (rows > kMaxRows || static_cast<size_t>(n_stages) * rows * kStepBytes + 256 > smem_cap) break;
+			G = g;
+		}
+	}
+	if (G == 0) return pl;
+	pl.G = G;
+	pl.n_stages = n_stages;
+	pl.pb = (nb + K - 1) / K;
+	pl.units_per_chunk = (pl.pb + G - 1) / G;
+	const uint64_t total = static_cast<uint64_t>(pl.units_per_chunk) * n_chunks;
+	if (total > 0x7fffffffull) return pl;
+	pl.total_units = static_cast<uint32_t>(total);
+	pl.smem = static_cast<size_t>(n_stages) * K * G * 4 * kStepBytes + 16 * n_stages + 64;
+	if (!direct) {   // the generic route reports the singular case
+		uint8_t V[16], W[16];
+		recover_syndrome_matrix(pl.par_row, pl.erased_idx, e, V);
+		if (gf_invert_matrix(V, W, static_cast<int>(e)) != 0) return pl;
+	}
+	bool consecutive = true;
+	for (uint32_t r = 0; r < e; ++r) consecutive &= pl.par_row[r] == r;
+	const bool k8 = K == 8 && (G == 8 || geo == 2);
+	// RAID-6 shape on a runtime-k instantiation: x0 doublings for 2^x0 S0 when x0 <= 4 (more cost more than the bit-plane multiply)
+	if (e == 2 && pl.par_row[0] == 0 && pl.par_row[1] == 1 && !k8 && pl.erased_idx[0] <= 4) pl.raid6_dbl = pl.erased_idx[0];
+	// three unknowns, parity rows 0, 1, 2: x0 doublings / fourfold steps for 2^x0 S0, 4^x0 S0 when x0 <= 3
+	if (e == 3 && consecutive && pl.erased_idx[0] <= 3) pl.elim3_dbl = pl.erased_idx[0];
+	pl.ok = true;
+	pl.E = static_cast<int>(e);
+	if (bs3) {
+		pl.form = kRecoverBs3;
+		pl.KT = (K == 5 || K == 8) ? K : 0;
+		pl.R0 = 0; pl.R1 = 1;
+		pl.geo = 2;
+		pl.item_words = 8;
+	} else if (direct) {
+		// item width: run 8: the 8 / 16-byte items win on every shape (ec(32,4) four lost: 12.0 ms against 38.0 per 64 chunks); 4-byte
+		// items stay for A/B
+		const bool wide = ov.direct_wide >= 0 ? ov.direct_wide != 0 : true;
+		pl.form = kRecoverDirectForm;
+		pl.R0 = kRecoverDirect;
+		pl.geo = 2;
+		pl.item_words = wide ? recover_direct_wide_words(pl.E) : 1;
+	} else {
+		const bool row0 = pl.par_row[0] == 0, row01 = e >= 2 && consecutive;
+		const bool k3 = ov.recover_k3 != 0;
+		const bool verify_image = any_crc && image;
+		auto pick = [&](int kt, int r0, int r1) { pl.KT = kt; pl.R0 = r0; pl.R1 = r1; };
+		bool picked = true;
+		// ec(3,2) / ec(5,3) on the 16-warp geometry: compile-time k (the walk over the columns unrolls, parameter loads become immediates).
+		// Measured (run 18): ec(3,2) two lost, rebuild only 0.689 -> 0.827 of the HBM peak; with verification and image 0.692 -> 0.703.
+		// ec(5,3) (run 19): two lost, rebuild only 0.585 -> 0.682 but with verification and image 0.749 -> 0.717 (the unrolled walk costs
+		// the CRC role registers), so that combination keeps the runtime-k kernel; three lost 0.329 -> 0.373 and 0.471 -> 0.519.
+		// ec(4,2), ec(6,2), ec(6,3): the same rule as for k = 5.
+		if (K == 3 && geo == 2 && k3 && e == 1 && row0) pick(3, 0, -1);
+		else if (K == 3 && geo == 2 && k3 && e == 2 && row01) pick(3, 0, 1);
+		else if ((K == 4 || K == 5 || K == 6) && geo == 2 && k3 && e == 2 && row01 && !verify_image) pick(K, 0, 1);
+		else if ((K == 5 || K == 6) && geo == 2 && k3 && e == 3 && row01) pick(K, 0, 1);
+		else picked = false;
+		if (!picked) {
+			if (e == 1) row0 ? pick(k8 ? 8 : 0, 0, -1) : pick(0, -1, -1);
+			else if (e == 2) row01 ? pick(k8 ? 8 : 0, 0, 1) : pick(0, -1, -1);
+			else row01 ? pick(0, 0, 1) : pick(0, -1, -1);
+		}
+		pl.form = kRecoverPacked;
+		pl.geo = geo;
+		pl.item_words = recover_item_words(pl.E, geo);
+	}
+	pl.ctas_per_sm = pl.geo == 1 ? 2 : 1;
+	pl.threads = pl.geo == 2 ? static_cast<uint32_t>(kBsRecoverThreads) : static_cast<uint32_t>(recover_threads(pl.geo));
 	return pl;
 }
 

@@ -487,6 +487,49 @@ int lzgpu_plan_convert(const lzgpu_goal *src, const lzgpu_goal *dst, const uint8
 	return LZGPU_OK;
 }
 
+int lzgpu_plan_recover(const lzgpu_goal *g, const uint8_t *available, const uint8_t *want, int verify, int image, uint32_t n_chunks,
+                       uint32_t nb, size_t part_stride, size_t chunk_out_stride, const lzgpu_recover_overrides *overrides,
+                       lzgpu_recover_plan *out) {
+	if (!out || !lzgpu_goal_valid(g) || !available || !want || nb == 0 || nb > LZGPU_BLOCKS_IN_CHUNK) return LZGPU_ERR_ARG;
+	*out = lzgpu_recover_plan{};
+	lzd::RecoverOverrides ov;
+	if (overrides) {
+		ov.recover_two = overrides->recover_two;
+		ov.recover_geo = overrides->recover_geo;
+		ov.recover_k3 = overrides->recover_k3;
+		ov.bs_recover = overrides->bs_recover;
+		ov.bs_recover_gf_warps = overrides->bs_recover_gf_warps;
+		ov.direct_wide = overrides->direct_wide;
+	}
+	const lzd::RecoverPlan pl = lzd::recover_plan(g->k, g->m, lz::uses_cauchy(g->k, g->m), available, want, verify != 0, image != 0, nb, n_chunks,
+	                                              part_stride, chunk_out_stride, ov);
+	for (int a = 0; a < g->k; ++a) out->used[a] = pl.used[a];
+	if (!pl.ok) return LZGPU_OK;
+	out->fused = 1;
+	out->form = pl.form;
+	out->e = pl.E;
+	out->kt = pl.KT;
+	out->r0 = pl.R0;
+	out->r1 = pl.R1;
+	out->geo = pl.geo;
+	out->item_words = pl.item_words;
+	out->stripes_per_unit = pl.G;
+	out->stages = pl.n_stages;
+	out->units_per_chunk = pl.units_per_chunk;
+	out->units = pl.total_units;
+	out->ctas_per_sm = pl.ctas_per_sm;
+	out->threads_per_cta = pl.threads;
+	out->smem_bytes = static_cast<uint32_t>(pl.smem);
+	out->raid6_dbl = pl.raid6_dbl;
+	out->elim3_dbl = pl.elim3_dbl;
+	for (int x = 0; x < 4; ++x) {
+		out->erased[x] = pl.erased_idx[x];
+		out->par_row[x] = pl.par_row[x];
+		out->par_slot[x] = pl.par_slot[x];
+	}
+	return LZGPU_OK;
+}
+
 const char *lzgpu_version(void) { return "lizardfs_b200 0.1 (sm_100a)"; }
 
 }  // extern "C"

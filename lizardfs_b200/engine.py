@@ -540,6 +540,42 @@ class Engine:
         _check(_lib.load().lzgpu_plan_convert(C.byref(src.c), C.byref(dst.c), _p(a), _p(w), C.byref(out)), "plan_convert")
         return {f: getattr(out, f) for f, _ in _lib.LzConvertPlan._fields_}
 
+    # the environment switch behind each override of plan_recover
+    RECOVER_OVERRIDES = {"recover_two": "LZGPU_RECOVER_TWO", "recover_geo": "LZGPU_RECOVER_GEO", "recover_k3": "LZGPU_RECOVER_K3",
+                         "bs_recover": "LZGPU_BS_RECOVER", "bs_recover_gf_warps": "LZGPU_BS_RECOVER_GFW", "direct_wide": "LZGPU_DIRECT_WIDE"}
+    RECOVER_FORMS = ("packed", "bs3", "direct")
+
+    @staticmethod
+    def plan_recover(goal, available, want, verify, image, n_chunks, nb, part_stride=None, chunk_out_stride=None, **overrides):
+        """which kernel recover_chunks* would run (pure host logic, csrc/fused_plan.h recover_plan; no GPU needed).  available / want:
+        flags per part (want: requested with an output buffer); verify: the parts read carry stored CRCs; image: the chunk image is
+        wanted; overrides: the context's environment switches by their keys in RECOVER_OVERRIDES (-1 or absent = automatic).
+        Returns a dict with fused (0 = the generic kernels), form ("packed", "bs3", "direct"), e, kt, r0, r1, geo, item_words,
+        stripes_per_unit, stages, units_per_chunk, units, ctas_per_sm, threads_per_cta, smem_bytes, raid6_dbl, elim3_dbl, used (slot ->
+        part), erased, par_row, par_slot, and instantiation = (form, e, kt, r0, r1, geo, item_words) (None when not fused)."""
+        unknown = set(overrides) - set(Engine.RECOVER_OVERRIDES)
+        if unknown:
+            raise TypeError(f"plan_recover: unknown overrides {sorted(unknown)}")
+        ov = _lib.LzRecoverOverrides(*[int(overrides.get(f, -1)) for f, _ in _lib.LzRecoverOverrides._fields_])
+        a = np.asarray(available, dtype=np.uint8)
+        w = np.asarray(want, dtype=np.uint8)
+        n = goal.k + goal.m
+        assert a.size == n and w.size == n
+        pb = (nb + goal.k - 1) // goal.k
+        part_stride = pb * BLOCK_SIZE if part_stride is None else part_stride
+        chunk_out_stride = (nb * BLOCK_SIZE if image else 0) if chunk_out_stride is None else chunk_out_stride
+        out = _lib.LzRecoverPlan()
+        _check(_lib.load().lzgpu_plan_recover(C.byref(goal.c), _p(a), _p(w), 1 if verify else 0, 1 if image else 0, n_chunks, nb, part_stride,
+                                              chunk_out_stride, C.byref(ov), C.byref(out)), "plan_recover")
+        d = {f: getattr(out, f) for f, _ in _lib.LzRecoverPlan._fields_}
+        d["used"] = list(out.used)[:goal.k]
+        e = out.e
+        for f in ("erased", "par_row", "par_slot"):
+            d[f] = list(getattr(out, f))[:e]
+        d["form"] = Engine.RECOVER_FORMS[out.form]
+        d["instantiation"] = (d["form"], e, out.kt, out.r0, out.r1, out.geo, out.item_words) if out.fused else None
+        return d
+
     def convert_chunks(self, src, dst, nb, parts, want, part_crc=None, with_crc=True):
         """Rebuild the `want`ed parts of slice type `dst` from the available `parts` of slice type `src`
         (SliceRecoveryPlanner, slice_recovery_planner.h:87-204).  parts[i]: (n_chunks, pb_src*65536) uint8 or None.

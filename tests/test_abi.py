@@ -64,7 +64,8 @@ def test_struct_layouts_match_the_header(tmp_path):
     import ctypes as C
     import subprocess
     from lizardfs_b200 import _lib
-    structs = {"lzgpu_goal": _lib.LzGoal, "lzgpu_stats": _lib.LzStats, "lzgpu_block_write": _lib.LzBlockWrite, "lzgpu_encode_plan": _lib.LzEncodePlan}
+    structs = {"lzgpu_goal": _lib.LzGoal, "lzgpu_stats": _lib.LzStats, "lzgpu_block_write": _lib.LzBlockWrite, "lzgpu_encode_plan": _lib.LzEncodePlan,
+               "lzgpu_convert_plan": _lib.LzConvertPlan, "lzgpu_recover_overrides": _lib.LzRecoverOverrides, "lzgpu_recover_plan": _lib.LzRecoverPlan}
     lines = ['#include <stdio.h>', '#include <stddef.h>', '#include "lzgpu.h"', 'int main(void) {']
     for name, cls in structs.items():
         lines.append(f'printf("{name} %zu", sizeof({name}));')

@@ -386,16 +386,17 @@ def test_recover_all_patterns(eng, oracle, text, nblocks):
             assert (out[i][0] == o_ref[i]).all()
 
 
-@pytest.mark.parametrize("two", ["0", "1"])
+@pytest.mark.parametrize("geo", ["0", "1"])
 @pytest.mark.parametrize("text,nblocks,lost", [("ec(8,2)", 40, (1, 4)), ("ec(8,2)", 40, (6,)), ("ec(3,2)", 31, (0, 2)), ("xor3", 22, (1,)), ("ec(5,3)", 23, (3,)), ("ec(6,2)", 30, (0, 5))])
-def test_recover_one_and_two_ctas_per_sm(oracle, two, text, nblocks, lost):
-    """both geometries of the degraded-read kernel (one CTA per SM with 6 stages, two with 3) give the reference's bytes,
-    with and without CRC verification and the chunk-order image"""
-    os.environ["LZGPU_RECOVER_TWO"] = two
+def test_recover_one_and_two_ctas_per_sm(oracle, geo, text, nblocks, lost):
+    """both 9-warp geometries of the degraded-read kernel (LZGPU_RECOVER_GEO: 0 = one CTA per SM with 6 stages, 1 = two with 3) give
+    the reference's bytes, with and without CRC verification and the chunk-order image; the plan confirms the geometry each call runs
+    (runtime-k shapes with two lost parts would take the 16-warp CTA unless forced) and that it is one launch"""
+    os.environ["LZGPU_RECOVER_GEO"] = geo
     try:
         e = L.Engine()
     finally:
-        del os.environ["LZGPU_RECOVER_TWO"]
+        del os.environ["LZGPU_RECOVER_GEO"]
     goal = L.SliceType(text)
     k, m = goal.k, goal.m
     data = rnd((5, nblocks * BLOCK), 77)
@@ -414,7 +415,11 @@ def test_recover_one_and_two_ctas_per_sm(oracle, two, text, nblocks, lost):
     acrc = [None if i in lost else part_crc[i] for i in range(k + m)]
     want = [1 if i in lost else 0 for i in range(k + m)]
     for crcs, image in [(None, False), (acrc, True), (acrc, False), (None, True)]:
+        plan = L.Engine.plan_recover(goal, [0 if a is None else 1 for a in avail], want, crcs is not None, image, 5, nblocks, recover_geo=int(geo))
+        assert plan["fused"] and plan["geo"] == int(geo) and plan["form"] == "packed", (text, lost, plan["instantiation"])
+        before = e.stats()["kernel_launches"]
         out, img = e.recover_chunks(goal, nblocks, avail, part_crc=crcs, want=want, chunk_image=image)
+        assert e.stats()["kernel_launches"] - before == 1
         for i in lost:
             assert (out[i] == parts[i]).all(), (text, lost, i)
         if image:

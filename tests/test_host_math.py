@@ -359,3 +359,183 @@ def test_bitslice_three_lost_matches_the_reference_recovery(oracle, k):
                 assert (out[x] == data[j]).all(), (k, lost, dbl, x)
     bad = (C.c_int * 3)(2, 1, 0)
     assert lib.lzgpu_debug_bitslice_recover3(k, bad, cols.ctypes.data_as(C.c_void_p), 0, out.ctypes.data_as(C.c_void_p)) != 0
+
+
+# ---- degraded-read route (csrc/fused_plan.h recover_plan, the decision of lz_fused_recover) --------------------------------------
+
+# Every instantiation fused.cu sets a shared-memory size for — set_all_recover_attrs with set_recover_attr (geometries 0, 1 for
+# E <= 2, and 2) and set_direct_attr (both item widths) — as (form, E, KT, R0, R1, geometry, item words).  A route the plan picks
+# outside this set would launch a kernel without its attribute.
+RECOVER_INSTANTIATIONS = {
+    ("packed", 1, 8, 0, -1, 0, 4), ("packed", 1, 8, 0, -1, 1, 4), ("packed", 1, 8, 0, -1, 2, 4),
+    ("packed", 1, 0, 0, -1, 0, 4), ("packed", 1, 0, 0, -1, 1, 4), ("packed", 1, 0, 0, -1, 2, 4),
+    ("packed", 1, 0, -1, -1, 0, 4), ("packed", 1, 0, -1, -1, 1, 4), ("packed", 1, 0, -1, -1, 2, 4),
+    ("packed", 2, 8, 0, 1, 0, 4), ("packed", 2, 8, 0, 1, 1, 4), ("packed", 2, 8, 0, 1, 2, 4),
+    ("packed", 2, 0, 0, 1, 0, 4), ("packed", 2, 0, 0, 1, 1, 4), ("packed", 2, 0, 0, 1, 2, 4),
+    ("packed", 2, 0, -1, -1, 0, 4), ("packed", 2, 0, -1, -1, 1, 4), ("packed", 2, 0, -1, -1, 2, 4),
+    ("packed", 3, 0, 0, 1, 0, 4), ("packed", 3, 0, 0, 1, 2, 2),
+    ("packed", 3, 0, -1, -1, 0, 4), ("packed", 3, 0, -1, -1, 2, 2),
+    ("packed", 4, 0, 0, 1, 0, 4), ("packed", 4, 0, 0, 1, 2, 2),
+    ("packed", 4, 0, -1, -1, 0, 4), ("packed", 4, 0, -1, -1, 2, 2),
+    # compile-time k on the 16-warp geometry
+    ("packed", 1, 3, 0, -1, 2, 4), ("packed", 2, 3, 0, 1, 2, 4), ("packed", 2, 4, 0, 1, 2, 4), ("packed", 2, 5, 0, 1, 2, 4),
+    ("packed", 3, 5, 0, 1, 2, 2), ("packed", 2, 6, 0, 1, 2, 4), ("packed", 3, 6, 0, 1, 2, 2),
+    ("bs3", 3, 0, 0, 1, 2, 8), ("bs3", 3, 5, 0, 1, 2, 8), ("bs3", 3, 8, 0, 1, 2, 8),
+    ("direct", 1, 0, -2, -1, 2, 1), ("direct", 1, 0, -2, -1, 2, 4), ("direct", 2, 0, -2, -1, 2, 1), ("direct", 2, 0, -2, -1, 2, 2),
+    ("direct", 3, 0, -2, -1, 2, 1), ("direct", 3, 0, -2, -1, 2, 2), ("direct", 4, 0, -2, -1, 2, 1), ("direct", 4, 0, -2, -1, 2, 2),
+}
+# Four lost data parts need four parity parts in use, and a Vandermonde generator has at most four parity rows: they are rows
+# 0..3, so the instantiation for four unknowns with other rows has an attribute but no route to it.
+RECOVER_UNREACHABLE = {("packed", 4, 0, -1, -1, 0, 4), ("packed", 4, 0, -1, -1, 2, 2)}
+RECOVER_SMEM_CAP = {0: 200 * 1024, 1: 100 * 1024, 2: 208 * 1024}      # fused.cu kRecoverSmemCap, kRecoverSmemCap2, kRecoverSmemCapBig
+RECOVER_THREADS = {0: 288, 1: 288, 2: 512}
+
+
+def _recover_plan(text, lost, verify=False, image=False, want=None, n_chunks=64, nb=1024, **ov):
+    g = L.SliceType(text)
+    n = g.k + g.m
+    avail = [0 if i in lost else 1 for i in range(n)]
+    want = want if want is not None else [1 if (i in lost and i < g.k) else 0 for i in range(n)]
+    return L.Engine.plan_recover(g, avail, want, verify, image, n_chunks, nb, **ov)
+
+
+def test_recover_route_policy():
+    """The routing rules the comments of lz_fused_recover document, on named cases (pure host logic, no GPU)."""
+    P = _recover_plan
+    # k = 8 keeps the 9-warp CTA: one per SM, two when forced
+    assert P("ec(8,2)", (1, 4))["instantiation"] == ("packed", 2, 8, 0, 1, 0, 4)
+    assert P("ec(8,2)", (6,))["instantiation"] == ("packed", 1, 8, 0, -1, 0, 4)
+    assert P("ec(8,2)", (1, 4), recover_two=1)["geo"] == 1
+    assert P("ec(8,2)", (1, 4), recover_geo=2)["instantiation"] == ("packed", 2, 8, 0, 1, 2, 4)
+    # runtime k, one lost part: two CTAs per SM unless the call writes the image
+    assert P("ec(4,2)", (1,))["instantiation"] == ("packed", 1, 0, 0, -1, 1, 4)
+    assert P("ec(4,2)", (1,), image=True)["instantiation"] == ("packed", 1, 0, 0, -1, 0, 4)
+    # runtime k with two or more lost parts: the 16-warp CTA, whatever LZGPU_RECOVER_TWO says
+    for two in (-1, 0, 1):
+        p = P("ec(3,2)", (0, 2), recover_two=two)
+        assert (p["geo"], p["instantiation"]) == (2, ("packed", 2, 3, 0, 1, 2, 4)), two
+        assert P("ec(7,2)", (0, 6), recover_two=two)["instantiation"] == ("packed", 2, 0, 0, 1, 2, 4)
+    # forcing geometry 1 with more than two lost parts gives geometry 0
+    assert P("ec(5,3)", (0, 1, 4), bs_recover=0, recover_geo=1)["instantiation"] == ("packed", 3, 0, 0, 1, 0, 4)
+    assert P("ec(8,4)", (0, 1, 2, 3), recover_geo=1)["geo"] == 0
+    # three lost data parts with parity rows 0, 1, 2: the bit-plane kernel (compile-time k = 5 and 8, runtime k otherwise)
+    assert P("ec(5,3)", (0, 1, 4))["instantiation"] == ("bs3", 3, 5, 0, 1, 2, 8)
+    assert P("ec(8,3)", (1, 4, 6))["instantiation"] == ("bs3", 3, 8, 0, 1, 2, 8)
+    assert P("ec(7,3)", (1, 2, 6))["instantiation"] == ("bs3", 3, 0, 0, 1, 2, 8)
+    assert P("ec(8,4)", (0, 2, 5))["instantiation"] == ("bs3", 3, 8, 0, 1, 2, 8)     # parity 3 is a surplus part
+    assert P("ec(5,3)", (0, 1, 4), bs_recover=0)["instantiation"] == ("packed", 3, 5, 0, 1, 2, 2)
+    assert P("ec(5,3)", (0, 1, 4), bs_recover=0, recover_k3=0)["instantiation"] == ("packed", 3, 0, 0, 1, 2, 2)
+    assert P("ec(4,4)", (0, 1, 2, 4))["instantiation"] == ("packed", 3, 0, -1, -1, 2, 2)   # parity 0 lost: rows 1, 2, 3
+    # more GF warps allowed = a larger G, fewer = a smaller one; with verification the stream warps take their share
+    g8 = P("ec(5,3)", (0, 1, 4))["stripes_per_unit"]
+    assert P("ec(5,3)", (0, 1, 4), bs_recover_gf_warps=4)["stripes_per_unit"] < g8
+    assert P("ec(5,3)", (0, 1, 4), verify=True)["stripes_per_unit"] <= g8
+    # k = 4, 5, 6 with two lost parts: compile-time k, except with verification and the image (the runtime-k kernel measured faster)
+    for text, lost in (("ec(4,2)", (0, 1)), ("ec(5,3)", (1, 3)), ("ec(6,2)", (0, 5))):
+        k = L.SliceType(text).k
+        for verify, image in ((False, False), (True, False), (False, True)):
+            assert P(text, lost, verify, image)["instantiation"] == ("packed", 2, k, 0, 1, 2, 4), (text, verify, image)
+        assert P(text, lost, True, True)["instantiation"] == ("packed", 2, 0, 0, 1, 2, 4), text
+        assert P(text, lost, recover_k3=0)["instantiation"] == ("packed", 2, 0, 0, 1, 2, 4), text
+    assert P("ec(3,2)", (1,), recover_geo=2)["instantiation"] == ("packed", 1, 3, 0, -1, 2, 4)
+    assert P("ec(3,2)", (1,), recover_geo=2, recover_k3=0)["instantiation"] == ("packed", 1, 0, 0, -1, 2, 4)
+    # parity row 0 lost: rows other than 0, 1 in use, read from the parameters
+    assert P("ec(4,3)", (0, 1, 4))["instantiation"] == ("packed", 2, 0, -1, -1, 2, 4)
+    assert P("ec(4,2)", (1, 4))["instantiation"] == ("packed", 1, 0, -1, -1, 1, 4)
+    # RAID-6 doublings up to a first unknown at position 4, the elimination's up to position 3; a product beyond
+    assert P("ec(7,2)", (4, 6))["raid6_dbl"] == 4 and P("ec(7,2)", (5, 6))["raid6_dbl"] == 0xff
+    assert P("ec(8,2)", (1, 4))["raid6_dbl"] == 0xff        # the k = 8 kernel multiplies
+    assert P("ec(7,3)", (3, 5, 6))["elim3_dbl"] == 3 and P("ec(7,3)", (4, 5, 6))["elim3_dbl"] == 0xff
+    # Cauchy generators: the DIRECT form on the 16-warp CTA for one lost part, or two with verification and the image; the rest goes to
+    # the generic kernels unless LZGPU_DIRECT_WIDE forces the form (0: 4-byte items, 1: wide), -2 switches the form off
+    assert P("ec(8,6)", (3,))["instantiation"] == ("direct", 1, 0, -2, -1, 2, 4)
+    assert P("ec(8,6)", (1, 4), True, True)["instantiation"] == ("direct", 2, 0, -2, -1, 2, 2)
+    for verify, image in ((False, False), (True, False), (False, True)):
+        assert P("ec(8,6)", (1, 4), verify, image)["fused"] == 0
+        assert P("ec(8,6)", (1, 4), verify, image, direct_wide=1)["instantiation"] == ("direct", 2, 0, -2, -1, 2, 2)
+    assert P("ec(8,6)", (1, 4, 7), True, True)["fused"] == 0
+    assert P("ec(8,6)", (1, 4, 7), direct_wide=0)["instantiation"] == ("direct", 3, 0, -2, -1, 2, 1)
+    assert P("ec(21,4)", (0, 20), True, True)["form"] == "direct"
+    assert P("ec(8,6)", (3,), direct_wide=-2)["fused"] == 0
+    # the generic kernels also take: a lost parity part that is asked for, nothing lost, an unaligned stride, too many units
+    assert P("ec(8,2)", (1, 8), want=[0, 1, 0, 0, 0, 0, 0, 0, 1, 0])["fused"] == 0
+    assert P("ec(8,2)", (8,))["fused"] == 0
+    assert L.Engine.plan_recover(L.SliceType("ec(8,2)"), [0] + [1] * 9, [1] + [0] * 9, False, False, 4, 64, part_stride=8 * BLOCK + 8)["fused"] == 0
+    assert _recover_plan("ec(8,2)", (1, 4), n_chunks=0xffffffff)["fused"] == 0
+    # the plan names the inputs: the first k available parts, the erased data parts and the parity rows in use
+    p = P("ec(8,4)", (1, 4, 8))
+    assert p["used"] == [0, 2, 3, 5, 6, 7, 9, 10] and p["erased"] == [1, 4] and p["par_row"] == [1, 2] and p["par_slot"] == [6, 7]
+
+
+def _recover_patterns(k, m, rng):
+    """loss patterns of up to four parts: every one where there are few, a seeded sample plus the edges otherwise"""
+    n = k + m
+    every = [p for r in range(1, min(4, m) + 1) for p in itertools.combinations(range(n), r)]
+    if len(every) <= 60:
+        return every
+    edges = [tuple(range(min(4, m))), tuple(range(k - min(4, m), k)), (0, k), (k - 1, k), tuple(range(k, k + min(4, m)))]
+    sample = [every[i] for i in rng.choice(len(every), size=36, replace=False)]
+    return edges + sample
+
+
+def test_recover_plan_sweep_fits_its_instantiation():
+    """Every plan over k = 2..32, m = 1..8 (Vandermonde and Cauchy generators), loss patterns of up to four parts, every verify / image
+    combination and every value of every override must name an instantiation the library sets up, with a geometry that fits it:
+    even G, a TMA box of G*4 <= 256 rows, the input rows on the CTA's threads, the stage ring in the geometry's shared memory, at least
+    three stages on the 16-warp CTA, fewer than 2^31 units.  A route without an instantiation, or one that does not fit, fails here."""
+    lib = L._lib.load()
+    ov_sets = [{}] + [{"recover_two": v} for v in (0, 1)] + [{"recover_geo": v} for v in (0, 1, 2)] + [{"recover_k3": 0}] + \
+              [{"bs_recover": 0}] + [{"bs_recover_gf_warps": v} for v in range(1, 17)] + [{"direct_wide": v} for v in (-2, 0, 1)] + \
+              [{"recover_geo": 1, "recover_two": 0}, {"recover_geo": 0, "recover_k3": 0, "bs_recover": 0}, {"recover_geo": 2, "recover_k3": 0}]
+    ovs = []
+    for d in ov_sets:
+        ovs.append((d, L._lib.LzRecoverOverrides(*[int(d.get(f, -1)) for f, _ in L._lib.LzRecoverOverrides._fields_])))
+    rng = np.random.default_rng(2024)
+    reached = set()
+    n_handled = 0
+    out = L._lib.LzRecoverPlan()
+    avail = (C.c_uint8 * 64)()
+    want = (C.c_uint8 * 64)()
+    n_chunks, nb = 37, 1000
+    for k in range(2, 33):
+        for m in range(1, 9):
+            goal = L.SliceType(1, k, m)
+            cauchy = m >= 5 or (m == 4 and k > 20)
+            for lost in _recover_patterns(k, m, rng):
+                for i in range(k + m):
+                    avail[i] = 0 if i in lost else 1
+                    want[i] = 1 if (i in lost and i < k) else 0
+                used = [i for i in range(k + m) if i not in lost][:k]
+                erased = [j for j in range(k) if j not in used]
+                rows = [i - k for i in used if i >= k]
+                pb = -(-nb // k)
+                for verify, image in itertools.product((0, 1), (0, 1)):
+                    for d, ov in ovs:
+                        assert lib.lzgpu_plan_recover(C.byref(goal.c), avail, want, verify, image, n_chunks, nb, pb * BLOCK,
+                                                      nb * BLOCK if image else 0, C.byref(ov), C.byref(out)) == 0
+                        where = (k, m, lost, verify, image, d)
+                        if not out.fused:
+                            continue
+                        n_handled += 1
+                        inst = (L.Engine.RECOVER_FORMS[out.form], out.e, out.kt, out.r0, out.r1, out.geo, out.item_words)
+                        assert inst in RECOVER_INSTANTIATIONS, (inst, where)
+                        reached.add(inst)
+                        e, G, K = out.e, out.stripes_per_unit, k
+                        assert e == len(erased) and list(out.erased)[:e] == erased and list(out.par_row)[:e] == rows, where
+                        assert (inst[0] == "direct") == cauchy, where
+                        assert G >= 2 and G % 2 == 0 and G * 4 <= 256, (G, where)
+                        if inst[0] == "bs3":
+                            gf_warps = (16 * G + 31) // 32
+                            assert rows == [0, 1, 2] and gf_warps <= d.get("bs_recover_gf_warps", 8), where
+                            assert gf_warps + (-(-K * G * 4 // 32) if verify else 0) <= 16, where
+                        else:
+                            assert K * G * 4 <= (256 if out.geo < 2 else 512) <= RECOVER_THREADS[out.geo], where
+                        smem = out.stages * K * G * 4 * 128 + 16 * out.stages + 64
+                        assert out.smem_bytes == smem and smem <= RECOVER_SMEM_CAP[out.geo], (smem, where)
+                        assert out.stages == {0: 6, 1: 3}[out.geo] if out.geo < 2 else 3 <= out.stages <= 6, where
+                        assert out.threads_per_cta == RECOVER_THREADS[out.geo] and out.ctas_per_sm == (2 if out.geo == 1 else 1), where
+                        assert out.units_per_chunk == -(-pb // G) and out.units == out.units_per_chunk * n_chunks < 2 ** 31, where
+                        assert out.raid6_dbl == (erased[0] if (e == 2 and rows == [0, 1] and k != 8 and erased[0] <= 4) else 0xff), where
+                        assert out.elim3_dbl == (erased[0] if (e == 3 and rows == [0, 1, 2] and erased[0] <= 3) else 0xff), where
+    assert n_handled > 100000
+    assert reached == RECOVER_INSTANTIATIONS - RECOVER_UNREACHABLE, sorted(RECOVER_INSTANTIATIONS - RECOVER_UNREACHABLE - reached)
