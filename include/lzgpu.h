@@ -271,6 +271,68 @@ int lzgpu_recover_chunks_dev(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_
                              int64_t *bad /* host, optional: chunk, part, block of the first mismatch */,
                              void *stream);
 
+/* Degraded read of a batch whose chunks have lost different parts: a loss pattern per chunk (a rebuild after a chunkserver loss,
+ * where each chunk of a file misses a different part index; ECReadPlan::recoverParts, ec_read_plan.h:113-146, per chunk).
+ *   masks[c]      (host, n_chunks) available: bit i = part i of chunk c can be read; want: bit i = part i of chunk c is requested.
+ *   d_parts[i]    part-major buffer of part i for all chunks, chunk c at + c*part_stride.  Only the regions of available parts are read;
+ *                 d_parts[i] may be NULL only when no chunk has part i.  d_part_crc, d_out, d_chunk_out as in lzgpu_recover_chunks_dev.
+ * For every chunk c the result is byte for byte what lzgpu_recover_chunks returns for that chunk alone with parts[i] = available bit i ?
+ * d_parts[i] + c*part_stride : NULL and want from masks[c].want: the first k available parts of THAT chunk are its inputs and the only
+ * parts verified; a requested part that is available is not written; output regions of chunks that do not rebuild that part stay
+ * untouched; with d_chunk_out every data part is implicitly wanted.  A chunk with fewer than k available parts makes the call return
+ * LZGPU_ERR_TOO_FEW_PARTS before anything is enqueued (lzgpu_last_error names the chunk).  A stored-CRC mismatch returns LZGPU_ERR_CRC
+ * with the smallest (chunk, part, block) in bad.  Waiting, deferred verification and statistics as in lzgpu_recover_chunks_dev (in
+ * deferred mode a call leaves one verdict per route it used; lzgpu_dev_sync reports the first mismatching one).
+ * Chunks that rebuild one to four data parts and no parity part run in one launch per rebuilt-part count, whatever their patterns;
+ * the others (nothing lost among the inputs, a lost parity part requested) go through lzgpu_recover_chunks' route, one call per pattern;
+ * a batch with one pattern is that call.  lzgpu_recover_chunks_masked: host pointers, the H2D | kernel | D2H pipeline of
+ * lzgpu_recover_chunks. */
+typedef struct lzgpu_chunk_mask {
+	uint64_t available; /* bit i: part i of this chunk can be read (this API's numbering, data 0..k-1, parity k..k+m-1) */
+	uint64_t want;      /* bit i: part i of this chunk is requested */
+} lzgpu_chunk_mask;
+int lzgpu_recover_chunks_masked_dev(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chunks, uint32_t nb,
+                                    const lzgpu_chunk_mask *masks /* host, n_chunks */,
+                                    const void *const *d_parts, size_t part_stride, const void *const *d_part_crc,
+                                    void *const *d_out, void *d_chunk_out, size_t chunk_out_stride,
+                                    int64_t *bad, void *stream);
+int lzgpu_recover_chunks_masked(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chunks, uint32_t nb,
+                                const lzgpu_chunk_mask *masks, const uint8_t *const *parts, size_t part_stride,
+                                const uint32_t *const *part_crc, uint8_t *const *out,
+                                uint8_t *chunk_out, size_t chunk_out_stride, int64_t *bad);
+/* How lzgpu_recover_chunks_masked* serves a batch (pure host logic, no GPU needed).  A pattern is (the first k available parts, the
+ * parts rebuilt = requested and unavailable, plus every unavailable data part with the image).  route[c] (optional, n_chunks): 0 the
+ * batch is delegated whole to lzgpu_recover_chunks' route, 1 the one-launch masked kernel, 2 lzgpu_recover_chunks' route for the
+ * chunk's pattern group.  LZGPU_ERR_TOO_FEW_PARTS for a chunk with fewer than k available parts. */
+#define LZGPU_MASKED_DELEGATED 0
+#define LZGPU_MASKED_ONE_LAUNCH 1
+#define LZGPU_MASKED_FALLBACK 2
+typedef struct lzgpu_masked_plan {
+	int delegated;              /* 1: one pattern in the batch, run as one lzgpu_recover_chunks_dev call */
+	uint32_t patterns;          /* distinct normalised patterns */
+	uint32_t one_launch_chunks, fallback_chunks, fallback_groups;
+	uint32_t rebuild_launches;  /* masked launches (one per rebuilt-part count present) + fallback groups; 1 when delegated */
+	uint32_t e_chunks[4];       /* one-launch chunks that rebuild e = 1..4 data parts */
+	/* the masked instantiation: fused_recover_kernel<e, 0, r0, -1, 64, 2, item_words, masked> (form 0: r0 = -1, Vandermonde rows at run
+	 * time; form 2: r0 = -2, the DIRECT rows of a Cauchy generator), one 16-warp CTA per SM; item_words for e = 1..4 */
+	int form;
+	uint32_t item_words[4];
+	uint32_t stripes_per_unit, stages, units_per_chunk, threads_per_cta, smem_bytes, desc_bytes;
+} lzgpu_masked_plan;
+int lzgpu_plan_recover_masked(const lzgpu_goal *g, uint32_t n_chunks, uint32_t nb, const lzgpu_chunk_mask *masks, int verify, int image,
+                              size_t part_stride, size_t chunk_out_stride, uint8_t *route /* optional, per chunk */, lzgpu_masked_plan *out);
+/* Diagnostics (pure host logic): the descriptor the masked kernel gets for one chunk.  one_launch = 0: the chunk is served by the
+ * existing route.  rows[x*32 + a]: what rebuilt part x (data part erased[x]) is as a combination of the k inputs in slot order
+ * (used[a]); for a Vandermonde generator the product of the kernel's V^-1 with the syndrome rows. */
+typedef struct lzgpu_masked_chunk {
+	int one_launch;
+	uint32_t e;
+	uint8_t used[32];
+	uint8_t erased[4];
+	uint8_t rows[4 * 32];
+} lzgpu_masked_chunk;
+int lzgpu_debug_masked_chunk(const lzgpu_goal *g, const lzgpu_chunk_mask *mask, int image, lzgpu_masked_chunk *out);
+
 /* Wire-format producer (SURVEY.md §8 f3): LIZ_CLTOCS_WRITE_DATA packet prefixes (src/protocol/cltocs.h:116-137) for
  * every block of every part of the encoded chunks, built on the GPU straight from the CRC array of
  * lzgpu_encode_chunks, so that WriteExecutor::addDataPacket (src/common/write_executor.cc:91-107) becomes a pointer

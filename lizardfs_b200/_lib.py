@@ -52,6 +52,21 @@ class LzRecoverPlan(C.Structure):
                 ("par_row", C.c_uint8 * 4), ("par_slot", C.c_uint8 * 4)]
 
 
+class LzChunkMask(C.Structure):
+    _fields_ = [("available", C.c_uint64), ("want", C.c_uint64)]
+
+
+class LzMaskedPlan(C.Structure):
+    _fields_ = [("delegated", C.c_int), ("patterns", C.c_uint32), ("one_launch_chunks", C.c_uint32), ("fallback_chunks", C.c_uint32),
+                ("fallback_groups", C.c_uint32), ("rebuild_launches", C.c_uint32), ("e_chunks", C.c_uint32 * 4), ("form", C.c_int),
+                ("item_words", C.c_uint32 * 4), ("stripes_per_unit", C.c_uint32), ("stages", C.c_uint32), ("units_per_chunk", C.c_uint32),
+                ("threads_per_cta", C.c_uint32), ("smem_bytes", C.c_uint32), ("desc_bytes", C.c_uint32)]
+
+
+class LzMaskedChunk(C.Structure):
+    _fields_ = [("one_launch", C.c_int), ("e", C.c_uint32), ("used", C.c_uint8 * 32), ("erased", C.c_uint8 * 4), ("rows", C.c_uint8 * 128)]
+
+
 class LzBlockWrite(C.Structure):
     _fields_ = [("block", C.c_uint32), ("offset", C.c_uint32), ("size", C.c_uint32), ("crc", C.c_uint32),
                 ("payload_off", C.c_uint64), ("exists", C.c_uint32), ("status", C.c_int32)]
@@ -88,6 +103,10 @@ SIGNATURES = {
     "lzgpu_encode_chunks_dev": (_int, [_vp, _goalp, _u32, _u32, _vp, _sz, _vp, _sz, _vp, _sz, _vp]),
     "lzgpu_recover_chunks": (_int, [_vp, _goalp, _u32, _u32, _vp, _sz, _vp, _vp, _vp, _vp, _sz, _vp]),
     "lzgpu_recover_chunks_dev": (_int, [_vp, _goalp, _u32, _u32, _vp, _sz, _vp, _vp, _vp, _vp, _sz, _vp, _vp]),
+    "lzgpu_recover_chunks_masked": (_int, [_vp, _goalp, _u32, _u32, _vp, _vp, _sz, _vp, _vp, _vp, _sz, _vp]),
+    "lzgpu_recover_chunks_masked_dev": (_int, [_vp, _goalp, _u32, _u32, _vp, _vp, _sz, _vp, _vp, _vp, _sz, _vp, _vp]),
+    "lzgpu_plan_recover_masked": (_int, [_goalp, _u32, _u32, _vp, _int, _int, _sz, _sz, _vp, _vp]),
+    "lzgpu_debug_masked_chunk": (_int, [_goalp, _vp, _int, _vp]),
     "lzgpu_write_data_prefixes": (_int, [_vp, _goalp, _u32, _u32, _vp, _sz, _vp, _u32, _vp]),
     "lzgpu_write_data_prefixes_dev": (_int, [_vp, _goalp, _u32, _u32, _vp, _sz, _vp, _u32, _vp, _vp]),
     "lzgpu_split_chunks": (_int, [_vp, _goalp, _u32, _u32, _vp, _sz, _vp, _sz]),

@@ -16,6 +16,7 @@
 #include <vector>
 
 #include "engine_internal.h"
+#include "fused_plan.h"
 #include "host_math.h"
 #include "kernels_generic.cuh"
 #include "lzgpu.h"
@@ -621,6 +622,8 @@ static int ticket_result(lzgpu_ctx *ctx, VerifyTicket *tk, int64_t *bad) {
 	lz_status_release(ctx, tk->slot);
 	tk->slot.index = -1;
 	if (best_chunk < 0) return LZGPU_OK;
+	if (tk->chunk_of) best_chunk = (*tk->chunk_of)[static_cast<size_t>(best_chunk)];
+	best_chunk += tk->chunk_base;
 	if (bad) { bad[0] = best_chunk; bad[1] = best_part; bad[2] = best_block; }
 	lz_set_error("CRC mismatch: chunk %lld part %lld block %lld", best_chunk, best_part, best_block);
 	return LZGPU_ERR_CRC;
@@ -955,6 +958,410 @@ extern "C" int lzgpu_recover_chunks(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint
 	for (uint32_t i = 0; i < static_cast<uint32_t>(n_slots); ++i) {
 		const int s = static_cast<int>((t + i) % n_slots);
 		if ((rc = retire_slot(ctx, s, &ss[s], bad))) { drain_slots(ctx, ss); return rc; }
+	}
+	return LZGPU_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// degraded read with a loss pattern per chunk (fused_plan.h masked_route: delegated / one launch per e / fallback groups)
+// ------------------------------------------------------------------------------------------------
+static void tickets_drop(lzgpu_ctx *ctx, std::vector<VerifyTicket> *tks) {
+	for (VerifyTicket &tk : *tks) ticket_drop(ctx, &tk);
+	tks->clear();
+}
+
+// after the stream has been synchronised: the smallest (chunk, part, block) over every route of the call
+static int tickets_result(lzgpu_ctx *ctx, std::vector<VerifyTicket> *tks, int64_t *bad) {
+	int rc = LZGPU_OK;
+	int64_t best[3] = {-1, -1, -1};
+	for (VerifyTicket &tk : *tks) {
+		int64_t b[3] = {-1, -1, -1};
+		const int r = ticket_result(ctx, &tk, b);
+		if (r == LZGPU_ERR_CRC) {
+			if (rc != LZGPU_ERR_CRC || std::lexicographical_compare(b, b + 3, best, best + 3)) std::copy(b, b + 3, best);
+			rc = LZGPU_ERR_CRC;
+		} else if (r != LZGPU_OK && rc == LZGPU_OK) {
+			rc = r;
+		}
+	}
+	tks->clear();
+	if (rc == LZGPU_ERR_CRC) {
+		if (bad) std::copy(best, best + 3, bad);
+		lz_set_error("CRC mismatch: chunk %lld part %lld block %lld", static_cast<long long>(best[0]), static_cast<long long>(best[1]),
+		             static_cast<long long>(best[2]));
+	}
+	return rc;
+}
+
+static MaskedRouting masked_routing(const lzgpu_goal *goal, uint32_t n_chunks, const lzgpu_chunk_mask *masks, bool image, bool verify, uint64_t store_ok) {
+	std::vector<uint64_t> avail(n_chunks), want(n_chunks);
+	for (uint32_t c = 0; c < n_chunks; ++c) { avail[c] = masks[c].available; want[c] = masks[c].want; }
+	return masked_route(goal->k, goal->m, lz::uses_cauchy(goal->k, goal->m), n_chunks, avail.data(), want.data(), image, verify, store_ok);
+}
+
+static int masked_too_few(const MaskedRouting &R, int k) {
+	lz_set_error("recover_masked: chunk %d has only %d of %d required parts available", R.too_few_chunk, R.too_few_parts, k);
+	return LZGPU_ERR_TOO_FEW_PARTS;
+}
+
+// algorithmic bytes (DESIGN.md §4.2) summed over the chunks, each with its own rebuilt-part count
+static uint64_t masked_alg_bytes(const lzgpu_goal *goal, uint32_t nb, const MaskedRouting &R, bool image, bool crcs) {
+	const uint64_t pb = (nb + goal->k - 1) / goal->k, B = LZGPU_BLOCK_SIZE;
+	uint64_t total = 0;
+	for (const MaskedPattern &pt : R.pattern)
+		total += goal->k * pb * B + (crcs ? 4ull * goal->k * pb : 0) + static_cast<uint64_t>(__builtin_popcountll(pt.rebuilt)) * pb * B +
+		         (image ? static_cast<uint64_t>(nb) * B : 0);
+	return total;
+}
+
+// enqueue the whole masked degraded read on `st`; *tks receives one pending verification per route that verified
+static int masked_enqueue(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chunks, uint32_t nb, const MaskedRouting &R,
+                          const void *const *d_parts, size_t part_stride, const void *const *d_part_crc, void *const *d_out, void *d_chunk_out,
+                          size_t chunk_out_stride, cudaStream_t st, std::vector<VerifyTicket> *tks) {
+	const int k = goal->k, n = goal->k + goal->m;
+	const uint32_t B = LZGPU_BLOCK_SIZE, pb = (nb + k - 1) / k;
+	const size_t part_bytes = static_cast<size_t>(pb) * B;
+	int rc;
+	auto fail = [&](int r) { tickets_drop(ctx, tks); return r; };
+	if (R.delegated) {
+		const MaskedPattern &pt = R.pattern[0];
+		const void *dp[LZGPU_MAX_PARTS] = {nullptr};
+		uint8_t want[LZGPU_MAX_PARTS] = {0};
+		for (int i = 0; i < n; ++i) {
+			dp[i] = (pt.used >> i & 1) ? d_parts[i] : nullptr;
+			want[i] = (pt.rebuilt >> i & 1) ? 1 : 0;
+		}
+		VerifyTicket tk;
+		if ((rc = recover_enqueue(ctx, goal, n_chunks, nb, dp, part_stride, d_part_crc, want, d_out, d_chunk_out, chunk_out_stride, st, &tk)))
+			return fail(rc);
+		if (tk.active()) tks->push_back(tk);
+		return LZGPU_OK;
+	}
+	// one launch per rebuilt-part count over every chunk that rebuilds data parts only
+	if (!R.desc.empty()) {
+		uint64_t used_any = 0;
+		for (const MaskedChunkDesc &d : R.desc) used_any |= R.pattern[d.chunk].used;
+		bool any_crc = false;
+		for (int i = 0; i < n; ++i) any_crc |= (used_any >> i & 1) && d_part_crc && d_part_crc[i];
+		TmpBuf t_desc(ctx, st);
+		const size_t desc_bytes = R.desc.size() * sizeof(MaskedChunkDesc);
+		if ((rc = t_desc.alloc(desc_bytes))) return fail(rc);
+		CUDA_TRY(cudaMemcpyAsync(t_desc.p, R.desc.data(), desc_bytes, cudaMemcpyHostToDevice, st));
+		VerifyTicket tk;
+		if (any_crc) {
+			if ((rc = lz_status_acquire(ctx, &tk.slot))) return fail(rc);
+			tks->push_back(tk);
+			CUDA_TRY(cudaMemsetAsync(tk.slot.d, 0xff, sizeof(unsigned long long), st));
+		}
+		if ((rc = lz_fused_recover_masked(ctx, goal, n_chunks, nb, d_parts, part_stride, any_crc ? d_part_crc : nullptr, d_out, d_chunk_out,
+		                                  chunk_out_stride, static_cast<const MaskedChunkDesc *>(t_desc.p), R.e_chunks, st, tk.slot.d)))
+			return fail(rc);
+		ctx->stats.chunks_recovered += R.desc.size();
+		if (any_crc) {
+			VerifyTicket &t = tks->back();
+			t.fused = true;
+			t.n_words = 1;
+			t.blocks = pb;
+			CUDA_TRY(cudaMemcpyAsync(t.slot.h, t.slot.d, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+		}
+	}
+	// the other chunks: the existing route, one call per pattern — on a run of consecutive chunks in place, otherwise on a compact copy
+	for (const auto &grp : R.groups) {
+		const MaskedPattern &pt = grp.first;
+		const std::vector<uint32_t> &list = grp.second;
+		const uint32_t ng = static_cast<uint32_t>(list.size());
+		uint8_t want[LZGPU_MAX_PARTS] = {0};
+		bool any_crc = false;
+		for (int i = 0; i < n; ++i) {
+			want[i] = (pt.rebuilt >> i & 1) ? 1 : 0;
+			any_crc |= (pt.used >> i & 1) && d_part_crc && d_part_crc[i];
+		}
+		const void *dp[LZGPU_MAX_PARTS] = {nullptr}, *dc[LZGPU_MAX_PARTS] = {nullptr};
+		void *dout[LZGPU_MAX_PARTS] = {nullptr};
+		VerifyTicket tk;
+		if (list.back() - list.front() + 1 == ng) {
+			const size_t c0 = list.front();
+			for (int i = 0; i < n; ++i) {
+				if (pt.used >> i & 1) {
+					dp[i] = static_cast<const uint8_t *>(d_parts[i]) + c0 * part_stride;
+					if (any_crc && d_part_crc[i]) dc[i] = static_cast<const uint32_t *>(d_part_crc[i]) + c0 * pb;
+				}
+				if ((pt.rebuilt >> i & 1) && d_out && d_out[i]) dout[i] = static_cast<uint8_t *>(d_out[i]) + c0 * part_stride;
+			}
+			uint8_t *img = d_chunk_out ? static_cast<uint8_t *>(d_chunk_out) + c0 * chunk_out_stride : nullptr;
+			if ((rc = recover_enqueue(ctx, goal, ng, nb, dp, part_stride, any_crc ? dc : nullptr, want, dout, img, chunk_out_stride, st, &tk)))
+				return fail(rc);
+			tk.chunk_base = static_cast<uint32_t>(c0);
+		} else {
+			// compact copy: the inputs (and their stored CRCs) gathered, the call run on it, the rebuilt parts and the image scattered back
+			RowsCopyArgs in{}, out{};
+			size_t off = 0;
+			size_t in_off[LZGPU_MAX_PARTS], crc_off[LZGPU_MAX_PARTS], out_off[LZGPU_MAX_PARTS], img_off = 0;
+			for (int i = 0; i < n; ++i) {
+				if (pt.used >> i & 1) { in_off[i] = off; off += ng * part_bytes; }
+				if ((pt.used >> i & 1) && any_crc && d_part_crc[i]) { crc_off[i] = off; off += (ng * pb * 4 + 15) & ~size_t(15); }
+				if ((pt.rebuilt >> i & 1) && d_out && d_out[i]) { out_off[i] = off; off += ng * part_bytes; }
+			}
+			if (d_chunk_out) { img_off = off; off += static_cast<size_t>(ng) * nb * B; }
+			TmpBuf t_buf(ctx, st), t_idx(ctx, st);
+			if ((rc = t_buf.alloc(off)) || (rc = t_idx.alloc(ng * sizeof(uint32_t)))) return fail(rc);
+			CUDA_TRY(cudaMemcpyAsync(t_idx.p, list.data(), ng * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+			uint8_t *base = static_cast<uint8_t *>(t_buf.p);
+			auto plane = [&](RowsCopyArgs &a, const void *src, void *dst, size_t src_stride, size_t dst_stride, size_t row_bytes, bool gather) {
+				RowsPlane &P = a.pl[a.n_rows++];   // (n_rows counts planes until the launch)
+				P.src = static_cast<const uint8_t *>(src);
+				P.dst = static_cast<uint8_t *>(dst);
+				P.src_stride = src_stride;
+				P.dst_stride = dst_stride;
+				P.row_bytes = row_bytes;
+				P.gather = gather ? 1u : 0u;
+				P.wide = ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst) | src_stride | dst_stride | row_bytes) & 15) == 0;
+			};
+			for (int i = 0; i < n; ++i) {
+				if (pt.used >> i & 1) {
+					dp[i] = base + in_off[i];
+					plane(in, d_parts[i], base + in_off[i], part_stride, part_bytes, part_bytes, true);
+					if (any_crc && d_part_crc[i]) {
+						dc[i] = base + crc_off[i];
+						plane(in, d_part_crc[i], base + crc_off[i], pb * 4ull, pb * 4ull, pb * 4ull, true);
+					}
+				}
+				if ((pt.rebuilt >> i & 1) && d_out && d_out[i]) {
+					dout[i] = base + out_off[i];
+					plane(out, base + out_off[i], d_out[i], part_bytes, part_stride, part_bytes, false);
+				}
+			}
+			if (d_chunk_out) plane(out, base + img_off, d_chunk_out, static_cast<size_t>(nb) * B, chunk_out_stride, static_cast<size_t>(nb) * B, false);
+			auto copy_rows = [&](RowsCopyArgs &a) -> int {
+				const unsigned n_planes = a.n_rows;
+				if (!n_planes) return LZGPU_OK;
+				a.n_rows = ng;
+				a.idx = static_cast<const uint32_t *>(t_idx.p);
+				const dim3 grid(static_cast<unsigned>(std::max(1, std::min(ctx->sm_count * 8 / static_cast<int>(n_planes) + 1, 1024))), n_planes);
+				rows_copy_kernel<<<grid, 256, 0, st>>>(a);
+				CUDA_TRY(cudaGetLastError());
+				ctx->stats.kernel_launches++;
+				return LZGPU_OK;
+			};
+			if ((rc = copy_rows(in))) return fail(rc);
+			if ((rc = recover_enqueue(ctx, goal, ng, nb, dp, part_bytes, any_crc ? dc : nullptr, want, dout, d_chunk_out ? base + img_off : nullptr,
+			                          static_cast<size_t>(nb) * B, st, &tk)))
+				return fail(rc);
+			if ((rc = copy_rows(out))) { ticket_drop(ctx, &tk); return fail(rc); }
+			tk.chunk_of = std::make_shared<const std::vector<uint32_t>>(list);
+		}
+		if (tk.active()) tks->push_back(tk);
+	}
+	return LZGPU_OK;
+}
+
+static int masked_check_args(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t nb, const lzgpu_chunk_mask *masks, const void *parts) {
+	if (!ctx || !masks || !parts) return LZGPU_ERR_ARG;
+	int rc = check_goal(goal);
+	if (rc) return rc;
+	if (nb == 0 || nb > LZGPU_BLOCKS_IN_CHUNK) { lz_set_error("nb out of range"); return LZGPU_ERR_ARG; }
+	return LZGPU_OK;
+}
+
+// store_ok of masked_route: data parts with an output buffer
+static uint64_t masked_store_ok(int k, const void *const *out) {
+	uint64_t s = 0;
+	for (int j = 0; j < k && out; ++j) s |= out[j] ? (1ull << j) : 0;
+	return s;
+}
+
+extern "C" int lzgpu_recover_chunks_masked_dev(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chunks, uint32_t nb, const lzgpu_chunk_mask *masks,
+                                                const void *const *d_parts, size_t part_stride, const void *const *d_part_crc, void *const *d_out,
+                                                void *d_chunk_out, size_t chunk_out_stride, int64_t *bad, void *stream) {
+	NvtxScope nvtx_scope("lzgpu::recover_chunks_masked_dev");
+	int rc = masked_check_args(ctx, goal, nb, masks, d_parts);
+	if (rc) return rc;
+	if (n_chunks == 0) return LZGPU_OK;
+	const int k = goal->k, n = goal->k + goal->m;
+	const uint32_t pb = (nb + k - 1) / k;
+	if (part_stride < static_cast<size_t>(pb) * LZGPU_BLOCK_SIZE || (part_stride & 15)) { lz_set_error("recover_masked: bad part_stride"); return LZGPU_ERR_ARG; }
+	if (d_chunk_out && (chunk_out_stride < static_cast<size_t>(nb) * LZGPU_BLOCK_SIZE || (chunk_out_stride & 15))) {
+		lz_set_error("recover_masked: chunk_out_stride must cover nb blocks and be a multiple of 16");
+		return LZGPU_ERR_ARG;
+	}
+	bool verify = false;
+	for (int i = 0; i < n && d_part_crc; ++i) verify |= d_part_crc[i] != nullptr;
+	const MaskedRouting R = masked_routing(goal, n_chunks, masks, d_chunk_out != nullptr, verify, masked_store_ok(k, d_out));
+	if (R.too_few_chunk >= 0) return masked_too_few(R, k);
+	uint64_t avail_any = 0;
+	for (uint32_t c = 0; c < n_chunks; ++c) avail_any |= masks[c].available;
+	for (int i = 0; i < n; ++i)
+		if ((avail_any >> i & 1) && !d_parts[i]) { lz_set_error("recover_masked: part %d is available in some chunk but d_parts[%d] is NULL", i, i); return LZGPU_ERR_ARG; }
+	DeviceGuard g(ctx->device);
+	cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+	std::vector<VerifyTicket> tks;
+	{
+		BatchTimer timer(ctx, st, masked_alg_bytes(goal, nb, R, d_chunk_out != nullptr, d_part_crc != nullptr));
+		if ((rc = masked_enqueue(ctx, goal, n_chunks, nb, R, d_parts, part_stride, d_part_crc, d_out, d_chunk_out, chunk_out_stride, st, &tks)))
+			return rc;
+	}
+	if (tks.empty()) return LZGPU_OK;
+	if (ctx->deferred_verify.load()) {  // the verdicts are collected by lzgpu_dev_sync
+		std::lock_guard<std::mutex> lk(ctx->pending_mu);
+		ctx->pending.insert(ctx->pending.end(), tks.begin(), tks.end());
+		return LZGPU_OK;
+	}
+	cudaError_t e = cudaStreamSynchronize(st);
+	if (e != cudaSuccess) {
+		tickets_drop(ctx, &tks);
+		cudaGetLastError();
+		lz_set_error("CUDA error %s while waiting for the verification result", cudaGetErrorName(e));
+		return LZGPU_ERR_CUDA;
+	}
+	return tickets_result(ctx, &tks, bad);
+}
+
+// host pointers: the tiles of lzgpu_recover_chunks (three slots, H2D | kernel | D2H); only the regions of available parts are copied in,
+// only the rebuilt regions copied out
+struct MaskedSlotState {
+	std::vector<VerifyTicket> tks;
+	uint32_t c0 = 0;
+	bool busy = false;
+};
+
+static int masked_retire_slot(lzgpu_ctx *ctx, int s, MaskedSlotState *ss, int64_t *bad) {
+	if (!ss->busy) return LZGPU_OK;
+	ss->busy = false;
+	cudaError_t e = cudaStreamSynchronize(ctx->slot_stream[s]);
+	if (e != cudaSuccess) {
+		tickets_drop(ctx, &ss->tks);
+		cudaGetLastError();
+		lz_set_error("CUDA error %s in the host pipeline", cudaGetErrorName(e));
+		return LZGPU_ERR_CUDA;
+	}
+	int64_t local[3] = {-1, -1, -1};
+	const int rc = tickets_result(ctx, &ss->tks, local);
+	if (rc == LZGPU_ERR_CRC && bad) { bad[0] = local[0] + ss->c0; bad[1] = local[1]; bad[2] = local[2]; }
+	return rc;
+}
+
+static void masked_drain_slots(lzgpu_ctx *ctx, MaskedSlotState *ss) {
+	for (int s = 0; s < kHostSlots; ++s) {
+		cudaStreamSynchronize(ctx->slot_stream[s]);
+		tickets_drop(ctx, &ss[s].tks);
+		ss[s].busy = false;
+	}
+	cudaGetLastError();
+}
+
+// runs [c, c_end) of chunks of a tile where bit i of bits(c) is set: fn(first chunk, count)
+template <typename Bits, typename Fn>
+static int for_runs(uint32_t c0, uint32_t nc, int i, Bits bits, Fn fn) {
+	for (uint32_t c = c0; c < c0 + nc;) {
+		if (!(bits(c) >> i & 1)) { ++c; continue; }
+		uint32_t e = c + 1;
+		while (e < c0 + nc && (bits(e) >> i & 1)) ++e;
+		const int rc = fn(c, e - c);
+		if (rc) return rc;
+		c = e;
+	}
+	return LZGPU_OK;
+}
+
+extern "C" int lzgpu_recover_chunks_masked(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chunks, uint32_t nb, const lzgpu_chunk_mask *masks,
+                                            const uint8_t *const *parts, size_t part_stride, const uint32_t *const *part_crc, uint8_t *const *out,
+                                            uint8_t *chunk_out, size_t chunk_out_stride, int64_t *bad) {
+	NvtxScope nvtx_scope("lzgpu::recover_chunks_masked");
+	int rc = masked_check_args(ctx, goal, nb, masks, parts);
+	if (rc) return rc;
+	if (n_chunks == 0) return LZGPU_OK;
+	const int k = goal->k, n = goal->k + goal->m;
+	const uint32_t B = LZGPU_BLOCK_SIZE;
+	const uint32_t pb = (nb + k - 1) / k;
+	const size_t part_bytes = static_cast<size_t>(pb) * B;
+	if (part_stride < part_bytes) { lz_set_error("recover_masked: part_stride too small"); return LZGPU_ERR_ARG; }
+	if (chunk_out && chunk_out_stride < static_cast<size_t>(nb) * B) { lz_set_error("recover_masked: chunk_out_stride too small"); return LZGPU_ERR_ARG; }
+	// every chunk is checked before anything is enqueued
+	const MaskedRouting all = masked_routing(goal, n_chunks, masks, chunk_out != nullptr, true, ~0ull);
+	if (all.too_few_chunk >= 0) return masked_too_few(all, k);
+	for (uint32_t c = 0; c < n_chunks; ++c)
+		for (int i = 0; i < n; ++i)
+			if ((masks[c].available >> i & 1) && !parts[i]) { lz_set_error("recover_masked: part %d is available in some chunk but parts[%d] is NULL", i, i); return LZGPU_ERR_ARG; }
+	auto rebuilt = [&](uint32_t c) { return all.pattern[c].rebuilt; };
+	auto avail = [&](uint32_t c) { return masks[c].available; };
+	std::lock_guard<std::mutex> lk(ctx->mu);
+	DeviceGuard g(ctx->device);
+	AutoPin pin(ctx);
+	for (int i = 0; i < n; ++i) {
+		if (parts[i]) pin.add(parts[i], static_cast<size_t>(n_chunks - 1) * part_stride + part_bytes);
+		else if (out && out[i]) pin.add(out[i], static_cast<size_t>(n_chunks - 1) * part_stride + part_bytes);
+	}
+	if (chunk_out) pin.add(chunk_out, static_cast<size_t>(n_chunks - 1) * chunk_out_stride + static_cast<size_t>(nb) * B);
+	const uint32_t tile = static_cast<uint32_t>(std::max<size_t>(1, std::min<size_t>(n_chunks, (2 * kHostTileBytes) / (part_bytes * k))));
+	const size_t dev_part = static_cast<size_t>(tile) * part_bytes;
+	const size_t dev_crc = static_cast<size_t>(tile) * pb * 4;
+	void *d_all[kHostSlots], *d_crc_all[kHostSlots], *d_img[kHostSlots] = {nullptr, nullptr, nullptr};
+	const int n_slots = n_chunks > tile ? kHostSlots : 1;
+	for (int s = 0; s < n_slots; ++s) {
+		if ((rc = lz_scratch(ctx, kScratchIn0 + s, dev_part * n, &d_all[s]))) return rc;
+		if ((rc = lz_scratch(ctx, kScratchCrc0 + s, dev_crc * n, &d_crc_all[s]))) return rc;
+		if (chunk_out && (rc = lz_scratch(ctx, kScratchPar0 + s, static_cast<size_t>(tile) * nb * B, &d_img[s]))) return rc;
+	}
+	MaskedSlotState ss[kHostSlots];
+	uint32_t t = 0;
+	for (uint32_t c0 = 0; c0 < n_chunks; c0 += tile, ++t) {
+		const uint32_t nc = std::min(tile, n_chunks - c0);
+		const int s = static_cast<int>(t % n_slots);
+		if ((rc = masked_retire_slot(ctx, s, &ss[s], bad))) { masked_drain_slots(ctx, ss); return rc; }
+		cudaStream_t st = ctx->slot_stream[s];
+		// a part's device region serves as input for the chunks that have it and as output for the chunks that rebuild it
+		std::vector<const void *> dp(n, nullptr), dc(n, nullptr);
+		std::vector<void *> dout(n, nullptr);
+		bool any_crc = false;
+		for (int i = 0; i < n; ++i) {
+			uint8_t *slot = static_cast<uint8_t *>(d_all[s]) + dev_part * i;
+			uint8_t *cs = static_cast<uint8_t *>(d_crc_all[s]) + dev_crc * i;
+			if (parts[i]) {
+				dp[i] = slot;
+				rc = for_runs(c0, nc, i, avail, [&](uint32_t c, uint32_t cnt) -> int {
+					CUDA_TRY(cudaMemcpy2DAsync(slot + static_cast<size_t>(c - c0) * part_bytes, part_bytes, parts[i] + static_cast<size_t>(c) * part_stride,
+					                           part_stride, part_bytes, cnt, cudaMemcpyHostToDevice, st));
+					ctx->stats.bytes_h2d += static_cast<uint64_t>(cnt) * part_bytes;
+					if (part_crc && part_crc[i]) {
+						CUDA_TRY(cudaMemcpyAsync(cs + static_cast<size_t>(c - c0) * pb * 4, part_crc[i] + static_cast<size_t>(c) * pb,
+						                         static_cast<size_t>(cnt) * pb * 4, cudaMemcpyHostToDevice, st));
+					}
+					return LZGPU_OK;
+				});
+				if (rc) { masked_drain_slots(ctx, ss); return rc; }
+				if (part_crc && part_crc[i]) { dc[i] = cs; any_crc = true; }
+			}
+			if (out && out[i]) dout[i] = slot;
+		}
+		const MaskedRouting R = masked_routing(goal, nc, masks + c0, chunk_out != nullptr, any_crc, masked_store_ok(k, dout.data()));
+		ss[s].c0 = c0;
+		{
+			BatchTimer timer(ctx, st, masked_alg_bytes(goal, nb, R, chunk_out != nullptr, any_crc));
+			rc = masked_enqueue(ctx, goal, nc, nb, R, dp.data(), part_bytes, any_crc ? dc.data() : nullptr, dout.data(), d_img[s],
+			                    static_cast<size_t>(nb) * B, st, &ss[s].tks);
+		}
+		if (rc) { masked_drain_slots(ctx, ss); return rc; }
+		ss[s].busy = true;
+		for (int i = 0; i < n; ++i) {
+			if (!dout[i]) continue;
+			uint8_t *slot = static_cast<uint8_t *>(dout[i]);
+			rc = for_runs(c0, nc, i, rebuilt, [&](uint32_t c, uint32_t cnt) -> int {
+				CUDA_TRY(cudaMemcpy2DAsync(out[i] + static_cast<size_t>(c) * part_stride, part_stride, slot + static_cast<size_t>(c - c0) * part_bytes,
+				                           part_bytes, part_bytes, cnt, cudaMemcpyDeviceToHost, st));
+				ctx->stats.bytes_d2h += static_cast<uint64_t>(cnt) * part_bytes;
+				return LZGPU_OK;
+			});
+			if (rc) { masked_drain_slots(ctx, ss); return rc; }
+		}
+		if (chunk_out) {
+			CUDA_TRY(cudaMemcpy2DAsync(chunk_out + static_cast<size_t>(c0) * chunk_out_stride, chunk_out_stride, d_img[s], static_cast<size_t>(nb) * B,
+			                           static_cast<size_t>(nb) * B, nc, cudaMemcpyDeviceToHost, st));
+			ctx->stats.bytes_d2h += static_cast<uint64_t>(nc) * nb * B;
+		}
+	}
+	for (uint32_t i = 0; i < static_cast<uint32_t>(n_slots); ++i) {
+		const int s = static_cast<int>((t + i) % n_slots);
+		if ((rc = masked_retire_slot(ctx, s, &ss[s], bad))) { masked_drain_slots(ctx, ss); return rc; }
 	}
 	return LZGPU_OK;
 }

@@ -5,6 +5,7 @@
 #include <atomic>
 #include <cstddef>
 #include <cstdint>
+#include <memory>
 #include <mutex>
 #include <vector>
 
@@ -64,6 +65,9 @@ struct VerifyTicket {
 	bool fused = false;    // fused route: one word (chunk*64 + part)*1024 + block; otherwise one word per part: chunk*blocks + block
 	int n_words = 0;
 	uint32_t blocks = 0;   // blocks per chunk of a verified part (generic encoding)
+	// the reported chunk is chunk_of[chunk] (a compact copy of some chunks of a call) or chunk + chunk_base (a run of them)
+	std::shared_ptr<const std::vector<uint32_t>> chunk_of;
+	uint32_t chunk_base = 0;
 	bool active() const { return slot.index >= 0; }
 };
 
@@ -163,6 +167,13 @@ int lz_fused_encode_split(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chu
 int lz_fused_recover(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chunks, uint32_t nb, const void *const *d_parts, size_t part_stride,
                      const void *const *d_part_crc, const uint8_t *want, void *const *d_out, void *d_chunk_out, size_t chunk_out_stride,
                      cudaStream_t st, unsigned long long *d_first_bad, bool *verifying);
+// Degraded read with a loss pattern per chunk (fused_recover_kernel's per-chunk descriptor mode): one launch per rebuilt-part count e,
+// over the e_chunks[e - 1] descriptors that follow those of the smaller counts in d_desc (device memory, fused_plan.h MaskedChunkDesc).
+// Parts, CRCs and outputs are indexed by part, chunk c at + c*stride as in lz_fused_recover; verification as there.
+namespace lzd { struct MaskedChunkDesc; }
+int lz_fused_recover_masked(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chunks, uint32_t nb, const void *const *d_parts, size_t part_stride,
+                            const void *const *d_part_crc, void *const *d_out, void *d_chunk_out, size_t chunk_out_stride,
+                            const lzd::MaskedChunkDesc *d_desc, const uint32_t *e_chunks, cudaStream_t st, unsigned long long *d_first_bad);
 // Fused slice conversion (convert_kernel.cuh): k parts of the source slice -> every wanted part of the destination slice (d_out[i],
 // nullptr = not wanted) + the destination slice's block CRCs in chunk order (nb data blocks, then m x pbd parity blocks per chunk),
 // one pass; verification as in lz_fused_recover.  LZGPU_NOT_HANDLED = take the two-pass route.

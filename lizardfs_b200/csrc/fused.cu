@@ -111,8 +111,16 @@ static int set_all_convert_attrs() {
 	return LZGPU_OK;
 }
 
+template <int E>
+constexpr int kMaskedWords = recover_item_words(E, 2);
+template <int E>
+static int set_masked_attr(int bytes) {  // per-chunk descriptor mode (lz_fused_recover_masked)
+	CUDA_TRY(cudaFuncSetAttribute(fused_recover_kernel<E, 0, -1, -1, 64, 2, kMaskedWords<E>, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+	CUDA_TRY(cudaFuncSetAttribute(fused_recover_kernel<E, 0, kRecoverDirect, -1, 64, 2, kDirectWide<E>, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+	return LZGPU_OK;
+}
 // function attributes are per device: done once per context
-static int set_all_recover_attrs() {
+static int set_all_recover_attrs(int max_smem) {
 	int rc;
 	if ((rc = set_recover_attr<1, 8, 0>())) return rc;
 	if ((rc = set_recover_attr<1, 0, 0>())) return rc;
@@ -136,6 +144,8 @@ static int set_all_recover_attrs() {
 	CUDA_TRY(cudaFuncSetAttribute(bs_recover3_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, kRecoverSmemCapBig));
 	// DIRECT (any generator; Cauchy codes): 16-warp geometry, 4-byte items
 	if ((rc = set_direct_attr<1>()) || (rc = set_direct_attr<2>()) || (rc = set_direct_attr<3>()) || (rc = set_direct_attr<4>())) return rc;
+	const int masked = std::min(max_smem, kMaskedSmemCap);
+	if ((rc = set_masked_attr<1>(masked)) || (rc = set_masked_attr<2>(masked)) || (rc = set_masked_attr<3>(masked)) || (rc = set_masked_attr<4>(masked))) return rc;
 	return LZGPU_OK;
 }
 
@@ -245,7 +255,7 @@ int lz_fused_init(lzgpu_ctx *ctx) {
 	if ((rc = set_smem_attr<3, false, 5, 8, 128>(smem128))) return rc;
 #endif
 	if ((rc = set_all_bs_attrs())) return rc;
-	if ((rc = set_all_recover_attrs())) return rc;
+	if ((rc = set_all_recover_attrs(fs->max_smem))) return rc;
 	if ((rc = set_all_convert_attrs())) return rc;
 	return LZGPU_OK;
 }
@@ -802,6 +812,85 @@ int lz_fused_recover(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chunks, 
 			if (r01) return launch_recover<4, 0, 0, 1>(ctx, maps, p, smem, st, pl.geo);
 			return launch_recover<4, 0>(ctx, maps, p, smem, st, pl.geo);
 	}
+}
+
+// ---------------------------------------------------------------------------------------------------
+// degraded read with a loss pattern per chunk: fused_recover_kernel in its per-chunk descriptor mode
+// ---------------------------------------------------------------------------------------------------
+template <int E>
+static void launch_masked(int grid, size_t smem, cudaStream_t st, bool direct, const TmapArray64 &maps, const MaskedRecoverParams &p) {
+	if (direct) fused_recover_kernel<E, 0, kRecoverDirect, -1, 64, 2, kDirectWide<E>, true><<<grid, recover_threads(2), smem, st>>>(maps, p);
+	else fused_recover_kernel<E, 0, -1, -1, 64, 2, kMaskedWords<E>, true><<<grid, recover_threads(2), smem, st>>>(maps, p);
+}
+
+int lz_fused_recover_masked(lzgpu_ctx *ctx, const lzgpu_goal *goal, uint32_t n_chunks, uint32_t nb, const void *const *d_parts, size_t part_stride,
+                            const void *const *d_part_crc, void *const *d_out, void *d_chunk_out, size_t chunk_out_stride,
+                            const MaskedChunkDesc *d_desc, const uint32_t *e_chunks, cudaStream_t st, unsigned long long *d_first_bad) {
+	FusedState *fs = ctx->fused;
+	const int K = goal->k, N = goal->k + goal->m;
+	const MaskedGeometry geo = masked_geometry(K, nb);
+	if (!fs || !geo.ok || geo.smem > static_cast<size_t>(fs->max_smem)) {
+		lz_set_error("recover_masked: no masked geometry for k = %d", K);
+		return LZGPU_ERR_ARG;
+	}
+	MaskedRecoverParams p{};
+	p.image = static_cast<uint8_t *>(d_chunk_out);
+	p.out_stride = part_stride;
+	p.image_stride = chunk_out_stride;
+	p.tables = ctx->d_crc_tables;
+	p.first_bad = d_first_bad;
+	p.n_chunks = n_chunks;
+	p.nb = nb;
+	p.pb = geo.pb;
+	p.K = static_cast<uint32_t>(K);
+	p.G = geo.G;
+	p.units_per_chunk = geo.units_per_chunk;
+	p.n_stages = geo.n_stages;
+	p.raid6_dbl = p.elim3_dbl = 0xffu;
+	std::memcpy(p.qmult, fs->qmult64, sizeof(p.qmult));
+	p.zconst = lz::crc_of_zeros(LZGPU_BLOCK_SIZE);
+	for (int j = 0; j < K; ++j) p.out_part[j] = d_out ? static_cast<uint8_t *>(d_out[j]) : nullptr;
+	for (int i = 0; i < N; ++i) p.stored_part[i] = d_part_crc ? static_cast<const uint32_t *>(d_part_crc[i]) : nullptr;
+	p.crc_fixed = lzgpu_crc_enabled() ? 0u : 1u;
+	// one tensor map per part that some chunk reads (the chunk dimension spans the whole call)
+	TmapArray64 maps;
+	std::memset(&maps, 0, sizeof(maps));
+	for (int i = 0; i < N; ++i) {
+		if (!d_parts[i]) continue;
+		const cuuint64_t dims[3] = {static_cast<cuuint64_t>(kRowBytes), static_cast<cuuint64_t>(geo.pb) * 4, n_chunks};
+		const cuuint64_t strides[2] = {static_cast<cuuint64_t>(kRowBytes), part_stride};
+		const cuuint32_t box[3] = {kStepBytes, geo.G * 4, 1};
+		const cuuint32_t estr[3] = {1, 1, 1};
+		CUresult r = fs->encode_tiled(&maps.m[i], CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void *>(d_parts[i]), dims, strides, box, estr,
+		                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, static_cast<CUtensorMapL2promotion>(fs->promo),
+		                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+		if (r != CUDA_SUCCESS) {
+			lz_set_error("recover_masked: cuTensorMapEncodeTiled failed with CUresult %d for part %d", static_cast<int>(r), i);
+			return LZGPU_ERR_CUDA;
+		}
+	}
+	const bool direct = lz::uses_cauchy(K, goal->m);
+	uint32_t first = 0;
+	for (int e = 1; e <= 4; ++e) {
+		const uint32_t n = e_chunks[e - 1];
+		if (!n) continue;
+		p.desc = d_desc + first;
+		p.e = static_cast<uint32_t>(e);
+		const uint64_t total = static_cast<uint64_t>(geo.units_per_chunk) * n;
+		if (total > 0x7fffffffull) { lz_set_error("recover_masked: too many work units"); return LZGPU_ERR_ARG; }
+		p.total_units = static_cast<uint32_t>(total);
+		const int grid = static_cast<int>(std::min<uint64_t>(total, static_cast<uint64_t>(ctx->sm_count)));
+		switch (e) {
+			case 1: launch_masked<1>(grid, geo.smem, st, direct, maps, p); break;
+			case 2: launch_masked<2>(grid, geo.smem, st, direct, maps, p); break;
+			case 3: launch_masked<3>(grid, geo.smem, st, direct, maps, p); break;
+			default: launch_masked<4>(grid, geo.smem, st, direct, maps, p); break;
+		}
+		CUDA_TRY(cudaGetLastError());
+		ctx->stats.kernel_launches++;
+		first += n;
+	}
+	return LZGPU_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------

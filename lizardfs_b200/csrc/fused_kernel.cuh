@@ -41,6 +41,8 @@
 #pragma once
 #include <cuda.h>
 
+#include <type_traits>
+
 #include "bitslice.cuh"
 #include "device_math.cuh"
 #include "fused_plan.h"
@@ -706,6 +708,25 @@ struct RecoverParams {
 	CoefPlanes rw[4 * 32];
 };
 
+// Per-chunk descriptor mode (MASKED instantiations, lzgpu_recover_chunks_masked*): every chunk of the launch has its own loss pattern.
+// What depends on the pattern (the slot -> part list, erased parts, parity rows, V^-1 or the DIRECT rows) comes from desc[unit chunk]
+// (MaskedChunkDesc, fused_plan.h), copied to shared memory when a work unit starts, coefficients expanded to CoefPlanes there.
+// The TMA maps, part outputs and stored CRCs are indexed by PART, so any chunk can use any part.
+struct MaskedRecoverParams : RecoverParams {
+	const MaskedChunkDesc *desc;   // one per chunk of this launch; unit u belongs to desc[u / units_per_chunk]
+	uint8_t *out_part[32];         // rebuilt data part j of chunk c at out_part[j] + c*out_stride (nullptr: not wanted)
+	const uint32_t *stored_part[64];   // stored CRCs of part i (chunk c at + c*pb) or nullptr = not verified
+	uint32_t crc_fixed;            // CRCs disabled (lzgpu_set_crc_enabled): a stored CRC is valid iff it equals LZGPU_FAKE_CRC
+};
+static_assert(sizeof(CoefPlanes) == kCoefPlanesBytes, "masked shared-memory layout (fused_plan.h masked_geometry)");
+struct TmapArray64 {
+	CUtensorMap m[64];
+};
+template <bool MASKED>
+using RecoverMaps = typename std::conditional<MASKED, TmapArray64, TmapArray>::type;
+template <bool MASKED>
+using RecoverArgs = typename std::conditional<MASKED, MaskedRecoverParams, RecoverParams>::type;
+
 // E = erased data parts; KT = compile-time K (0 = runtime); R0, R1 = generator rows of the first two parity
 // parts in use when known at compile time (-1 = read p.par_row): the RAID-6 shapes (row 0 = XOR, row 1 = powers of 2)
 // get constant doubling counts and the "last unknown = S0 ^ others" shortcut.
@@ -721,9 +742,11 @@ struct RecoverParams {
 // the elimination forms end their item with `continue` under a template-constant condition: the general solve below them is
 // dead code in those instantiations (warning 128)
 #pragma nv_diag_suppress 128
-template <int E, int KT, int R0, int R1, int kRecoverFW, int GEO = 0, int W = recover_item_words(E, GEO)>
+// MASKED: per-chunk descriptor mode (MaskedRecoverParams above; GEO 2, runtime k and parity rows, or the DIRECT form)
+template <int E, int KT, int R0, int R1, int kRecoverFW, int GEO = 0, int W = recover_item_words(E, GEO), bool MASKED = false>
 __global__ void __launch_bounds__(recover_threads(GEO), GEO == 1 ? 2 : 1)
-fused_recover_kernel(const __grid_constant__ TmapArray tmaps, const __grid_constant__ RecoverParams p) {
+fused_recover_kernel(const __grid_constant__ RecoverMaps<MASKED> tmaps, const __grid_constant__ RecoverArgs<MASKED> p) {
+	static_assert(!MASKED || (GEO == 2 && KT == 0 && R1 == -1 && (R0 == -1 || R0 == kRecoverDirect)), "masked: runtime k and parity rows");
 	constexpr int kThreads = recover_threads(GEO);
 	const uint32_t kRecoverStages = GEO == 2 ? p.n_stages : static_cast<uint32_t>(recover_stages(GEO));
 	extern __shared__ __align__(1024) uint8_t smem[];
@@ -749,11 +772,20 @@ fused_recover_kernel(const __grid_constant__ TmapArray tmaps, const __grid_const
 	const uint32_t my_units = blockIdx.x < p.total_units ? (p.total_units - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
 	const uint32_t total_steps = my_units * kStepsPerUnit;
 
+	// (masked: c is the unit's chunk in this launch, its descriptor names the chunk of the call and the part of every slot)
 	auto issue_load = [&](uint32_t c, uint32_t gi, uint32_t step, uint32_t st) {
 		mbar_expect_tx(a_full + 8 * st, stage_bytes);
-		for (uint32_t a = 0; a < K; ++a)
-			tma_load_3d(sbase + st * stage_bytes + a * region_bytes, &tmaps.m[a], static_cast<int>(step * kStepBytes),
-			            static_cast<int>(gi * RG), static_cast<int>(c), a_full + 8 * st);
+		if constexpr (MASKED) {
+			const MaskedChunkDesc *d = p.desc + c;
+			const int cc = static_cast<int>(__ldg(&d->chunk));
+			for (uint32_t a = 0; a < K; ++a)
+				tma_load_3d(sbase + st * stage_bytes + a * region_bytes, &tmaps.m[__ldg(&d->part_of_slot[a])], static_cast<int>(step * kStepBytes),
+				            static_cast<int>(gi * RG), cc, a_full + 8 * st);
+		} else {
+			for (uint32_t a = 0; a < K; ++a)
+				tma_load_3d(sbase + st * stage_bytes + a * region_bytes, &tmaps.m[a], static_cast<int>(step * kStepBytes),
+				            static_cast<int>(gi * RG), static_cast<int>(c), a_full + 8 * st);
+		}
 	};
 
 	if (tid == 0) {
@@ -770,18 +802,48 @@ fused_recover_kernel(const __grid_constant__ TmapArray tmaps, const __grid_const
 
 	const bool has_stream = tid < ROWS;
 	const uint32_t slot = tid / RG, rr = tid % RG;           // this thread's stream: slot `slot`, block rr/4, quarter rr%4
-	const bool verify = has_stream && p.stored[has_stream ? slot : 0] != nullptr;
+	const bool verify0 = !MASKED && has_stream && p.stored[has_stream ? slot : 0] != nullptr;
 	const uint32_t row_addr0 = (sbase + tid * kStepBytes) ^ ((tid & 7) << 4);
 	const bool warp_has_items = cw < n_gf_warps;
+	// masked: the unit's descriptor and its coefficient planes, behind the stage ring and its barriers (host: masked_geometry)
+	MaskedChunkDesc *const md = reinterpret_cast<MaskedChunkDesc *>(smem + ((kRecoverStages * (stage_bytes + 16) + 64 + 127) & ~127u));
+	CoefPlanes *const mplanes = reinterpret_cast<CoefPlanes *>(reinterpret_cast<uint8_t *>(md) + sizeof(MaskedChunkDesc));
+	// what depends on the loss pattern: the launch's parameters, or the unit's descriptor
+	auto slot_of_data = [&](uint32_t j) -> uint32_t { if constexpr (MASKED) return md->slot_of_data[j]; else return p.slot_of_data[j]; };
+	auto data_of_slot = [&](uint32_t a) -> uint32_t {
+		if constexpr (MASKED) { const uint32_t i = md->part_of_slot[a]; return i < K ? i : 0xffu; } else return p.data_of_slot[a];
+	};
+	auto par_slot = [&](int r) -> uint32_t { if constexpr (MASKED) return md->par_slot[r]; else return p.par_slot[r]; };
+	auto par_row = [&](int r) -> uint32_t { if constexpr (MASKED) return md->par_row[r]; else return p.par_row[r]; };
+	auto erased_idx = [&](int x) -> uint32_t { if constexpr (MASKED) return md->erased_idx[x]; else return p.erased_idx[x]; };
+	auto part_id = [&](uint32_t a) -> uint32_t { if constexpr (MASKED) return md->part_of_slot[a]; else return p.part_id[a]; };
+	auto out_ptr = [&](int x) -> uint8_t * {
+		if constexpr (MASKED) return (md->store >> x & 1) ? p.out_part[md->erased_idx[x]] : nullptr; else return p.out[x];
+	};
+	auto stored_ptr = [&](uint32_t a) -> const uint32_t * { if constexpr (MASKED) return p.stored_part[md->part_of_slot[a]]; else return p.stored[a]; };
+	auto w_planes = [&](int i) -> const CoefPlanes & { if constexpr (MASKED) return mplanes[i]; else return p.w[i]; };
+	auto rw_planes = [&](int i) -> const CoefPlanes & { if constexpr (MASKED) return mplanes[i]; else return p.rw[i]; };
 
 	uint32_t win[kRecoverFW];
 	FoldAux aux;
 	uint32_t it = 0, st = 0, ph = 0;
 	for (uint32_t unit = blockIdx.x; unit < p.total_units; unit += gridDim.x) {
-		const uint32_t c = unit / p.units_per_chunk, gi = unit % p.units_per_chunk;
+		const uint32_t cu = unit / p.units_per_chunk, gi = unit % p.units_per_chunk;
 		const uint32_t stripe0 = gi * G;
 		const uint32_t next_unit = unit + gridDim.x;
 		const uint32_t next_c = next_unit / p.units_per_chunk, next_gi = next_unit % p.units_per_chunk;
+		if constexpr (MASKED) {
+			// every stage warp is done with the previous unit's descriptor; fetch this one, expand its coefficients, publish.  (The TMA
+			// loads of this unit's first steps were issued during the previous one: the pipeline does not drain here.)
+			asm volatile("bar.sync 1, %0;" ::"r"(n_stage_warps * 32) : "memory");
+			const MaskedChunkDesc *gd = p.desc + cu;
+			for (uint32_t i = tid; i < sizeof(MaskedChunkDesc) / 4; i += n_stage_warps * 32)
+				reinterpret_cast<uint32_t *>(md)[i] = __ldg(reinterpret_cast<const uint32_t *>(gd) + i);
+			for (uint32_t i = tid; i < kMaskedPlanes; i += n_stage_warps * 32) coef_planes_set(mplanes[i], __ldg(&gd->coef[i]));
+			asm volatile("bar.sync 1, %0;" ::"r"(n_stage_warps * 32) : "memory");
+		}
+		const uint32_t c = MASKED ? md->chunk : cu;   // chunk of the call: parts, CRCs, outputs, image
+		const bool verify = MASKED ? has_stream && stored_ptr(slot) != nullptr : verify0;
 #pragma unroll
 		for (int i = 0; i < kRecoverFW; ++i) win[i] = 0;
 #pragma unroll
@@ -815,29 +877,29 @@ fused_recover_kernel(const __grid_constant__ TmapArray tmaps, const __grid_const
 							for (uint32_t a = 0; a < K; ++a) {
 								uint32_t v[W];
 								lds_item<W>(a_item + a * region_bytes, v);
-								const uint32_t j = p.data_of_slot[a];
+								const uint32_t j = data_of_slot(a);
 								if (j != 0xffu) {
 									const uint32_t b = stripe * K + j;
 									if (img && b < p.nb) stg_item<W>(img + (static_cast<unsigned long long>(b) << 16), v);
 								}
 #pragma unroll
 								for (int x = 0; x < E; ++x) {
-									const CoefPlanes &cp = p.rw[x * 32 + a];
+									const CoefPlanes &cp = rw_planes(x * 32 + a);
 #pragma unroll
 									for (int w = 0; w < W; ++w) acc[x][w] = gf_mac<kMacNS>(acc[x][w], v[w], cp);
 								}
 							}
 #pragma unroll
 							for (int x = 0; x < E; ++x) {
-								if (p.out[x] && stripe < p.pb) stg_item<W>(p.out[x] + c * p.out_stride + (static_cast<unsigned long long>(stripe) << 16) + in_block, acc[x]);
-								const uint32_t b = stripe * K + p.erased_idx[x];
+								if (out_ptr(x) && stripe < p.pb) stg_item<W>(out_ptr(x) + c * p.out_stride + (static_cast<unsigned long long>(stripe) << 16) + in_block, acc[x]);
+								const uint32_t b = stripe * K + erased_idx(x);
 								if (img && b < p.nb) stg_item<W>(img + (static_cast<unsigned long long>(b) << 16), acc[x]);
 							}
 							continue;
 						}
 #pragma unroll
 						for (int j = static_cast<int>(K) - 1; j >= 0; --j) {
-							const uint32_t sl = p.slot_of_data[j];
+							const uint32_t sl = slot_of_data(j);
 							uint32_t v[W];
 #pragma unroll
 							for (int w = 0; w < W; ++w) v[w] = 0;
@@ -851,7 +913,7 @@ fused_recover_kernel(const __grid_constant__ TmapArray tmaps, const __grid_const
 								// (R0, R1) = (0, 1): the host guarantees that the parity rows in use are 0, 1, .., E-1, so row r multiplies
 								// by 2^r in one step; otherwise only row 0 may be known at compile time
 								const int fixed = (R0 == 0 && R1 == 1) ? r : (r == 0 ? R0 : -1);
-								const uint32_t dbl = fixed >= 0 ? static_cast<uint32_t>(fixed) : p.par_row[r];
+								const uint32_t dbl = fixed >= 0 ? static_cast<uint32_t>(fixed) : par_row(r);
 #pragma unroll
 								for (int w = 0; w < W; ++w) {
 									uint32_t a = acc[r][w];
@@ -872,7 +934,7 @@ fused_recover_kernel(const __grid_constant__ TmapArray tmaps, const __grid_const
 #pragma unroll
 						for (int r = 0; r < E; ++r) {
 							uint32_t pv[W];
-							lds_item<W>(a_item + p.par_slot[r] * region_bytes, pv);
+							lds_item<W>(a_item + par_slot(r) * region_bytes, pv);
 #pragma unroll
 							for (int w = 0; w < W; ++w) acc[r][w] ^= pv[w];
 						}
@@ -955,15 +1017,15 @@ fused_recover_kernel(const __grid_constant__ TmapArray tmaps, const __grid_const
 							} else {
 #pragma unroll
 								for (int r = 0; r < E; ++r) {
-									const CoefPlanes &cp = p.w[x * 4 + r];
+									const CoefPlanes &cp = w_planes(x * 4 + r);
 #pragma unroll
 									for (int w = 0; w < W; ++w) d[w] = gf_mac<kMacNS>(d[w], acc[r][w], cp);
 								}
 #pragma unroll
 								for (int w = 0; w < W; ++w) others[w] ^= d[w];
 							}
-							if (p.out[x] && stripe < p.pb) stg_item<W>(p.out[x] + c * p.out_stride + (static_cast<unsigned long long>(stripe) << 16) + in_block, d);
-							const uint32_t b = stripe * K + p.erased_idx[x];
+							if (out_ptr(x) && stripe < p.pb) stg_item<W>(out_ptr(x) + c * p.out_stride + (static_cast<unsigned long long>(stripe) << 16) + in_block, d);
+							const uint32_t b = stripe * K + erased_idx(x);
 							if (img && b < p.nb) stg_item<W>(img + (static_cast<unsigned long long>(b) << 16), d);
 						}
 					}
@@ -978,7 +1040,7 @@ fused_recover_kernel(const __grid_constant__ TmapArray tmaps, const __grid_const
 				__syncwarp();
 				if (lane == 0 && mbar_arrive_is_last(a_empty + 8 * st) && it + kRecoverStages < total_steps) {
 					asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-					if (step + kRecoverStages < kStepsPerUnit) issue_load(c, gi, step + kRecoverStages, st);
+					if (step + kRecoverStages < kStepsPerUnit) issue_load(cu, gi, step + kRecoverStages, st);
 					else issue_load(next_c, next_gi, step + kRecoverStages - kStepsPerUnit, st);
 				}
 				++it;
@@ -994,9 +1056,12 @@ fused_recover_kernel(const __grid_constant__ TmapArray tmaps, const __grid_const
 		if (verify && (rr & 3) == 0) {
 			const uint32_t s = stripe0 + (rr >> 2);
 			if (s < p.pb) {
-				const uint32_t have = lin ^ p.zconst;
-				const uint32_t want = __ldg(p.stored[slot] + static_cast<unsigned long long>(c) * p.pb + s);
-				if (have != want) atomicMin(p.first_bad, (static_cast<unsigned long long>(c) * 64ull + p.part_id[slot]) * 1024ull + s);
+				uint32_t have = lin ^ p.zconst;
+				if constexpr (MASKED) {
+					if (p.crc_fixed) have = LZGPU_FAKE_CRC;
+				}
+				const uint32_t want = __ldg(stored_ptr(slot) + static_cast<unsigned long long>(c) * p.pb + s);
+				if (have != want) atomicMin(p.first_bad, (static_cast<unsigned long long>(c) * 64ull + part_id(slot)) * 1024ull + s);
 			}
 		}
 	}

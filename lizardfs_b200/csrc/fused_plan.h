@@ -4,6 +4,9 @@
 #pragma once
 #include <cstddef>
 #include <cstdint>
+#include <map>
+#include <utility>
+#include <vector>
 
 #include "host_math.h"
 
@@ -495,6 +498,198 @@ inline RecoverPlan recover_plan(int K, int M, bool cauchy, const uint8_t *availa
 	pl.ctas_per_sm = pl.geo == 1 ? 2 : 1;
 	pl.threads = pl.geo == 2 ? static_cast<uint32_t>(kBsRecoverThreads) : static_cast<uint32_t>(recover_threads(pl.geo));
 	return pl;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Degraded read with a loss pattern per chunk (lzgpu_recover_chunks_masked*): routing, per-chunk descriptors and the geometry of
+// the masked instantiations fused_recover_kernel<E, 0, -1, -1, 64, 2, W, true> (DIRECT: <E, 0, kRecoverDirect, -1, 64, 2, W, true>).
+// ---------------------------------------------------------------------------------------------------
+// One descriptor per chunk of a masked launch, read by the kernel when a work unit starts (224 bytes).
+struct MaskedChunkDesc {
+	uint32_t chunk;               // index of the chunk in the call (addresses its parts, CRCs, outputs and image)
+	uint8_t e;                    // erased data parts = the launch's E
+	uint8_t store;                // bit x: rebuilt part x (data part erased_idx[x]) is stored to its part buffer
+	uint8_t pad0[2];
+	uint8_t part_of_slot[32];     // slot a -> part: the first k available parts of this chunk (TMA maps are indexed by part)
+	uint8_t slot_of_data[32];     // data part j -> slot, 0xff = erased
+	uint8_t erased_idx[4];        // erased data parts, ascending
+	uint8_t par_slot[4], par_row[4];  // parity parts in use: slot and generator row
+	uint8_t pad1[12];
+	uint8_t coef[128];            // raw coefficients: Vandermonde W = V^-1 as coef[x*4 + r]; DIRECT rows over the k slots as coef[x*32 + a]
+};
+static_assert(sizeof(MaskedChunkDesc) == 224, "descriptor layout");
+
+enum MaskedRoute { kMaskedDelegated = 0, kMaskedOneLaunch = 1, kMaskedFallback = 2 };
+
+// A chunk's loss pattern, normalised: the first k available parts (its inputs) and the parts it rebuilds (requested and lost; every
+// lost data part when the image is wanted).  Parts past the first k available ones do not matter.
+struct MaskedPattern {
+	uint64_t used = 0, rebuilt = 0;
+	uint32_t e = 0;               // lost data parts (all of them are among the unknowns the kernel solves for)
+	bool ok = false;              // false: fewer than k parts available
+	bool operator==(const MaskedPattern &o) const { return used == o.used && rebuilt == o.rebuilt; }
+	bool operator<(const MaskedPattern &o) const { return used != o.used ? used < o.used : rebuilt < o.rebuilt; }
+};
+
+inline MaskedPattern masked_pattern(int K, int M, uint64_t available, uint64_t want, bool image) {
+	MaskedPattern pt;
+	const int N = K + M;
+	const uint64_t all = N >= 64 ? ~0ull : ((1ull << N) - 1), data = (1ull << K) - 1;
+	available &= all;
+	int n = 0;
+	for (int i = 0; i < N && n < K; ++i)
+		if (available >> i & 1) { pt.used |= 1ull << i; ++n; }
+	if (n < K) return pt;
+	pt.ok = true;
+	pt.rebuilt = ~available & all & (want | (image ? data : 0));
+	for (int j = 0; j < K; ++j) pt.e += (available >> j & 1) ? 0 : 1;
+	return pt;
+}
+
+// Descriptor of one chunk for the masked kernel (pure host logic, shared by the launcher and lzgpu_debug_masked_chunk).
+// store_ok: bit j = data part j has an output buffer.  false: the chunk cannot take the masked kernel (a lost parity part is rebuilt,
+// no or more than four data parts are lost, or the Vandermonde syndrome system is singular) — the existing route takes it.
+inline bool masked_chunk_desc(int K, int M, bool cauchy, const MaskedPattern &pt, uint64_t store_ok, MaskedChunkDesc &d) {
+	d = MaskedChunkDesc{};
+	const uint64_t data = (1ull << K) - 1;
+	if (!pt.ok || pt.e < 1 || pt.e > 4 || (pt.rebuilt & ~data)) return false;
+	for (int j = 0; j < 32; ++j) d.slot_of_data[j] = 0xff;
+	uint32_t a = 0, n_par = 0, e = 0;
+	for (int i = 0; i < K + M; ++i) {
+		if (!(pt.used >> i & 1)) continue;
+		d.part_of_slot[a] = static_cast<uint8_t>(i);
+		if (i < K) d.slot_of_data[i] = static_cast<uint8_t>(a);
+		else { d.par_slot[n_par] = static_cast<uint8_t>(a); d.par_row[n_par] = static_cast<uint8_t>(i - K); ++n_par; }
+		++a;
+	}
+	for (int j = 0; j < K; ++j)
+		if (d.slot_of_data[j] == 0xff) {
+			d.erased_idx[e] = static_cast<uint8_t>(j);
+			if ((pt.rebuilt >> j & 1) && (store_ok >> j & 1)) d.store |= static_cast<uint8_t>(1u << e);
+			++e;
+		}
+	d.e = static_cast<uint8_t>(e);
+	if (!cauchy) {
+		uint8_t V[16], W[16];
+		recover_syndrome_matrix(d.par_row, d.erased_idx, e, V);
+		if (gf_invert_matrix(V, W, static_cast<int>(e)) != 0) return false;
+		for (uint32_t x = 0; x < e; ++x)
+			for (uint32_t r = 0; r < e; ++r) d.coef[x * 4 + r] = W[x * e + r];
+	} else {
+		// rows of the reference's inverted k x k system for the erased data parts, over the k used parts in slot order
+		uint8_t erased[64] = {0}, wanted[64] = {0}, rows[32 * 32];
+		for (int i = 0; i < K + M; ++i) erased[i] = (pt.used >> i & 1) ? 0 : 1;
+		for (uint32_t x = 0; x < e; ++x) wanted[d.erased_idx[x]] = 1;
+		bool singular = false;
+		if (lz::rs_recovery_matrix(K, M, erased, wanted, rows, &singular) != static_cast<int>(e)) return false;
+		for (uint32_t x = 0; x < e; ++x)
+			for (int s = 0; s < K; ++s) d.coef[x * 32 + s] = rows[x * K + s];
+	}
+	return true;
+}
+
+// geometry of the masked instantiations: one 16-warp CTA per SM, G as on geometry 2 of recover_plan (a function of k only), the stage
+// ring sized so that the unit's descriptor and its coefficient planes fit next to it
+constexpr int kMaskedSmemCap = 226 * 1024;
+constexpr uint32_t kMaskedPlanes = 4 * 32;   // CoefPlanes in shared memory (DIRECT: e x k; Vandermonde: the 4 x 4 of W)
+constexpr size_t kCoefPlanesBytes = 96;      // sizeof(CoefPlanes), device_math.cuh
+struct MaskedGeometry {
+	bool ok = false;
+	uint32_t G = 0, n_stages = 0, pb = 0, units_per_chunk = 0, threads = 512;
+	size_t smem = 0, extra_offset = 0;   // extra_offset: descriptor + planes, from the dynamic shared-memory base
+};
+inline MaskedGeometry masked_geometry(int K, uint32_t nb) {
+	MaskedGeometry g;
+	uint32_t best = 0, best16 = 0;
+	for (uint32_t gg = 2; gg <= 64; gg += 2) {
+		const uint32_t rows = K * gg * 4;
+		if (rows > 512 || 3 * static_cast<size_t>(rows) * kStepBytes + 256 > kRecoverSmemCapBig) break;
+		best = gg;
+		if (gg % 16 == 0) best16 = gg;
+	}
+	g.G = best16 ? best16 : best;
+	if (!g.G) return g;
+	const size_t stage = static_cast<size_t>(K) * g.G * 4 * kStepBytes;
+	const size_t extra = sizeof(MaskedChunkDesc) + kMaskedPlanes * kCoefPlanesBytes;
+	g.n_stages = recover_big_stages(K, g.G);
+	while (g.n_stages > 2 && g.n_stages * (stage + 16) + 64 + extra > static_cast<size_t>(kMaskedSmemCap)) --g.n_stages;
+	g.extra_offset = (g.n_stages * (stage + 16) + 64 + 127) & ~size_t(127);
+	g.smem = g.extra_offset + extra;
+	g.pb = (nb + K - 1) / K;
+	g.units_per_chunk = (g.pb + g.G - 1) / g.G;
+	g.ok = g.smem <= static_cast<size_t>(kMaskedSmemCap);
+	return g;
+}
+
+// How a batch with a pattern per chunk is served.  A batch whose chunks all share one normalised pattern is delegated whole to the
+// existing route (route kMaskedDelegated: today's kernels).  Otherwise chunks that rebuild data parts only, one to four of them, take the
+// masked kernel, one launch per rebuilt-part count e (kMaskedOneLaunch); the others — nothing lost among the inputs (verify and / or
+// image only), a lost parity part requested, more than four lost data parts, a singular system — go through the existing route, one
+// call per normalised pattern (kMaskedFallback; a pattern with nothing to do — nothing rebuilt, no image, nothing verified — needs no
+// call).  store_ok: bit j = data part j has an output buffer.
+struct MaskedRouting {
+	int too_few_chunk = -1;      // first chunk with fewer than k available parts (nothing else is filled in then)
+	int too_few_parts = 0;
+	bool delegated = false;
+	uint32_t patterns = 0;
+	std::vector<uint8_t> route;                        // per chunk
+	std::vector<MaskedPattern> pattern;                // per chunk
+	uint32_t e_chunks[4] = {0, 0, 0, 0};               // one-launch chunks per e
+	std::vector<MaskedChunkDesc> desc;                 // one-launch descriptors, e = 1 first, ascending chunk index within each e
+	std::vector<std::pair<MaskedPattern, std::vector<uint32_t>>> groups;   // fallback groups, ordered by their first chunk
+	uint32_t launches() const {
+		if (delegated) return 1;
+		uint32_t n = static_cast<uint32_t>(groups.size());
+		for (uint32_t c : e_chunks) n += c ? 1 : 0;
+		return n;
+	}
+};
+
+inline MaskedRouting masked_route(int K, int M, bool cauchy, uint32_t n_chunks, const uint64_t *available, const uint64_t *want, bool image,
+                                  bool verify, uint64_t store_ok) {
+	MaskedRouting R;
+	R.pattern.resize(n_chunks);
+	std::map<std::pair<uint64_t, uint64_t>, uint32_t> seen;
+	for (uint32_t c = 0; c < n_chunks; ++c) {
+		const MaskedPattern pt = masked_pattern(K, M, available[c], want[c], image);
+		if (!pt.ok) {
+			R.too_few_chunk = static_cast<int>(c);
+			const uint64_t all = K + M >= 64 ? ~0ull : ((1ull << (K + M)) - 1);
+			R.too_few_parts = __builtin_popcountll(available[c] & all);
+			return R;
+		}
+		R.pattern[c] = pt;
+		seen.emplace(std::make_pair(pt.used, pt.rebuilt), 0u);
+	}
+	R.patterns = static_cast<uint32_t>(seen.size());
+	R.delegated = R.patterns == 1;
+	R.route.assign(n_chunks, static_cast<uint8_t>(kMaskedDelegated));
+	if (R.delegated) return R;
+	std::vector<MaskedChunkDesc> by_e[4];
+	std::map<std::pair<uint64_t, uint64_t>, uint32_t> group_of;
+	for (uint32_t c = 0; c < n_chunks; ++c) {
+		const MaskedPattern &pt = R.pattern[c];
+		MaskedChunkDesc d;
+		if (masked_chunk_desc(K, M, cauchy, pt, store_ok, d)) {
+			d.chunk = c;
+			by_e[d.e - 1].push_back(d);
+			R.route[c] = kMaskedOneLaunch;
+			continue;
+		}
+		R.route[c] = kMaskedFallback;
+		if (!pt.rebuilt && !image && !verify) continue;
+		auto it = group_of.find(std::make_pair(pt.used, pt.rebuilt));
+		if (it == group_of.end()) {
+			it = group_of.emplace(std::make_pair(pt.used, pt.rebuilt), static_cast<uint32_t>(R.groups.size())).first;
+			R.groups.emplace_back(pt, std::vector<uint32_t>());
+		}
+		R.groups[it->second].second.push_back(c);
+	}
+	for (int e = 0; e < 4; ++e) {
+		R.e_chunks[e] = static_cast<uint32_t>(by_e[e].size());
+		R.desc.insert(R.desc.end(), by_e[e].begin(), by_e[e].end());
+	}
+	return R;
 }
 
 }  // namespace lzd

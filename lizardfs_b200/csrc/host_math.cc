@@ -530,6 +530,76 @@ int lzgpu_plan_recover(const lzgpu_goal *g, const uint8_t *available, const uint
 	return LZGPU_OK;
 }
 
+int lzgpu_plan_recover_masked(const lzgpu_goal *g, uint32_t n_chunks, uint32_t nb, const lzgpu_chunk_mask *masks, int verify, int image,
+                              size_t part_stride, size_t chunk_out_stride, uint8_t *route, lzgpu_masked_plan *out) {
+	if (!out || !lzgpu_goal_valid(g) || g->kind == LZGPU_KIND_STD || (n_chunks && !masks) || nb == 0 || nb > LZGPU_BLOCKS_IN_CHUNK) return LZGPU_ERR_ARG;
+	*out = lzgpu_masked_plan{};
+	const uint32_t pb = (nb + g->k - 1) / g->k;
+	if (part_stride < static_cast<size_t>(pb) * LZGPU_BLOCK_SIZE || (part_stride & 15)) return LZGPU_ERR_ARG;
+	if (image && (chunk_out_stride < static_cast<size_t>(nb) * LZGPU_BLOCK_SIZE || (chunk_out_stride & 15))) return LZGPU_ERR_ARG;
+	std::vector<uint64_t> avail(n_chunks), want(n_chunks);
+	for (uint32_t c = 0; c < n_chunks; ++c) { avail[c] = masks[c].available; want[c] = masks[c].want; }
+	const bool cauchy = lz::uses_cauchy(g->k, g->m);
+	const lzd::MaskedRouting R = lzd::masked_route(g->k, g->m, cauchy, n_chunks, avail.data(), want.data(), image != 0, verify != 0, ~0ull);
+	if (R.too_few_chunk >= 0) return LZGPU_ERR_TOO_FEW_PARTS;
+	out->delegated = R.delegated ? 1 : 0;
+	out->patterns = R.patterns;
+	out->fallback_groups = static_cast<uint32_t>(R.groups.size());
+	out->rebuild_launches = n_chunks ? R.launches() : 0;
+	for (int e = 0; e < 4; ++e) {
+		out->e_chunks[e] = R.e_chunks[e];
+		out->one_launch_chunks += R.e_chunks[e];
+		out->item_words[e] = static_cast<uint32_t>(cauchy ? lzd::recover_direct_wide_words(e + 1) : lzd::recover_item_words(e + 1, 2));
+	}
+	for (uint32_t c = 0; c < n_chunks && !R.delegated; ++c) out->fallback_chunks += R.route[c] == lzd::kMaskedFallback ? 1u : 0u;
+	const lzd::MaskedGeometry geo = lzd::masked_geometry(g->k, nb);
+	out->form = cauchy ? lzd::kRecoverDirectForm : lzd::kRecoverPacked;
+	out->stripes_per_unit = geo.G;
+	out->stages = geo.n_stages;
+	out->units_per_chunk = geo.units_per_chunk;
+	out->threads_per_cta = geo.threads;
+	out->smem_bytes = static_cast<uint32_t>(geo.smem);
+	out->desc_bytes = static_cast<uint32_t>(sizeof(lzd::MaskedChunkDesc));
+	if (route)
+		for (uint32_t c = 0; c < n_chunks; ++c) route[c] = R.route[c];
+	return LZGPU_OK;
+}
+
+int lzgpu_debug_masked_chunk(const lzgpu_goal *g, const lzgpu_chunk_mask *mask, int image, lzgpu_masked_chunk *out) {
+	if (!out || !mask || !lzgpu_goal_valid(g) || g->kind == LZGPU_KIND_STD) return LZGPU_ERR_ARG;
+	*out = lzgpu_masked_chunk{};
+	const int K = g->k, M = g->m;
+	const bool cauchy = lz::uses_cauchy(K, M);
+	const lzd::MaskedPattern pt = lzd::masked_pattern(K, M, mask->available, mask->want, image != 0);
+	if (!pt.ok) return LZGPU_ERR_TOO_FEW_PARTS;
+	lzd::MaskedChunkDesc d;
+	const bool one = lzd::masked_chunk_desc(K, M, cauchy, pt, ~0ull, d);
+	for (int a = 0, i = 0; i < K + M; ++i)
+		if (pt.used >> i & 1) out->used[a++] = static_cast<uint8_t>(i);
+	if (!one) return LZGPU_OK;
+	out->one_launch = 1;
+	out->e = d.e;
+	for (uint32_t x = 0; x < d.e; ++x) out->erased[x] = d.erased_idx[x];
+	for (uint32_t x = 0; x < d.e; ++x)
+		for (int a = 0; a < K; ++a) {
+			if (cauchy) { out->rows[x * 32 + a] = d.coef[x * 32 + a]; continue; }
+			// d_x = sum_r W[x][r] (p_r ^ sum_{j kept} g_r^j d_j): the coefficient of an input is W[x][r] for parity row r, and
+			// sum_r W[x][r] g_r^j for data part j
+			const int part = d.part_of_slot[a];
+			uint8_t v = 0;
+			for (uint32_t r = 0; r < d.e; ++r) {
+				const uint8_t w = d.coef[x * 4 + r];
+				if (part >= K) { if (d.par_slot[r] == a) v ^= w; continue; }
+				uint8_t gen = 1, gj = 1;
+				for (int t = 0; t < d.par_row[r]; ++t) gen = lz::gf_mul_host(gen, 2);
+				for (int t = 0; t < part; ++t) gj = lz::gf_mul_host(gj, gen);
+				v ^= lz::gf_mul_host(w, gj);
+			}
+			out->rows[x * 32 + a] = v;
+		}
+	return LZGPU_OK;
+}
+
 const char *lzgpu_version(void) { return "lizardfs_b200 0.1 (sm_100a)"; }
 
 }  // extern "C"

@@ -480,4 +480,36 @@ __global__ void __launch_bounds__(256) fill_chunks_kernel(uint8_t *base, unsigne
 	}
 }
 
+// Chunk rows between a batch and a compact copy of some of its chunks (the fallback groups of the per-chunk-pattern degraded read):
+// row r of plane y is copied from src + (gather ? idx[r] : r) * src_stride to dst + (gather ? r : idx[r]) * dst_stride, row_bytes
+// bytes, in 16-byte words (wide: every address and length a multiple of 16) or in 4-byte words (the stored CRC arrays).
+struct RowsPlane {
+	const uint8_t *src;
+	uint8_t *dst;
+	unsigned long long src_stride, dst_stride, row_bytes;
+	unsigned int gather, wide;
+};
+constexpr int kMaxRowsPlanes = 2 * 64 + 1;
+struct RowsCopyArgs {
+	RowsPlane pl[kMaxRowsPlanes];
+	const uint32_t *idx;
+	unsigned int n_rows;
+};
+
+__global__ void __launch_bounds__(256) rows_copy_kernel(const __grid_constant__ RowsCopyArgs a) {
+	const RowsPlane &P = a.pl[blockIdx.y];
+	const unsigned sh = P.wide ? 4u : 2u;
+	const unsigned long long words = P.row_bytes >> sh, total = words * a.n_rows;
+	const unsigned long long stride = static_cast<unsigned long long>(gridDim.x) * blockDim.x;
+	for (unsigned long long u = static_cast<unsigned long long>(blockIdx.x) * blockDim.x + threadIdx.x; u < total; u += stride) {
+		const unsigned r = static_cast<unsigned>(u / words);
+		const unsigned long long w = u - static_cast<unsigned long long>(r) * words;
+		const unsigned long long rs = P.gather ? a.idx[r] : r, rd = P.gather ? r : a.idx[r];
+		const uint8_t *s = P.src + rs * P.src_stride + (w << sh);
+		uint8_t *d = P.dst + rd * P.dst_stride + (w << sh);
+		if (P.wide) st_stream(reinterpret_cast<uint4 *>(d), ld_stream(reinterpret_cast<const uint4 *>(s)));
+		else *reinterpret_cast<uint32_t *>(d) = *reinterpret_cast<const uint32_t *>(s);
+	}
+}
+
 }  // namespace lzd

@@ -487,6 +487,99 @@ class Engine:
             raise ChunkCrcError(rc, "recover_chunks_dev", (bad[0], bad[1], bad[2]))
         _check(rc, "recover_chunks_dev")
 
+    # ---- degraded read with a loss pattern per chunk ------------------------------------------------
+    @staticmethod
+    def chunk_masks(masks):
+        """masks: (n, 2) uint64 array of (available, want) bit masks, or a list of (available, want) pairs whose entries are bit masks
+        or lists of per-part flags.  Returns the (n, 2) uint64 array lzgpu_chunk_mask[] reads."""
+        if isinstance(masks, np.ndarray) and masks.dtype == np.uint64 and masks.ndim == 2 and masks.shape[1] == 2:
+            return np.ascontiguousarray(masks)
+
+        def bits(v):
+            if isinstance(v, (int, np.integer)):
+                return int(v)
+            return sum(1 << i for i, f in enumerate(v) if f)
+        return np.array([[bits(a), bits(w)] for a, w in masks], dtype=np.uint64).reshape(-1, 2)
+
+    def recover_chunks_masked(self, goal, nb, parts, masks, part_crc=None, chunk_image=False):
+        """Degraded read with a loss pattern per chunk (lzgpu_recover_chunks_masked).  parts: list of k+m arrays [n_chunks, pb*64K] or None
+        (no chunk has the part); only the chunks whose mask marks a part available have it read.  masks: see chunk_masks.  Returns
+        (out_list, chunk_out or None): out[i] is [n, pb*64K] for every part some chunk rebuilds (zeros where a chunk does not rebuild it)."""
+        n_parts = goal.k + goal.m
+        assert len(parts) == n_parts
+        pb = (nb + goal.k - 1) // goal.k
+        parts = [None if p is None else _u8(p).reshape(-1, pb * BLOCK_SIZE) for p in parts]
+        mk = self.chunk_masks(masks)
+        n = mk.shape[0]
+        lost_wanted = int(np.bitwise_or.reduce(~mk[:, 0] & mk[:, 1])) if n else 0
+        lost_data = int(np.bitwise_or.reduce(~mk[:, 0])) & ((1 << goal.k) - 1) if (n and chunk_image) else 0
+        out = [np.zeros((n, pb * BLOCK_SIZE), dtype=np.uint8) if ((lost_wanted | lost_data) >> i & 1) else None for i in range(n_parts)]
+        crcs = None
+        if part_crc is not None:
+            crcs = [None if c is None else np.ascontiguousarray(c, dtype=np.uint32) for c in part_crc]
+        img = np.zeros((n, nb * BLOCK_SIZE), dtype=np.uint8) if chunk_image else None
+        bad = (C.c_int64 * 3)(-1, -1, -1)
+        rc = self.lib.lzgpu_recover_chunks_masked(self.h, C.byref(goal.c), n, nb, _p(mk), _ptr_array(parts), pb * BLOCK_SIZE,
+                                                  _ptr_array(crcs) if crcs is not None else None, _ptr_array(out), _p(img), nb * BLOCK_SIZE, bad)
+        if rc == _lib.ERR_CRC:
+            raise ChunkCrcError(rc, "recover_chunks_masked", (bad[0], bad[1], bad[2]))
+        _check(rc, "recover_chunks_masked")
+        return out, img
+
+    def recover_chunks_masked_dev(self, goal, n_chunks, nb, masks, d_parts, part_stride, d_part_crc, d_out, d_chunk_out=None,
+                                  chunk_out_stride=None, stream=None):
+        """Device-pointer twin of recover_chunks_masked (lzgpu_recover_chunks_masked_dev); waiting and errors as in recover_chunks_dev."""
+        n_parts = goal.k + goal.m
+        if d_chunk_out and chunk_out_stride is None:
+            raise ValueError("recover_chunks_masked_dev: chunk_out_stride is required with d_chunk_out")
+        chunk_out_stride = chunk_out_stride or 0
+        mk = self.chunk_masks(masks)
+        assert mk.shape[0] == n_chunks
+        dp = (C.c_void_p * n_parts)(*[p if p else None for p in d_parts])
+        dc = (C.c_void_p * n_parts)(*[p if p else None for p in d_part_crc]) if d_part_crc is not None else None
+        do = (C.c_void_p * n_parts)(*[p if p else None for p in d_out])
+        bad = (C.c_int64 * 3)(-1, -1, -1)
+        rc = self.lib.lzgpu_recover_chunks_masked_dev(self.h, C.byref(goal.c), n_chunks, nb, _p(mk), dp, part_stride, dc, do, d_chunk_out,
+                                                      chunk_out_stride, bad, stream)
+        if rc == _lib.ERR_CRC:
+            raise ChunkCrcError(rc, "recover_chunks_masked_dev", (bad[0], bad[1], bad[2]))
+        _check(rc, "recover_chunks_masked_dev")
+
+    MASKED_ROUTES = ("delegated", "one_launch", "fallback")
+
+    @staticmethod
+    def plan_recover_masked(goal, nb, masks, verify=False, image=False, part_stride=None, chunk_out_stride=None):
+        """how recover_chunks_masked* would serve the batch (pure host logic, csrc/fused_plan.h masked_route; no GPU needed).  Returns a
+        dict with delegated, patterns, one_launch_chunks, fallback_chunks, fallback_groups, rebuild_launches, e_chunks, form ("packed" or
+        "direct"), item_words, stripes_per_unit, stages, units_per_chunk, threads_per_cta, smem_bytes, desc_bytes, and route: per chunk one
+        of MASKED_ROUTES.  Raises LzGpuError (status ERR_TOO_FEW_PARTS) for a chunk with fewer than k available parts."""
+        mk = Engine.chunk_masks(masks)
+        n = mk.shape[0]
+        pb = (nb + goal.k - 1) // goal.k
+        part_stride = pb * BLOCK_SIZE if part_stride is None else part_stride
+        chunk_out_stride = (nb * BLOCK_SIZE if image else 0) if chunk_out_stride is None else chunk_out_stride
+        route = np.zeros(max(n, 1), dtype=np.uint8)
+        out = _lib.LzMaskedPlan()
+        _check(_lib.load().lzgpu_plan_recover_masked(C.byref(goal.c), n, nb, _p(mk), 1 if verify else 0, 1 if image else 0, part_stride,
+                                                     chunk_out_stride, _p(route), C.byref(out)), "plan_recover_masked")
+        d = {f: getattr(out, f) for f, _ in _lib.LzMaskedPlan._fields_}
+        d["e_chunks"] = list(out.e_chunks)
+        d["item_words"] = list(out.item_words)
+        d["form"] = Engine.RECOVER_FORMS[out.form]
+        d["route"] = [Engine.MASKED_ROUTES[r] for r in route[:n]]
+        return d
+
+    @staticmethod
+    def masked_chunk(goal, available, want, image=False):
+        """the masked kernel's descriptor of one chunk (lzgpu_debug_masked_chunk): dict with one_launch, e, used (slot -> part), erased,
+        rows (e lists of k coefficients: each rebuilt part as a combination of the inputs in slot order)"""
+        mk = Engine.chunk_masks([(available, want)])
+        out = _lib.LzMaskedChunk()
+        _check(_lib.load().lzgpu_debug_masked_chunk(C.byref(goal.c), _p(mk), 1 if image else 0, C.byref(out)), "debug_masked_chunk")
+        e = out.e
+        return {"one_launch": out.one_launch, "e": e, "used": list(out.used)[:goal.k], "erased": list(out.erased)[:e],
+                "rows": [list(out.rows)[x * 32:x * 32 + goal.k] for x in range(e)]}
+
     # ---- wire format --------------------------------------------------------------------------
     def write_data_prefixes(self, goal, nb, crc, chunk_ids, write_id_base=0):
         """LIZ_CLTOCS_WRITE_DATA prefixes (cltocs.h:116-137) for every block of every part: uint8 [n, k+m, pb, 38]
